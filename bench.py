@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- env-steps/s of the fused quadcopter env step and of the PPO rollout + update on B200 (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--workload c4|c2|k1|c3|c5|c1] [--only] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload c4|c2|k1|c3|c5|c1] [--only] [--impl reference] [--dump-outputs DIR]
 
 ONE JSON line on stdout.  Its top level is the step-only workload `c4` (configs[3]'s per-GPU shard: the configuration the
 metric's "at 1/2/4/8 B200" is quoted on); `"workloads"` carries the other halves of the metric measured in the same run:
@@ -22,7 +22,15 @@ with CUDA events on the launching stream, max over ranks; `roofline` = the domin
 CUDA events inside the run; `e2e` = the same metric through the reference-facing API with host buffers / host results
 (wall clock, copies inside); `cpu_baseline` = the reference's CPU path for that workload on this box's host cores.
 
+--steps K times K steps of every workload's value (the e2e, sustained and fp32 parity-path figures keep their own counts).
+A full run therefore times K PPO iterations of c3 and of c5 at 1M envs, and the reference arm runs K iterations of its CPU
+PPO loop for each: at large K that, not the step-only workloads, sets the wall time of a run.
 --only runs just the workload named by --workload (A/B timing, ncu captures).
+--dump-outputs DIR writes, for every workload timed in the run, what its timed path returned in its last step as
+DIR/<workload>_<name>.npy (float32; float64 for the env index): all envs, or a fixed sample of env columns where the full
+arrays exceed 12 MB (<workload>_env_index.npy says which; a --fuse at which one env alone exceeds it is refused), so a run
+writes at most 64 MB.  Inputs are seeded (--seed), so two builds run with the same arguments can be compared output for
+output.
 --impl reference times the reference's CPU implementation: the UNMODIFIED reference env staged by oracle/make_ref.py
 (oracle/_ref/reference_py.zip; kind "reference") where the reference has the path, the oracle port otherwise (the PPO loop
 lives in stable-baselines3, which is not installable here: kind "port").
@@ -44,6 +52,7 @@ sys.path.insert(0, ROOT)
 STATE_BYTES = 80                              # 5 quads per env, read once + written once per launch
 MLP_FLOP = 20864.0                            # policy + value forward per env-step (2 x (15*64 + 64*64) + 64*4 + 64) x 2
 MOTOR_MAX = 7.3575
+DUMP_BYTES = 12 << 20                         # --dump-outputs, per workload: the four workloads of one run stay under 64 MB
 
 
 def json_safe(o):
@@ -352,18 +361,17 @@ def reference_ppo_line(args, wl, cores):
         loop.collect_rollouts()
         if update:
             loop.train()
-    steps = args.steps if wl == args.workload else max(2, min(args.steps, 4))
     for _ in range(max(1, min(args.warmup, 2))):
         one()
     t0 = time.perf_counter()
-    for _ in range(steps):
+    for _ in range(args.steps):
         one()
     dt = time.perf_counter() - t0
-    v = steps * c["n_envs"] * c["n_steps"] / dt
+    v = args.steps * c["n_envs"] * c["n_steps"] / dt
     sample = (f"restated SB3 loop on CPU (torch, all host threads + numpy env port; SB3 itself is not installable): {c['n_envs']} envs x "
               f"{c['n_steps']} steps per bench step" + (f", {c['n_epochs']} epochs x {c['minibatches']} minibatches" if update else ", rollout only"))
     return {"impl": "reference", "metric": "env_steps_per_sec", "value": v, "unit": "env-steps/s", "n_gpus": args.gpus,
-            "steps": steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / steps,
+            "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps,
             "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": WORKLOAD_NAMES[wl], "sample": sample},
             "cpu_baseline": {"value": v, "unit": "env-steps/s", "cores": cores, "kind": "port", "sample": sample},
@@ -391,10 +399,11 @@ def run_reference(args):
 # GPU arm
 # ------------------------------------------------------------------------------------------------
 class Ctx:
-    def __init__(self):
+    def __init__(self, dump=False):
         import torch
         import torch.distributed as dist
         self.torch, self.dist = torch, dist
+        self.dump = {} if dump else None          # name -> array, filled by capture()
         self.world = int(os.environ.get("WORLD_SIZE", "1"))
         self.rank = int(os.environ.get("RANK", "0"))
         self.local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -426,6 +435,24 @@ class Ctx:
             self.dist.barrier()
             self.dist.destroy_process_group()
 
+    def capture(self, wl, arrays):
+        """--dump-outputs: host float32 copies of `arrays` ({name: device tensor [steps, n, ...]}, what a caller of the timed path
+        receives) -- every env, or a fixed, seeded sample of env columns where the arrays exceed DUMP_BYTES."""
+        if self.dump is None:
+            return
+        torch = self.torch
+        n = next(iter(arrays.values())).shape[1]
+        per_env = 4 * sum(t[:, 0].numel() for t in arrays.values())
+        if per_env > DUMP_BYTES:
+            raise SystemExit(f"bench.py --dump-outputs: one env of {wl} returns {per_env} bytes per step, more than the "
+                             f"{DUMP_BYTES}-byte sample; use a smaller --fuse")
+        m = min(n, DUMP_BYTES // per_env)
+        idx = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+        sel = torch.from_numpy(idx).to(self.dev)
+        self.dump[f"{wl}_env_index"] = idx.astype(np.float64)
+        for name, t in arrays.items():
+            self.dump[f"{wl}_{name}"] = t.index_select(1, sel).float().cpu().numpy()
+
 
 def bench_env(ctx, args, wl, steps, warmup, want_cpu):
     """c4 / c2 / k1: one launch of the fused kernel per bench step."""
@@ -442,7 +469,8 @@ def bench_env(ctx, args, wl, steps, warmup, want_cpu):
     if wl == "c4":
         acts_in, acts_out = None, torch.empty(fuse, n, 4, device=dev)
     else:
-        acts_in, acts_out = torch.rand(fuse, n, 4, device=dev) * MOTOR_MAX, None
+        gen = torch.Generator(device=dev).manual_seed(args.seed + rank)
+        acts_in, acts_out = torch.rand(fuse, n, 4, device=dev, generator=gen) * MOTOR_MAX, None
 
     def one_step():
         if wl == "k1":
@@ -469,6 +497,9 @@ def bench_env(ctx, args, wl, steps, warmup, want_cpu):
                 batch.reset()
         ctx.barrier()
     launches = batch.launch_count - l0
+    last = slice(0, 1 if wl == "k1" else fuse)
+    ctx.capture(wl, dict(next_obs=nxt[last], reward=rew[last], done=done[last],
+                         **({"actions": acts_out} if acts_out is not None else {})))
     per = [ev[2 * i].elapsed_time(ev[2 * i + 1]) for i in range(steps)]      # ms per launch of the dominant kernel
     sustained = None
     if wl == "c4" and args.sustain_s > 0:
@@ -600,7 +631,8 @@ def e2e_env(ctx, args, wl, n, cfg, steps):
     return res
 
 
-def ppo_variant(ctx, args, wl, n, K, minibatches, epochs, rollout_precision, update_precision, steps, warmup, want_e2e):
+def ppo_variant(ctx, args, wl, n, K, minibatches, epochs, rollout_precision, update_precision, steps, warmup, want_e2e,
+                dump=False):
     """One precision variant of c3 / c5 / c1: timed region + the dominant kernel's CUDA-event time."""
     torch, drl, dev, world = ctx.torch, ctx.drl, ctx.dev, ctx.world
     from drone_rl_b200.ppo import PPO
@@ -645,6 +677,12 @@ def ppo_variant(ctx, args, wl, n, K, minibatches, epochs, rollout_precision, upd
         ev1.record()
         ctx.barrier()
     launches = env.launch_count + model.launches - l0
+    if dump and ctx.dump is not None:
+        b = model.buf
+        ctx.capture(wl, dict(obs=b.obs, actions=b.actions, logp=b.logp, value=b.value, reward=b.reward, done=b.done, adv=b.adv,
+                             ret=b.ret, last_value=b.last_value[None]))
+        if full:
+            ctx.dump[f"{wl}_params"] = model.params.cpu().numpy()
     total_ms = ctx.max_over_ranks(ev0.elapsed_time(ev1))
     value = n * K * steps * world / (total_ms * 1e-3)
     up = update_precision
@@ -722,7 +760,7 @@ def bench_ppo(ctx, args, wl, steps, warmup, want_cpu, both=True):
     else:
         n, K, mb, ep = args.ppo_envs, args.fuse, args.ppo_minibatches, args.ppo_epochs
     rp, up = args.precision, (args.update_precision or args.precision)
-    main = ppo_variant(ctx, args, wl, n, K, mb, ep, rp, up, steps, warmup, not args.no_e2e)
+    main = ppo_variant(ctx, args, wl, n, K, mb, ep, rp, up, steps, warmup, not args.no_e2e, dump=True)
     res = {"value": main["value"], "unit": "env-steps/s", "steps": main["steps"], "warmup": warmup, "ms_per_step": main["ms_per_step"],
            "dtype": ("f32" if rp == "fp32" else "tf32 (fp32 accumulate)") if wl == "c3" else
                     "rollout MLP %s, update %s (fp32 accumulate; env step, loss, Adam in f32)" % (rp, up),
@@ -768,12 +806,17 @@ def main():
     ap.add_argument("--precision", default="tf32", choices=["fp32", "tf32"], help="policy MLP in the rollout: CUDA cores or tcgen05")
     ap.add_argument("--update-precision", default="bf16", choices=["fp32", "tf32", "bf16"], help="PPO minibatch gradient: fp32 = CUDA cores (parity path), tf32 = tcgen05 all-tf32, bf16 = tcgen05 with bf16 weight-gradient operands, three tiles per SM (default)")
     ap.add_argument("--dp-backend", default="peer", choices=["peer", "nccl"], help="N > 1: gradient exchange + clip + Adam as one kernel over NVLink peer memory (default), or NCCL all-reduce between the kernels")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what each timed path returned in its last step as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs: not with --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
 
-    ctx = Ctx()
+    ctx = Ctx(dump=bool(args.dump_outputs))
     wl = args.workload
     want_cpu = ctx.world == 1 and not args.no_cpu and ctx.rank == 0
     if wl in ("c3", "c5", "c1"):
@@ -782,11 +825,15 @@ def main():
         top = bench_env(ctx, args, wl, args.steps, args.warmup, want_cpu)
     extra = {}
     if wl == "c4" and not args.only:
-        # the rest of the metric in the same run; PPO iterations are 10-100x longer than a step-only launch: fewer steps
+        # the rest of the metric in the same run
         if ctx.world == 1:
-            extra["c2"] = bench_env(ctx, args, "c2", max(5, min(args.steps, 20)), 3, want_cpu)
-        extra["c3"] = bench_ppo(ctx, args, "c3", max(3, min(args.steps, 10)), 3, want_cpu)
-        extra["c5"] = bench_ppo(ctx, args, "c5", max(3, min(args.steps, 5)), 3, want_cpu)
+            extra["c2"] = bench_env(ctx, args, "c2", args.steps, args.warmup, want_cpu)
+        extra["c3"] = bench_ppo(ctx, args, "c3", args.steps, args.warmup, want_cpu)
+        extra["c5"] = bench_ppo(ctx, args, "c5", args.steps, args.warmup, want_cpu)
+    if ctx.rank == 0 and ctx.dump is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in ctx.dump.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if ctx.rank == 0:
         line = {"metric": "env_steps_per_sec", "value": top["value"], "unit": "env-steps/s", "n_gpus": ctx.world,
                 "steps": top["steps"], "warmup": top["warmup"], "ms_per_step": top["ms_per_step"], "higher_is_better": True,

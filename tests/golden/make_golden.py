@@ -126,8 +126,15 @@ def gen_vector_rollout(vd_mod, batch=16, n_steps=1003):
     print("vector_rollout: bonus steps", int((rew > 0).sum()), "done frac", float(done.mean()))
 
 
+def teacher_forced_rows(n_drawn=4096, n_corner=16, n_keep=2048):
+    """The rows of the teacher-forced draw that are stored (the file stays under 1 MB): the hand-made corner cases at the
+    front, then a fixed, seeded sample of the random rows.  Every row is an independent one-step case."""
+    rest = np.random.default_rng(4).choice(np.arange(n_corner, n_drawn), n_keep - n_corner, replace=False)
+    return np.concatenate([np.arange(n_corner), np.sort(rest)])
+
+
 def gen_teacher_forced(drone_mod, vd_mod, n=4096):
-    """One step from injected float32-representable states, through BOTH reference envs."""
+    """One step from injected float32-representable states, through BOTH reference envs (the rows teacher_forced_rows keeps)."""
     rng = np.random.default_rng(3)
     f32 = np.float32
     pos = (rng.normal(0, 3, (n, 3))).astype(f32)
@@ -158,6 +165,9 @@ def gen_teacher_forced(drone_mod, vd_mod, n=4096):
     step_count[k] = 199; k += 1                                          # time limit this step
     step_count[k] = 198; k += 1
 
+    keep = teacher_forced_rows(n, k)
+    pos, vel, euler, omega, target, action, step_count = (a[keep] for a in (pos, vel, euler, omega, target, action, step_count))
+    n = keep.size
     out = {"pos": pos, "vel": vel, "euler": euler, "omega": omega, "target": target,
            "action": action, "step_count": step_count.astype(np.int32)}
     with np.errstate(all="ignore"):

@@ -94,7 +94,7 @@ def _done_margin_ok(o_env, spec):
 
 @pytest.mark.parametrize("spec", [do.SINGLE, do.VECTOR], ids=["single", "vector"])
 def test_teacher_forced_golden(drl, golden, spec):
-    """4096 one-step cases incl. crash / out-of-range / bonus / near-singular pitch / NaN / inf /
+    """2048 one-step cases incl. crash / out-of-range / bonus / near-singular pitch / NaN / inf /
     huge angles / unclipped actions / time limit -- against the unmodified reference's outputs."""
     g = golden("teacher_forced")
     n = g["pos"].shape[0]
