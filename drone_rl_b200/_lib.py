@@ -66,6 +66,18 @@ class PPOConfig(C.Structure):
                 ("max_grad_norm", C.c_float)]
 
 
+class NormPassArgs(C.Structure):
+    """Mirror of ``dronecu_norm_pass_args`` (include/dronecu.h)."""
+    _fields_ = [("d_obs", C.c_void_p), ("obs_stride", C.c_int32), ("K", C.c_int32), ("n", C.c_int64),
+                ("d_affine", C.c_void_p), ("d_reward", C.c_void_p), ("d_done", C.c_void_p), ("d_returns", C.c_void_p),
+                ("d_stats", C.c_void_p), ("gamma", C.c_double), ("epsilon", C.c_double), ("clip_reward", C.c_double),
+                ("update", C.c_int32), ("side_env", C.c_int32), ("d_side_obs", C.c_void_p), ("d_partials", C.c_void_p)]
+
+
+NORM_AFFINE = 31
+NORM_STATS = 34
+NORM_MOMENTS = 34
+NORM_BLOCK = 256
 POLICY_PARAMS = 10697
 GRAD_LEN = POLICY_PARAMS + 8
 IPC_HANDLE_BYTES = 64
@@ -108,6 +120,10 @@ _SIGNATURES = {
     "dronecu_set_rollout_kernel": (C.c_int, [C.c_int]),
     "dronecu_rollout_policy_tc": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(PolicyOut), _P]),
     "dronecu_policy_forward_tc": (C.c_int, [C.c_int, C.c_int64, _P, _P, _P, _P, _P, _P, _P]),
+    "dronecu_rollout_policy_norm": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(PolicyOut), _P, C.c_int, _P]),
+    "dronecu_norm_pass": (C.c_int, [C.c_int, C.POINTER(NormPassArgs), _P]),
+    "dronecu_norm_reduce": (C.c_int, [C.c_int, _P, C.c_int64, _P, _P]),
+    "dronecu_norm_combine": (C.c_int, [C.c_int, _P, _P, C.c_double, C.c_float, _P, _P]),
     "dronecu_gae": (C.c_int, [C.c_int, C.c_int, C.c_int64, _P, _P, _P, _P, C.c_float, C.c_float, _P, _P, _P]),
     "dronecu_ppo_config_default": (None, [C.POINTER(PPOConfig)]),
     "dronecu_ppo_create": (C.c_int, [C.POINTER(PPOConfig), C.c_int, C.POINTER(_P)]),

@@ -15,6 +15,7 @@
 #include "ppo_update_tc.cuh"
 #include "ppo_update_tc3.cuh"
 #include "ppo_dp.cuh"
+#include "obs_norm.cuh"
 
 using namespace dronecu;
 
@@ -51,8 +52,27 @@ extern "C" int dronecu_set_rollout_kernel(int mode) {
   return DRONECU_OK;
 }
 
+enum RolloutKernel { kThreadPerEnv, kWarpPerEnv, kTensorCores };
+
+template <bool RANDOMIZED, bool NORM>
+static int launch_policy_rollout(RolloutKernel which, int64_t n, const PolicyArgs& a, cudaStream_t st) {
+  if (which == kTensorCores) {
+    static_assert(tc::kTile == kPolBlock, "tile size");
+    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_tc_kernel<RANDOMIZED, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem));
+    policy_rollout_tc_kernel<RANDOMIZED, NORM><<<(unsigned)((n + kPolBlock - 1) / kPolBlock), tc::kTile, kTcSmem, st>>>(a);
+  } else if (which == kWarpPerEnv) {
+    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_warp_kernel<RANDOMIZED, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmallSmem));
+    policy_rollout_warp_kernel<RANDOMIZED, NORM><<<(unsigned)((n + kSmallWarps - 1) / kSmallWarps), 32 * kSmallWarps, kPolicySmallSmem, st>>>(a);
+  } else {
+    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_kernel<RANDOMIZED, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmem));
+    policy_rollout_kernel<RANDOMIZED, NORM><<<(unsigned)((n + kPolBlock - 1) / kPolBlock), kPolBlock, kPolicySmem, st>>>(a);
+  }
+  return DRONECU_OK;
+}
+
 static int rollout_policy_impl(dronecu_env* e, int K, const float* d_params, int deterministic,
-                               const dronecu_policy_out* out, void* stream, bool tensor_cores) {
+                               const dronecu_policy_out* out, void* stream, bool tensor_cores,
+                               const float* d_norm_affine = nullptr) {
   if (!e || !d_params) return fail(DRONECU_ERR_INVALID, "dronecu_rollout_policy: null argument");
   if (K <= 0) return fail(DRONECU_ERR_INVALID, "K must be positive");
   if (e->cfg.obs_dim != 15 || !(e->cfg.flags & DRONECU_AUTORESET))
@@ -66,40 +86,22 @@ static int rollout_policy_impl(dronecu_env* e, int K, const float* d_params, int
   std::memset(&a, 0, sizeof(a));
   a.state = e->sp; a.P = e->P; a.n = e->n; a.K = K; a.t0 = e->t; a.theta = d_params; a.deterministic = deterministic;
   a.stats = e->stats;
+  a.norm = d_norm_affine;
   if (out) {
     a.obs = out->d_obs; a.obs_padded = out->obs_padded ? 1 : 0;
     a.actions = reinterpret_cast<float4*>(out->d_actions); a.logp = out->d_logp;
     a.value = out->d_value; a.reward = out->d_reward; a.done = out->d_done; a.last_value = out->d_last_value;
     a.last_obs = out->d_last_obs;
   }
-  const unsigned grid = (unsigned)((e->n + kPolBlock - 1) / kPolBlock);
+  // small batches: one warp per env (ppo_rollout.cuh)
+  const RolloutKernel which = tensor_cores ? kTensorCores
+      : (g_rollout_kernel_mode == 2 || (g_rollout_kernel_mode == 0 && e->n <= kWarpRolloutMaxEnvs)) ? kWarpPerEnv : kThreadPerEnv;
   cudaStream_t st = (cudaStream_t)stream;
-  if (tensor_cores) {
-    static_assert(tc::kTile == kPolBlock, "tile size");
-    if (e->cfg.flags & DRONECU_RANDOMIZED) {
-      CUDA_TRY(cudaFuncSetAttribute(policy_rollout_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem));
-      policy_rollout_tc_kernel<true><<<grid, tc::kTile, kTcSmem, st>>>(a);
-    } else {
-      CUDA_TRY(cudaFuncSetAttribute(policy_rollout_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem));
-      policy_rollout_tc_kernel<false><<<grid, tc::kTile, kTcSmem, st>>>(a);
-    }
-  } else if (g_rollout_kernel_mode == 2 || (g_rollout_kernel_mode == 0 && e->n <= kWarpRolloutMaxEnvs)) {
-    // small batches: one warp per env (ppo_rollout.cuh)
-    const unsigned gw = (unsigned)((e->n + kSmallWarps - 1) / kSmallWarps);
-    if (e->cfg.flags & DRONECU_RANDOMIZED) {
-      CUDA_TRY(cudaFuncSetAttribute(policy_rollout_warp_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmallSmem));
-      policy_rollout_warp_kernel<true><<<gw, 32 * kSmallWarps, kPolicySmallSmem, st>>>(a);
-    } else {
-      CUDA_TRY(cudaFuncSetAttribute(policy_rollout_warp_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmallSmem));
-      policy_rollout_warp_kernel<false><<<gw, 32 * kSmallWarps, kPolicySmallSmem, st>>>(a);
-    }
-  } else if (e->cfg.flags & DRONECU_RANDOMIZED) {
-    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmem));
-    policy_rollout_kernel<true><<<grid, kPolBlock, kPolicySmem, st>>>(a);
-  } else {
-    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmem));
-    policy_rollout_kernel<false><<<grid, kPolBlock, kPolicySmem, st>>>(a);
-  }
+  const bool randomized = (e->cfg.flags & DRONECU_RANDOMIZED) != 0;
+  int rc;
+  if (d_norm_affine) rc = randomized ? launch_policy_rollout<true, true>(which, e->n, a, st) : launch_policy_rollout<false, true>(which, e->n, a, st);
+  else rc = randomized ? launch_policy_rollout<true, false>(which, e->n, a, st) : launch_policy_rollout<false, false>(which, e->n, a, st);
+  if (rc != DRONECU_OK) return rc;
   e->launches += 1;
   CUDA_TRY(cudaGetLastError());
   e->t += (uint64_t)K;
@@ -115,6 +117,56 @@ extern "C" int dronecu_rollout_policy(dronecu_env* e, int K, const float* d_para
 extern "C" int dronecu_rollout_policy_tc(dronecu_env* e, int K, const float* d_params, int deterministic,
                                          const dronecu_policy_out* out, void* stream) {
   return rollout_policy_impl(e, K, d_params, deterministic, out, stream, true);
+}
+
+extern "C" int dronecu_rollout_policy_norm(dronecu_env* e, int K, const float* d_params, int deterministic,
+                                           const dronecu_policy_out* out, const float* d_norm_affine, int tensor_cores,
+                                           void* stream) {
+  return rollout_policy_impl(e, K, d_params, deterministic, out, stream, tensor_cores != 0, d_norm_affine);
+}
+
+// ------------------------------------------------------------------------------------------------
+// observation / reward normalisation (csrc/obs_norm.cuh)
+// ------------------------------------------------------------------------------------------------
+static_assert(kNormAffine == DRONECU_NORM_AFFINE && kNormStats == DRONECU_NORM_STATS && kNormMoments == DRONECU_NORM_MOMENTS &&
+              kNormBlock == DRONECU_NORM_BLOCK, "header / kernel normaliser layout mismatch");
+
+extern "C" int dronecu_norm_pass(int device, const dronecu_norm_pass_args* p, void* stream) {
+  if (!p || p->K <= 0 || p->n <= 0) return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: bad argument");
+  if (p->d_obs && (p->obs_stride != 15 && p->obs_stride != 16))
+    return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: obs_stride must be 15 or 16");
+  if (p->d_obs && p->obs_stride == 16 && (reinterpret_cast<uintptr_t>(p->d_obs) & 15))
+    return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: padded d_obs must be 16-byte aligned");
+  if (p->d_obs && !p->d_affine) return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: d_obs needs d_affine");
+  if (p->d_reward && (!p->d_done || !p->d_stats || (p->update && !p->d_returns)))
+    return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: d_reward needs d_done, d_stats and (update) d_returns");
+  if (p->update && (!p->d_stats || !p->d_partials)) return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: update needs d_stats and d_partials");
+  DeviceGuard guard(device);
+  NormPassArgs a;
+  a.obs = p->d_obs; a.stride = p->obs_stride; a.K = p->K; a.n = p->n; a.affine = p->d_affine;
+  a.reward = p->d_reward; a.done = p->d_done; a.returns = p->d_returns; a.stats = p->d_stats;
+  a.gamma = p->gamma; a.epsilon = p->epsilon; a.clip_reward = p->clip_reward; a.update = p->update;
+  a.side_env = p->side_env; a.side_obs = p->d_side_obs; a.partials = p->d_partials;
+  obs_norm_pass_kernel<<<(unsigned)((p->n + kNormBlock - 1) / kNormBlock), kNormBlock, 0, (cudaStream_t)stream>>>(a);
+  CUDA_TRY(cudaGetLastError());
+  return DRONECU_OK;
+}
+
+extern "C" int dronecu_norm_reduce(int device, const double* d_partials, int64_t n_partials, double* d_moments, void* stream) {
+  if (!d_partials || !d_moments || n_partials <= 0) return fail(DRONECU_ERR_INVALID, "dronecu_norm_reduce: bad argument");
+  DeviceGuard guard(device);
+  obs_norm_reduce_kernel<<<1, kNormReduceThreads, 0, (cudaStream_t)stream>>>(d_partials, n_partials, d_moments);
+  CUDA_TRY(cudaGetLastError());
+  return DRONECU_OK;
+}
+
+extern "C" int dronecu_norm_combine(int device, double* d_stats, const double* d_moments, double epsilon, float clip_obs,
+                                    float* d_affine, void* stream) {
+  if (!d_stats || !(epsilon >= 0) || !(clip_obs > 0)) return fail(DRONECU_ERR_INVALID, "dronecu_norm_combine: bad argument");
+  DeviceGuard guard(device);
+  obs_norm_combine_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(d_stats, d_moments, epsilon, clip_obs, d_affine);
+  CUDA_TRY(cudaGetLastError());
+  return DRONECU_OK;
 }
 
 extern "C" int dronecu_policy_forward_tc(int device, int64_t B, const float* d_params, const float* d_obs, float* d_mean,

@@ -8,6 +8,7 @@
 #pragma once
 #include "env_kernels.cuh"
 #include "ppo_common.cuh"
+#include "obs_norm.cuh"
 
 namespace dronecu {
 
@@ -131,17 +132,22 @@ struct PolicyArgs {
   float* last_value;      // [n]      V(observation after the K-th step)
   float* last_obs;        // [n,15]
   StatSlot* stats;
+  const float* norm;      // [31] float32 affine record (obs_norm.cuh): read only by the NORM instantiations
 };
 
-template <bool RANDOMIZED>
+// NORM: the towers see norm_obs_row(x) (obs_norm.cuh) -- the buffer still receives the raw row, obs_norm_pass_kernel
+// normalises it afterwards with the same function and the same record
+template <bool RANDOMIZED, bool NORM = false>
 __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_constant__ PolicyArgs A) {
   extern __shared__ __align__(128) unsigned char smem_raw[];      // > 48 KB: dynamic shared memory
   MlpSmem& S = *reinterpret_cast<MlpSmem*>(smem_raw);
   float (*tiles)[32 * kObs] = reinterpret_cast<float (*)[32 * kObs]>(smem_raw + sizeof(MlpSmem));
   __shared__ unsigned long long blk_stats[3];
   __shared__ double blk_ret;
+  __shared__ float s_norm[NORM ? kNormAffine : 1];
 
   load_mlp_smem(S, A.theta);
+  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s_norm[threadIdx.x] = A.norm[threadIdx.x]; }
   if (threadIdx.x < 3) blk_stats[threadIdx.x] = 0;
   if (threadIdx.x == 3) blk_ret = 0.0;
   __syncthreads();
@@ -186,6 +192,7 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
         st_quad(d + 3, make_float4(x[12], x[13], x[14], 1.0f));
       }
     } else if (A.obs != nullptr && valid > 0) emit_obs_rows<kObs>(tile, p_obs, s, lane, valid, active, fast_obs);
+    if constexpr (NORM) norm_obs_row(x, s_norm);
 
     float mean[kAct], val[1];
     tower_forward<kAct>(S, 0, x, mean);
@@ -230,6 +237,7 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
     float x[kObs], val[1];
     write_obs<kObs>(x, s);
     if (A.last_value != nullptr) {
+      if constexpr (NORM) norm_obs_row(x, s_norm);
       tower_forward<1>(S, 1, x, val);
       if (active) A.last_value[i] = val[0];
     }
@@ -313,13 +321,15 @@ __device__ __forceinline__ void tower_forward_warp(const MlpSmem& S, float* __re
   }
 }
 
-template <bool RANDOMIZED>
+template <bool RANDOMIZED, bool NORM = false>
 __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(const __grid_constant__ PolicyArgs A) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   MlpSmem& S = *reinterpret_cast<MlpSmem*>(smem_raw);
   __shared__ unsigned long long blk_stats[3];
   __shared__ double blk_ret;
+  __shared__ float s_norm[NORM ? kNormAffine : 1];
   load_mlp_smem(S, A.theta);
+  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s_norm[threadIdx.x] = A.norm[threadIdx.x]; }
   if (threadIdx.x < 3) blk_stats[threadIdx.x] = 0;
   if (threadIdx.x == 3) blk_ret = 0.0;
   __syncthreads();
@@ -355,6 +365,7 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(c
         for (int c = 0; c < kObs; ++c) A.obs[row * kObs + c] = x[c];
       }
     }
+    if constexpr (NORM) norm_obs_row(x, s_norm);
     float mean[kAct], val[1];
     tower_forward_warp<kAct>(S, hbuf, 0, x, mean, lane);
     tower_forward_warp<1>(S, hbuf, 1, x, val, lane);
@@ -393,7 +404,15 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(c
     float x[kObs], val[1];
     write_obs<kObs>(x, s);
     if (A.last_value != nullptr) {
-      tower_forward_warp<1>(S, hbuf, 1, x, val, lane);
+      if constexpr (NORM) {                     // x itself is stored raw to last_obs below
+        float xn[kObs];
+#pragma unroll
+        for (int c = 0; c < kObs; ++c) xn[c] = x[c];
+        norm_obs_row(xn, s_norm);
+        tower_forward_warp<1>(S, hbuf, 1, xn, val, lane);
+      } else {
+        tower_forward_warp<1>(S, hbuf, 1, x, val, lane);
+      }
       if (writer) A.last_value[i] = val[0];
     }
     if (writer && A.last_obs != nullptr) {

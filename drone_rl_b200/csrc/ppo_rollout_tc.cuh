@@ -35,15 +35,17 @@ __global__ void __launch_bounds__(tc::kTile) policy_forward_tc_kernel(const floa
   tc::teardown(S);
 }
 
-template <bool RANDOMIZED>
+template <bool RANDOMIZED, bool NORM = false>
 __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __grid_constant__ PolicyArgs A) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   tc::Smem& S = tc_smem(smem_raw);
   float (*tiles)[32 * kObs] = reinterpret_cast<float (*)[32 * kObs]>(reinterpret_cast<unsigned char*>(&S) + sizeof(tc::Smem));
   __shared__ unsigned long long blk_stats[3];
   __shared__ double blk_ret;
+  __shared__ float s_norm[NORM ? kNormAffine : 1];
   if (threadIdx.x < 3) blk_stats[threadIdx.x] = 0;
   if (threadIdx.x == 3) blk_ret = 0.0;
+  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s_norm[threadIdx.x] = A.norm[threadIdx.x]; }
   tc::setup(S, A.theta);
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -84,6 +86,7 @@ __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __gr
         st_quad(d + 3, make_float4(x[12], x[13], x[14], 1.0f));
       }
     } else if (A.obs != nullptr && valid > 0) emit_obs_rows<kObs>(tile, p_obs, s, lane, valid, active, fast_obs);
+    if constexpr (NORM) norm_obs_row(x, s_norm);
 
     float mean[kAct], val;
     tc::forward(S, x, phase, mean, val);
@@ -124,6 +127,7 @@ __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __gr
     float x[kObs], val;
     write_obs<kObs>(x, s);
     if (A.last_value != nullptr) {       // uniform across the CTA: every thread takes part in the forward
+      if constexpr (NORM) norm_obs_row(x, s_norm);
       val = tc::forward_value(S, x, phase);
       if (active) A.last_value[i] = val;
     }

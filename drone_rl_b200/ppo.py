@@ -106,6 +106,13 @@ class PPO:
     int = number of envs to create.  Defaults are SB3's (n_steps 2048, batch_size 64, n_epochs 10,
     gamma 0.99, gae_lambda 0.95, clip 0.2, ent 0, vf 0.5, max_grad_norm 0.5, lr 3e-4, Adam eps 1e-5).
     ``batch_size`` counts samples PER RANK.
+
+    ``norm_obs`` / ``norm_reward``: SB3's ``VecNormalize`` (clip_obs, clip_reward, norm_epsilon as there; gamma is PPO's),
+    computed inside the rollout (normalize.py).  The running statistics are frozen for the length of one rollout and merged
+    after it (SB3 updates them after every env step).  The rollout buffer then holds normalised observations and rewards, as
+    SB3's does under VecNormalize; episode statistics stay in raw reward.  ``obs_rms`` / ``ret_rms`` / ``training`` /
+    ``normalize_obs`` mirror the VecNormalize attributes, and ``predict`` normalises its input with the model's statistics
+    (under SB3 the wrapped env does that).
     """
 
     tc_min_envs = 1024       # rollout_precision "tf32": tensor-core rollout kernel above this many envs per rank
@@ -115,7 +122,8 @@ class PPO:
                  max_grad_norm: float = 0.5, learning_rate: float = 3e-4, normalize_advantage: bool = True,
                  seed: int = 0, device: int = 0, verbose: int = 0, policy_seed: Optional[int] = None,
                  rollout_precision: str = "fp32", update_precision: str = "fp32", cuda_graph: Optional[bool] = None,
-                 dp_backend: str = "peer", padded_obs: Optional[bool] = None):
+                 dp_backend: str = "peer", padded_obs: Optional[bool] = None, norm_obs: bool = False,
+                 norm_reward: bool = False, clip_obs: float = 10.0, clip_reward: float = 10.0, norm_epsilon: float = 1e-8):
         self.lib = _lib.load()
         self.rank, self.world = 0, 1
         if torch.distributed.is_available() and torch.distributed.is_initialized():
@@ -160,6 +168,12 @@ class PPO:
         if self.world > 1:
             self._dp_setup()
         self._gen = torch.Generator(device=self.device).manual_seed(seed + 1)
+        self.normalizer = None
+        if norm_obs or norm_reward:
+            from .normalize import ObsNormalizer
+            self.normalizer = ObsNormalizer(self.n_envs, self.device, norm_obs, norm_reward, clip_obs, clip_reward, norm_epsilon,
+                                            gamma)
+        self.side_env, self.side_obs = -1, None     # set_raw_obs_tap(): raw rows of one env per rollout
         self.num_timesteps, self.n_updates = 0, 0
         self._perm, self._epochs_done = None, 0
         self.grad_events = None                   # set to [] to collect (start, end, samples) events per gradient launch
@@ -252,17 +266,61 @@ class PPO:
         except Exception:
             pass
 
+    # -- normalisation (SB3 VecNormalize attributes) ------------------------------------------------------
+    @property
+    def obs_rms(self):
+        """Running mean / var / count of the observations (numpy, float64), or None without normalisation."""
+        return None if self.normalizer is None else self.normalizer.obs_rms
+
+    @property
+    def ret_rms(self):
+        return None if self.normalizer is None else self.normalizer.ret_rms
+
+    @property
+    def training(self) -> bool:
+        """False (evaluation): the rollout keeps normalising but leaves the statistics and per-env returns unchanged."""
+        return True if self.normalizer is None else self.normalizer.training
+
+    @training.setter
+    def training(self, value: bool):
+        if self.normalizer is not None:
+            self.normalizer.training = bool(value)
+
+    def normalize_obs(self, obs) -> torch.Tensor:
+        """Observations [.., 15] normalised with the current statistics (a device copy; unchanged without norm_obs)."""
+        x = torch.as_tensor(np.asarray(obs, dtype=np.float32) if not torch.is_tensor(obs) else obs)
+        if self.normalizer is None:
+            return x.to(self.device, torch.float32).reshape(-1, 15)
+        return self.normalizer.normalize_obs(x)
+
+    def set_raw_obs_tap(self, env_index: int):
+        """Keep the RAW observation rows of env ``env_index`` of every rollout in ``self.side_obs`` [n_steps, 15] (the
+        rollout buffer holds normalised rows when norm_obs is on)."""
+        self.side_env = int(env_index)
+        self.side_obs = torch.empty(self.n_steps, 15, dtype=torch.float32, device=self.device)
+
     # -- rollout ------------------------------------------------------------------------------------
     def collect_rollouts(self, deterministic: bool = False):
-        """One launch: n_steps env steps for every env, policy evaluated in-kernel; then GAE."""
+        """One launch: n_steps env steps for every env, policy evaluated in-kernel; then GAE.  With normalisation: the
+        rollout's towers see normalised observations, then one pass rewrites the buffer normalised, the moments are
+        reduced [and summed over the ranks] and merged into the statistics (training only), then GAE."""
         b, K, n = self.buf, self.n_steps, self.n_envs
         out = PolicyOut(b.obs_store.data_ptr(), b.actions.data_ptr(), b.logp.data_ptr(), b.value.data_ptr(),
                         b.reward.data_ptr(), b.done.data_ptr(), b.last_value.data_ptr(), None, int(self.padded_obs), 0)
         st = _stream_ptr(self.device)
         # tensor cores pay from ~1k envs (a tile is 128 envs; below that the float32 warp-per-env kernel is both faster and exact)
         use_tc = self.rollout_precision == "tf32" and self.n_envs > self.tc_min_envs
-        fn = self.lib.dronecu_rollout_policy_tc if use_tc else self.lib.dronecu_rollout_policy
-        _lib.check(fn(self.batch._h, K, _ptr(self.params), int(deterministic), C.byref(out), st), "dronecu_rollout_policy")
+        nz = self.normalizer
+        if nz is None:
+            fn = self.lib.dronecu_rollout_policy_tc if use_tc else self.lib.dronecu_rollout_policy
+            _lib.check(fn(self.batch._h, K, _ptr(self.params), int(deterministic), C.byref(out), st), "dronecu_rollout_policy")
+        else:
+            _lib.check(self.lib.dronecu_rollout_policy_norm(self.batch._h, K, _ptr(self.params), int(deterministic), C.byref(out),
+                                                            nz.affine_ptr(), int(use_tc), st), "dronecu_rollout_policy_norm")
+            self.launches += nz.process_rollout(b.obs_store, b.reward, b.done, K, self._allreduce_f64 if self.world > 1 else None,
+                                                self.side_env, self.side_obs)
+        if nz is None and self.side_obs is not None:
+            self.side_obs.copy_(b.obs[:, self.side_env])
         _lib.check(self.lib.dronecu_gae(self.device.index, K, n, _ptr(b.reward), _ptr(b.value), _ptr(b.done),
                                         _ptr(b.last_value), self.gamma, self.gae_lambda, _ptr(b.adv), _ptr(b.ret), st),
                    "dronecu_gae")
@@ -464,7 +522,10 @@ class PPO:
         """SB3 ``predict``: numpy obs [15] or [n,15] -> (clipped action, None)  (train.py:48, test.py:14)."""
         obs = np.asarray(observation, dtype=np.float32)
         single = obs.ndim == 1
-        mean, _ = self.policy_forward(torch.from_numpy(obs.reshape(-1, 15)))
+        x = torch.from_numpy(obs.reshape(-1, 15))
+        if self.normalizer is not None:        # the model owns the VecNormalize statistics (SB3: the wrapped env applies them)
+            x = self.normalizer.normalize_obs(x)
+        mean, _ = self.policy_forward(x)
         if not deterministic:
             std = torch.exp(self.params[-4:])
             mean = mean + std * torch.randn(mean.shape, device=self.device, generator=self._gen)
@@ -481,7 +542,9 @@ class PPO:
                 "num_timesteps": self.num_timesteps, "n_updates": self.n_updates, "epochs_done": self._epochs_done,
                 "env_state": self.batch.get_state(), "env_global_step": self.batch.global_step,
                 "env_offset": int(self.batch.env_offset), "world": self.world,
-                "sb3_policy": {SB3_NAMES[k]: v.clone() for k, v in unpack_params(self.params.cpu()).items()}}
+                "sb3_policy": {SB3_NAMES[k]: v.clone() for k, v in unpack_params(self.params.cpu()).items()},
+                **({} if self.normalizer is None else {"normalizer": self.normalizer.state_dict(),
+                                                       "norm_returns": self.normalizer.returns.cpu().clone()})}
 
     def load_state_dict(self, sd: dict, load_env: bool = True):
         self.params.copy_(sd["params"].to(self.device))
@@ -499,6 +562,10 @@ class PPO:
             self.batch.set_state(**sd["env_state"])
             self.batch.global_step = sd.get("env_global_step", self.batch.global_step)
             self.env_state_restored = True
+            if self.normalizer is not None and "norm_returns" in sd:      # per-env returns: same shard only
+                self.normalizer.returns.copy_(sd["norm_returns"].to(self.device))
+        if self.normalizer is not None and "normalizer" in sd:
+            self.normalizer.load_state_dict(sd["normalizer"])
 
     def save(self, path: str):
         """SB3 ``model.save(path)`` (train.py:70): no suffix -> ``path + ".zip"``, an archive in SB3's layout
@@ -512,16 +579,24 @@ class PPO:
             # data parallel: policy and Adam state are replicas (rank 0's archive holds them); the env / curriculum /
             # Philox state differs per shard -> every other rank writes its shard next to the archive
             base = path[:-4] if path.endswith(".zip") else path
-            torch.save({k: sd[k] for k in ("env_state", "env_global_step", "env_offset", "world")}, f"{base}.env.rank{self.rank}.pt")
+            torch.save({k: sd[k] for k in ("env_state", "env_global_step", "env_offset", "world", "norm_returns") if k in sd},
+                       f"{base}.env.rank{self.rank}.pt")
             return
         hyper = {"n_steps": self.n_steps, "batch_size": self.batch_size, "n_epochs": self.n_epochs, "gamma": self.gamma,
                  "gae_lambda": self.gae_lambda, "learning_rate": float(self.cfg.learning_rate),
                  "clip_range": float(self.cfg.clip_range), "ent_coef": float(self.cfg.ent_coef),
                  "vf_coef": float(self.cfg.vf_coef), "max_grad_norm": float(self.cfg.max_grad_norm),
                  "n_envs": self.n_envs, "num_timesteps": self.num_timesteps, "_n_updates": self.n_updates, "seed": self.seed}
-        extra = {k: sd[k] for k in ("num_timesteps", "n_updates", "epochs_done", "env_state", "env_global_step", "env_offset", "world")}
+        extra = {k: sd[k] for k in ("num_timesteps", "n_updates", "epochs_done", "env_state", "env_global_step", "env_offset", "world",
+                                    "normalizer", "norm_returns") if k in sd}
         sb3_zip.export_zip(path if path.endswith(".zip") else path + ".zip", sd["params"], sd["adam"], sd["adam_step"],
                            hyper, extra)
+
+    @staticmethod
+    def _norm_settings(sd: dict, kw: dict) -> dict:
+        """A checkpoint trained with normalisation turns it on (with its clip / epsilon) unless the caller says otherwise."""
+        saved = sd.get("normalizer")
+        return kw if not saved else {**{k: saved[k] for k in ("norm_obs", "norm_reward", "clip_obs", "clip_reward", "norm_epsilon")}, **kw}
 
     @classmethod
     def load(cls, path: str, env=1, **kw):
@@ -532,8 +607,9 @@ class PPO:
         if not path.endswith((".pt", ".zip")) and os.path.isfile(path + ".zip"):
             path = path + ".zip"
         if path.endswith(".pt"):
-            model = cls(env, **kw)
-            model.load_state_dict(torch.load(path, weights_only=False))
+            sd = torch.load(path, weights_only=False)
+            model = cls(env, **cls._norm_settings(sd, kw))
+            model.load_state_dict(sd)
             return model
         from . import sb3_zip
         z = sb3_zip.import_zip(path)
@@ -541,7 +617,7 @@ class PPO:
                   "vf_coef", "max_grad_norm"):
             if k in z["hyper"] and k not in kw and isinstance(z["hyper"][k], (int, float)):
                 kw[k] = z["hyper"][k]
-        model = cls(env, **kw)
+        model = cls(env, **cls._norm_settings(z["extra"] or {}, kw))
         sd = {"params": z["params"], "adam": z["adam"] if z["adam"] is not None else torch.zeros(2 * POLICY_PARAMS),
               "adam_step": z["adam_step"], "num_timesteps": int(z["hyper"].get("num_timesteps", 0) or 0),
               "n_updates": int(z["hyper"].get("_n_updates", 0) or 0)}
@@ -550,6 +626,7 @@ class PPO:
         if model.world > 1 and model.rank > 0:          # this rank's env shard, written by save() next to the archive
             side = f"{path[:-4]}.env.rank{model.rank}.pt"
             sd.pop("env_state", None)
+            sd.pop("norm_returns", None)
             if os.path.isfile(side):
                 sd.update(torch.load(side, weights_only=False))
         model.load_state_dict(sd)

@@ -91,7 +91,10 @@ class TrajectoryCallback:
         self.blocks_written = 0
 
     def __call__(self, model) -> bool:
-        pos = model.buf.obs[:, self.env_index, 0:3].cpu().numpy()          # position BEFORE step t (drone.py:77-79)
+        # position BEFORE step t (drone.py:77-79); with norm_obs the buffer is normalised and the raw rows come from the tap
+        tap = getattr(model, "side_obs", None)
+        rows = tap if tap is not None and model.side_env == self.env_index else model.buf.obs[:, self.env_index]
+        pos = rows[:, 0:3].cpu().numpy()
         done = model.buf.done[:, self.env_index].cpu().numpy().astype(bool)
         for t in range(pos.shape[0]):
             self.positions.append(pos[t])
@@ -150,6 +153,9 @@ def main(argv=None):
     ap.add_argument("--update-precision", default=None, choices=["fp32", "tf32", "bf16"],
                     help="minibatch gradient: fp32 CUDA cores, tcgen05 all-tf32, or tcgen05 with bf16 weight-gradient operands "
                          "(default: fp32 with --precision fp32, bf16 with --precision tf32)")
+    ap.add_argument("--norm-obs", action="store_true", help="normalise observations (SB3 VecNormalize norm_obs) in the rollout")
+    ap.add_argument("--norm-reward", action="store_true", help="normalise rewards by the running std of the discounted return")
+    ap.add_argument("--clip-obs", type=float, default=10.0, help="clip of the normalised observations")
     ap.add_argument("--tensorboard-root", default="./tensorboard")
     ap.add_argument("--save", default="ppo_drone_rel_obs_pos_reward")
     ap.add_argument("--quiet", action="store_true")
@@ -171,6 +177,8 @@ def main(argv=None):
     kw = dict(n_steps=n_steps, batch_size=args.batch_size, learning_rate=args.learning_rate, n_epochs=args.n_epochs,
               seed=args.seed, rollout_precision=args.precision,
               update_precision=args.update_precision or ("bf16" if args.precision == "tf32" else "fp32"))
+    if args.norm_obs or args.norm_reward:       # else: PPO.load takes the archive's own settings
+        kw.update(norm_obs=args.norm_obs, norm_reward=args.norm_reward, clip_obs=args.clip_obs)
     if os.path.exists(args.resume):
         model = PPO.load(args.resume, env, **kw)
         if rank == 0:
@@ -191,6 +199,8 @@ def main(argv=None):
         run_dir = make_run_dir(args.tensorboard_root, prefix="drone_runs_")
         logger = RunLogger(run_dir, stdout=not args.quiet)
         cb = TrajectoryCallback(run_dir, tb=logger.tb)
+        if model.normalizer is not None and model.normalizer.norm_obs:
+            model.set_raw_obs_tap(cb.env_index)
 
     def on_iteration(m):
         if rank == 0:

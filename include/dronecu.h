@@ -235,6 +235,60 @@ int dronecu_policy_forward(int device, int64_t B, const float* d_params, const f
 int dronecu_gae(int device, int K, int64_t n, const float* d_reward, const float* d_value, const uint8_t* d_done,
                 const float* d_last_value, float gamma, float lam, float* d_advantage, float* d_returns, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Observation and reward normalisation (SB3 VecNormalize(norm_obs, norm_reward) inside the fused rollout; csrc/obs_norm.cuh,
+ * DESIGN.md section 9).  The running statistics are FROZEN for one rollout launch: rollout i normalises with the
+ * statistics as they stood after rollout i-1, then its moments are merged in one update (SB3 updates after every step).
+ * Per rollout, on one stream (nothing here synchronises; every call can be captured in a CUDA graph):
+ *   dronecu_rollout_policy_norm(..., d_affine)   towers see the normalised rows, the buffer receives the raw rows
+ *   dronecu_norm_pass                            buffer rows -> normalised in place, rewards -> normalised, moments
+ *   dronecu_norm_reduce                          CTA partials -> one moment record (fixed order: bit-reproducible)
+ *   [data parallel: sum the DRONECU_NORM_MOMENTS doubles over the ranks, e.g. dronecu_ppo_dp_allreduce_f64]
+ *   dronecu_norm_combine                         parallel-variance update of the statistics, next affine record
+ * Layouts (device memory):
+ *   affine  float32 [31]: mean_f[15] | rstd_f[15] | clip_obs;  x_norm = min(max((x - mean_f) * rstd_f, -clip), clip) with
+ *           a round-to-nearest subtract and multiply (no FMA), rstd_f = (float)(1 / sqrt(var + epsilon))
+ *   stats   float64 [34]: obs_mean[15] | obs_var[15] | obs_count | ret_mean | ret_var | ret_count  (SB3 RunningMeanStd;
+ *           initial state mean 0, var 1, count 1e-4)
+ *   moments float64 [34]: sum(x - c)[15] | sum((x - c)^2)[15] | obs count | sum(ret - c_r) | sum((ret - c_r)^2) | return
+ *           count, where c, c_r are the running means the pass read (a shift, so that features far from zero do not cancel)
+ * ---------------------------------------------------------------------------------------------- */
+#define DRONECU_NORM_AFFINE 31
+#define DRONECU_NORM_STATS 34
+#define DRONECU_NORM_MOMENTS 34
+#define DRONECU_NORM_BLOCK 256 /* envs per CTA of dronecu_norm_pass: ceil(n / 256) partial records */
+
+/* dronecu_rollout_policy (tensor_cores == 0) or dronecu_rollout_policy_tc (!= 0) whose towers see every observation, and
+ * the bootstrap observation, normalised with d_norm_affine [DRONECU_NORM_AFFINE].  out->d_obs / d_last_obs still receive
+ * the RAW rows.  d_norm_affine == NULL: exactly dronecu_rollout_policy / _tc (same kernels, same results). */
+int dronecu_rollout_policy_norm(dronecu_env* env, int K, const float* d_params, int deterministic,
+                                const dronecu_policy_out* out, const float* d_norm_affine, int tensor_cores, void* stream);
+
+/* One thread per env walks its K steps of the step-major buffers [K,n,...]. */
+typedef struct dronecu_norm_pass_args {
+  float* d_obs;             /* [K,n,obs_stride] raw rows, rewritten normalised; NULL: observations untouched, no obs moments */
+  int32_t obs_stride;       /* 15 or 16 (64-byte rows: the 16th value is kept, 1.0)                                         */
+  int32_t K;
+  int64_t n;
+  const float* d_affine;    /* [31] the record the rollout used (required with d_obs)                                       */
+  float* d_reward;          /* [K,n] raw in, out clip(r / sqrt(ret_var + epsilon), +-clip_reward) (float64, then cast); NULL: off */
+  const uint8_t* d_done;    /* [K,n] the per-env return restarts after done                                                 */
+  double* d_returns;        /* [n] per-env discounted return ret = ret * gamma + r, persistent across rollouts                */
+  const double* d_stats;    /* [34] running statistics (moment shift, reward scale)                                         */
+  double gamma, epsilon, clip_reward;
+  int32_t update;           /* != 0 (training): returns advance, d_partials written; 0 (evaluation): statistics untouched   */
+  int32_t side_env;         /* >= 0 with d_side_obs: copy that env's raw rows to d_side_obs [K,15] before normalising       */
+  float* d_side_obs;
+  double* d_partials;       /* [ceil(n / DRONECU_NORM_BLOCK), DRONECU_NORM_MOMENTS] scratch, one record per CTA (update != 0) */
+} dronecu_norm_pass_args;
+int dronecu_norm_pass(int device, const dronecu_norm_pass_args* args, void* stream);
+/* d_moments [34] = fixed-order sum of the n_partials records of dronecu_norm_pass (written, not accumulated). */
+int dronecu_norm_reduce(int device, const double* d_partials, int64_t n_partials, double* d_moments, void* stream);
+/* d_moments != NULL: merge the batch into d_stats (SB3 RunningMeanStd.update_from_moments, float64; a part whose count is 0
+ * is skipped).  Then, d_affine != NULL: write the affine record of d_stats (clip = clip_obs). */
+int dronecu_norm_combine(int device, double* d_stats, const double* d_moments, double epsilon, float clip_obs, float* d_affine,
+                         void* stream);
+
 typedef struct dronecu_ppo_config {
   float learning_rate; /* 3e-4  */
   float beta1, beta2;  /* 0.9, 0.999 */
