@@ -44,7 +44,7 @@ struct UpdArgs {
   const int32_t* index;      // [m] rows of this minibatch (nullptr: rows first .. first+m)
   int64_t first, m;
   float adv_mean, adv_inv_std;   // (adv - mean) * inv_std ; (0, 1) disables normalisation
-  const double* adv_stats;       // nullable: [sum, sum of squares, count] -> overrides the two scalars
+  const double* adv_stats;       // nullable: [sum, sum of squares, count] -> overrides the two scalars (count <= 1: (0, 1))
   float clip, vf_coef, ent_coef;
   float* partials;           // [gridDim.x, kGradLen]
   float* direct;             // ppo_grad_bf16_kernel with ONE CTA per tower: the gradient vector itself (no reduce launch); else nullptr
@@ -250,11 +250,14 @@ __global__ void __launch_bounds__(kUpdBlock, 1) ppo_grad_kernel(const __grid_con
 #pragma unroll
   for (int o = 0; o < kAct; ++o) { std_inv[o] = expf(-U.fwd.log_std[o]); logstd_sum += U.fwd.log_std[o]; }
   float adv_mean = A.adv_mean, adv_inv_std = A.adv_inv_std;
-  if (A.adv_stats != nullptr) {        // SB3: (adv - adv.mean()) / (adv.std() + 1e-8), torch.std is unbiased
+  if (A.adv_stats != nullptr && A.adv_stats[2] > 1.0) {   // SB3: (adv - adv.mean()) / (adv.std() + 1e-8), torch.std is unbiased
     const double cnt = A.adv_stats[2], mu = A.adv_stats[0] / cnt;
     const double var = (A.adv_stats[1] - A.adv_stats[0] * mu) / (cnt - 1.0);
     adv_mean = (float)mu;
     adv_inv_std = (float)(1.0 / (sqrt(fmax(var, 0.0)) + 1e-8));
+  } else if (A.adv_stats != nullptr) {   // SB3 normalises only `if len(advantages) > 1`: one sample keeps its raw advantage
+    adv_mean = 0.f;
+    adv_inv_std = 1.f;
   }
 
   const int64_t n_tiles = (A.m + kUpdBlock - 1) / kUpdBlock;

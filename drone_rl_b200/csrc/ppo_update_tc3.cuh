@@ -371,11 +371,14 @@ __global__ void __launch_bounds__(tcb::kThreads3, 1) ppo_grad_bf16_kernel(const 
 #pragma unroll
     for (int o = 0; o < kAct; ++o) { std_inv[o] = expf(-S.log_std[o]); logstd_sum += S.log_std[o]; }
     float adv_mean = A.adv_mean, adv_inv_std = A.adv_inv_std;
-    if (A.adv_stats != nullptr) {        // SB3: (adv - adv.mean()) / (adv.std() + 1e-8), torch.std is unbiased
+    if (A.adv_stats != nullptr && A.adv_stats[2] > 1.0) {   // SB3: (adv - adv.mean()) / (adv.std() + 1e-8), torch.std is unbiased
       const double cnt = A.adv_stats[2], mu = A.adv_stats[0] / cnt;
       const double var = (A.adv_stats[1] - A.adv_stats[0] * mu) / (cnt - 1.0);
       adv_mean = (float)mu;
       adv_inv_std = (float)(1.0 / (sqrt(fmax(var, 0.0)) + 1e-8));
+    } else if (A.adv_stats != nullptr) {   // SB3 normalises only `if len(advantages) > 1`: one sample keeps its raw advantage
+      adv_mean = 0.f;
+      adv_inv_std = 1.f;
     }
 
     unsigned char* const rowA = S.bufA[wg] + r * 16;       // + g * kGrp: this sample's 16 bytes of feature group g

@@ -338,7 +338,9 @@ int dronecu_ppo_adv_stats_epoch(dronecu_ppo* ppo, const float* d_adv, const int3
  * the sums of: policy loss, squared value error, approx_kl, clip fraction, sample count.  Advantages
  * enter as (adv - adv_mean) * adv_inv_std; when d_adv_stats (the [sum, sumsq, count] written by
  * dronecu_ppo_adv_stats) is not NULL, mean and 1/(unbiased std + 1e-8) are formed from it on the
- * device instead -- no host round trip.  Deterministic for a fixed launch configuration. */
+ * device instead -- no host round trip; with a count of 1 or less the raw advantages are used (SB3
+ * normalises only a minibatch of more than one sample; the count is global over data-parallel ranks).
+ * Deterministic for a fixed launch configuration. */
 int dronecu_ppo_grad(dronecu_ppo* ppo, const float* d_params, const float* d_obs, const float* d_actions,
                      const float* d_old_logp, const float* d_adv, const float* d_returns, const int32_t* d_index,
                      int64_t first, int64_t m, float adv_mean, float adv_inv_std, const double* d_adv_stats,

@@ -14,7 +14,8 @@ Restated pieces
   * GAE(gamma=0.99, lambda=0.95) with SB3's episode_start convention, no bootstrap on time-outs
     (the reference env never sets "TimeLimit.truncated").
   * the clipped-surrogate loss with per-minibatch advantage normalisation (std + 1e-8, unbiased
-    std as torch.std), value MSE x 0.5, entropy x 0, global-norm clip 0.5, Adam(3e-4, eps 1e-5).
+    std as torch.std; skipped for a minibatch of one sample, as SB3's ``len(advantages) > 1``),
+    value MSE x 0.5, entropy x 0, global-norm clip 0.5, Adam(3e-4, eps 1e-5).
 
 Flat parameter layout (shared with drone_rl_b200/csrc/ppo_common.cuh), float32, 10697 values:
     pi.W1[64,15] pi.b1[64] pi.W2[64,64] pi.b2[64] pi.W3[4,64] pi.b3[4]
@@ -131,10 +132,11 @@ def gae(rewards, values, dones, last_values, gamma=0.99, lam=0.95):
 def ppo_loss(flat, obs, actions, old_logp, adv, returns, clip=0.2, vf_coef=0.5, ent_coef=0.0,
              normalize=True, adv_mean=None, adv_std=None):
     """SB3 PPO.train() loss for one minibatch.  adv_mean/adv_std override the per-minibatch
-    statistics (used for the data-parallel path, where they are global over the ranks)."""
+    statistics (used for the data-parallel path, where they are global over the ranks).  Without them a
+    minibatch of one sample keeps its raw advantage: SB3 normalises only ``if len(advantages) > 1``."""
     mean, value, log_std = forward(flat, obs)
     logp = log_prob(mean, log_std, actions)
-    if normalize:
+    if normalize and (adv_mean is not None or adv.numel() > 1):
         m = adv.mean() if adv_mean is None else adv_mean
         s = adv.std() if adv_std is None else adv_std          # torch.std: unbiased, as SB3
         adv = (adv - m) / (s + 1e-8)
@@ -174,11 +176,12 @@ def clip_and_adam(flat, grad, st: AdamState, lr=3e-4, b1=0.9, b2=0.999, eps=1e-5
     return flat - (lr / bc1) * st.m / denom, float(total)
 
 
-def minibatch_update(flat, st, batch, **kw):
-    """One optimiser step on one minibatch; returns (new flat params, stats)."""
+def minibatch_update(flat, st, batch, lr=3e-4, max_norm=0.5, **kw):
+    """One optimiser step on one minibatch; returns (new flat params, stats, gradient).  ``lr`` and ``max_norm``
+    go to clip_and_adam, every other keyword to ppo_loss."""
     p = flat.clone().requires_grad_(True)
     loss, stats = ppo_loss(p, *batch, **kw)
     (g,) = torch.autograd.grad(loss, p)
-    new, gnorm = clip_and_adam(flat, g, st)
+    new, gnorm = clip_and_adam(flat, g, st, lr=lr, max_norm=max_norm)
     stats["grad_norm"] = gnorm
     return new.detach(), stats, g.detach()

@@ -111,13 +111,15 @@ def _grad(model, index, m, first=0, tc=True):
     return model._grad.cpu().double().numpy().copy()
 
 
-def _separated_buffers(model, seed):
+def _separated_buffers(model, seed, clip=None):
     """Like tests/test_gpu_ppo._fake_buffers, but the old log-probs sit at offsets {-0.45, -0.08, 0, 0.07,
     0.4} (+- 0.01) from the current policy's: ratios of 1.57 / 1.08 / 1 / 0.93 / 0.67 exercise both sides
     of the clip, and no sample lies within the tf32 forward error of the 0.8 / 1.2 boundaries -- the clipped
     objective's gradient is discontinuous there, so a borderline sample would make ANY reduced-precision
     forward differ from float64 by that sample's whole gradient (measured with the unseparated buffers:
-    1-2 % of the samples flip, 5 % error on the policy blocks, value blocks unaffected)."""
+    1-2 % of the samples flip, 5 % error on the policy blocks, value blocks unaffected).
+    ``clip``: place the offsets around the boundaries log(1 -+ clip) of that clip range instead: 0.2 outside
+    each boundary, 0.45 of the way from 0 to each boundary, and 0."""
     b = model.buf
     K, n = b.obs.shape[0], b.obs.shape[1]
     g = torch.Generator().manual_seed(seed)
@@ -125,7 +127,11 @@ def _separated_buffers(model, seed):
     theta = model.params.cpu().double()
     mean, value, log_std = po.forward(theta, obs.double().reshape(-1, 15))
     act = mean + torch.exp(log_std) * torch.randn(K * n, 4, generator=g, dtype=torch.float64)
-    offs = torch.tensor([-0.45, -0.08, 0.0, 0.07, 0.4], dtype=torch.float64)[torch.randint(0, 5, (K * n,), generator=g)]
+    table = [-0.45, -0.08, 0.0, 0.07, 0.4]
+    if clip is not None:
+        lo, hi = np.log1p(-clip), np.log1p(clip)
+        table = [lo - 0.2, 0.45 * lo, 0.0, 0.45 * hi, hi + 0.2]
+    offs = torch.tensor(table, dtype=torch.float64)[torch.randint(0, 5, (K * n,), generator=g)]
     old_logp = po.log_prob(mean, log_std, act) + offs + 0.01 * torch.randn(K * n, generator=g, dtype=torch.float64)
     adv = torch.randn(K * n, generator=g, dtype=torch.float64) * 3 + 0.5
     # a biased value function: with ret - value pure noise the reference gradient is a sqrt(m)-sized noise sum

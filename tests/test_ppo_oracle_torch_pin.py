@@ -73,7 +73,8 @@ class TorchMlpPolicy(nn.Module):
 def sb3_loss(policy, obs, actions, old_logp, adv, returns, clip=0.2, vf_coef=0.5, ent_coef=0.0):
     """The body of SB3's PPO.train() minibatch loop, line for line in torch ops."""
     values, log_prob, entropy = policy.evaluate_actions(obs, actions)
-    adv = (adv - adv.mean()) / (adv.std() + 1e-8)
+    if len(adv) > 1:                                   # SB3: `if self.normalize_advantage and len(advantages) > 1`
+        adv = (adv - adv.mean()) / (adv.std() + 1e-8)
     ratio = torch.exp(log_prob - old_logp)
     policy_loss = -torch.min(adv * ratio, adv * torch.clamp(ratio, 1 - clip, 1 + clip)).mean()
     value_loss = torch.nn.functional.mse_loss(returns, values)
@@ -181,6 +182,56 @@ def test_clip_and_adam_equal_torch_optim_over_25_steps(dtype):
         tol = 1e-12 if dtype == torch.float64 else 2e-7
         assert torch.allclose(theta, p.detach(), rtol=0, atol=tol), f"step {k}: {float((theta - p.detach()).abs().max())}"
     assert 0 < clipped < 25
+
+
+def test_size_one_minibatch_keeps_the_raw_advantage():
+    """A minibatch of one sample (the ragged tail of n_envs * n_steps = 1 mod batch_size) is not normalised: SB3 skips it,
+    where torch.std of one element would be NaN.  Loss and gradient equal SB3's rule and the unnormalised loss; with global
+    statistics passed in (data parallel) the one sample is normalised with them."""
+    torch.manual_seed(13)
+    pol = TorchMlpPolicy().double()
+    with torch.no_grad():
+        for p in pol.parameters():
+            p.add_(0.1 * torch.randn(p.shape, dtype=torch.float64))
+    batch = _batch(1, 7, torch.float64)
+    assert abs(float(batch[3][0])) > 0.1                # a raw advantage far from 0, where normalising would zero it
+    loss_ref = sb3_loss(pol, *batch)
+    loss_ref.backward()
+    flat = pol.flat().clone().requires_grad_(True)
+    loss, stats = po.ppo_loss(flat, *batch)
+    (g,) = torch.autograd.grad(loss, flat)
+    assert torch.isfinite(g).all()
+    assert abs(float(loss.detach()) - float(loss_ref.detach())) <= 1e-12 * max(1.0, abs(float(loss_ref.detach())))
+    assert torch.allclose(g, pol.flat_grad(), rtol=1e-10, atol=1e-13)
+    loss_raw, _ = po.ppo_loss(flat, *batch, normalize=False)
+    assert float(loss.detach()) == float(loss_raw.detach())
+    pi = po.offsets()["pi.W3"][0]
+    assert float(g[pi:pi + 256].abs().max()) > 0          # the policy head moves (normalising one sample would zero it)
+    mu, sd = torch.tensor(0.25, dtype=torch.float64), torch.tensor(2.0, dtype=torch.float64)
+    loss_g, _ = po.ppo_loss(flat, *batch, adv_mean=mu, adv_std=sd)
+    loss_n, _ = po.ppo_loss(flat, *batch[:3], (batch[3] - mu) / (sd + 1e-8), batch[4], normalize=False)
+    assert float(loss_g.detach()) == float(loss_n.detach())
+
+
+def test_minibatch_update_passes_lr_and_max_norm():
+    """oracle.minibatch_update with non-default learning rate and clip norm == clip_grad_norm_(max_norm) + Adam(lr) over
+    nn.Modules, on both sides of the clip threshold."""
+    torch.manual_seed(22)
+    pol = TorchMlpPolicy().double()
+    opt = torch.optim.Adam(pol.parameters(), lr=1e-3, eps=1e-5)
+    theta, st = pol.flat().clone(), po.AdamState(po.N_PARAMS, torch.float64)
+    clipped = 0
+    for k in range(6):
+        batch = _batch(64, 200 + k, torch.float64)
+        opt.zero_grad()
+        sb3_loss(pol, *batch).backward()
+        total = nn.utils.clip_grad_norm_(pol.parameters(), 2.0)
+        clipped += float(total) > 2.0
+        opt.step()
+        theta, stats, _ = po.minibatch_update(theta, st, batch, lr=1e-3, max_norm=2.0)
+        assert abs(stats["grad_norm"] - float(total)) <= 1e-12 * float(total)
+        assert torch.allclose(theta, pol.flat(), rtol=0, atol=1e-12), f"step {k}"
+    assert 0 < clipped < 6
 
 
 def test_minibatch_updates_equal_torch_training_loop():
