@@ -74,6 +74,14 @@ class NormPassArgs(C.Structure):
                 ("update", C.c_int32), ("side_env", C.c_int32), ("d_side_obs", C.c_void_p), ("d_partials", C.c_void_p)]
 
 
+class EvalArgs(C.Structure):
+    """Mirror of ``dronecu_eval_args`` (include/dronecu.h)."""
+    _fields_ = [("t0", C.c_int64), ("limit", C.c_int32), ("catch_up", C.c_int32), ("deterministic", C.c_int32),
+                ("max_eps", C.c_int32), ("env_index0", C.c_int64), ("n_global", C.c_int64), ("n_eval_episodes", C.c_int64),
+                ("d_steps", C.c_void_p), ("d_count", C.c_void_p), ("d_ep_return", C.c_void_p), ("d_ep_length", C.c_void_p),
+                ("d_pending", C.c_void_p)]
+
+
 NORM_AFFINE = 31
 NORM_STATS = 34
 NORM_MOMENTS = 34
@@ -121,6 +129,7 @@ _SIGNATURES = {
     "dronecu_rollout_policy_tc": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(PolicyOut), _P]),
     "dronecu_policy_forward_tc": (C.c_int, [C.c_int, C.c_int64, _P, _P, _P, _P, _P, _P, _P]),
     "dronecu_rollout_policy_norm": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(PolicyOut), _P, C.c_int, _P]),
+    "dronecu_evaluate_policy": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(EvalArgs), _P]),
     "dronecu_norm_pass": (C.c_int, [C.c_int, C.POINTER(NormPassArgs), _P]),
     "dronecu_norm_reduce": (C.c_int, [C.c_int, _P, C.c_int64, _P, _P]),
     "dronecu_norm_combine": (C.c_int, [C.c_int, _P, _P, C.c_double, C.c_float, _P, _P]),

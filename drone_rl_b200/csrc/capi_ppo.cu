@@ -12,6 +12,7 @@
 #include "env_handle.h"
 #include "ppo_update.cuh"
 #include "ppo_rollout_tc.cuh"
+#include "ppo_eval.cuh"
 #include "ppo_update_tc.cuh"
 #include "ppo_update_tc3.cuh"
 #include "ppo_dp.cuh"
@@ -123,6 +124,58 @@ extern "C" int dronecu_rollout_policy_norm(dronecu_env* e, int K, const float* d
                                            const dronecu_policy_out* out, const float* d_norm_affine, int tensor_cores,
                                            void* stream) {
   return rollout_policy_impl(e, K, d_params, deterministic, out, stream, tensor_cores != 0, d_norm_affine);
+}
+
+// ------------------------------------------------------------------------------------------------
+// policy evaluation (csrc/ppo_eval.cuh)
+// ------------------------------------------------------------------------------------------------
+template <bool RANDOMIZED, bool NORM>
+static int launch_policy_eval(RolloutKernel which, int64_t n, const EvalArgs& a, cudaStream_t st) {
+  if (which == kTensorCores) {
+    CUDA_TRY(cudaFuncSetAttribute(policy_eval_tc_kernel<RANDOMIZED, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(tc::Smem)));
+    policy_eval_tc_kernel<RANDOMIZED, NORM><<<(unsigned)((n + tc::kTile - 1) / tc::kTile), tc::kTile, sizeof(tc::Smem), st>>>(a);
+  } else if (which == kWarpPerEnv) {
+    CUDA_TRY(cudaFuncSetAttribute(policy_eval_warp_kernel<RANDOMIZED, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmallSmem));
+    policy_eval_warp_kernel<RANDOMIZED, NORM><<<(unsigned)((n + kSmallWarps - 1) / kSmallWarps), 32 * kSmallWarps, kPolicySmallSmem, st>>>(a);
+  } else {
+    CUDA_TRY(cudaFuncSetAttribute(policy_eval_kernel<RANDOMIZED, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(MlpSmem)));
+    policy_eval_kernel<RANDOMIZED, NORM><<<(unsigned)((n + kPolBlock - 1) / kPolBlock), kPolBlock, sizeof(MlpSmem), st>>>(a);
+  }
+  return DRONECU_OK;
+}
+
+extern "C" int dronecu_evaluate_policy(dronecu_env* e, const float* d_params, const float* d_norm_affine, int tensor_cores,
+                                       const dronecu_eval_args* p, void* stream) {
+  if (!e || !d_params || !p) return fail(DRONECU_ERR_INVALID, "dronecu_evaluate_policy: null argument");
+  if (e->cfg.obs_dim != 15 || !(e->cfg.flags & DRONECU_AUTORESET))
+    return fail(DRONECU_ERR_UNSUPPORTED, "policy evaluation needs the 15-dim observation and DRONECU_AUTORESET");
+  if (!p->d_steps || !p->d_count || !p->d_ep_return || !p->d_ep_length || (!p->catch_up && !p->d_pending))
+    return fail(DRONECU_ERR_INVALID, "dronecu_evaluate_policy: d_steps, d_count, d_ep_return, d_ep_length and (probe) d_pending are required");
+  if (p->t0 < 0 || p->limit < 0 || p->n_eval_episodes < 1 || p->env_index0 < 0 || p->n_global < e->n ||
+      p->env_index0 > p->n_global - e->n)
+    return fail(DRONECU_ERR_INVALID, "dronecu_evaluate_policy: need t0 >= 0, limit >= 0, n_eval_episodes >= 1 and "
+                                     "0 <= env_index0 <= n_global - n");
+  if ((int64_t)p->max_eps < (p->n_eval_episodes + p->n_global - 1) / p->n_global)
+    return fail(DRONECU_ERR_INVALID, "dronecu_evaluate_policy: max_eps is below ceil(n_eval_episodes / n_global)");
+  DeviceGuard guard(e->device);
+  EvalArgs a;
+  std::memset(&a, 0, sizeof(a));
+  a.state = e->sp; a.P = e->P; a.n = e->n; a.t0 = (uint64_t)p->t0; a.limit = p->limit; a.catch_up = p->catch_up ? 1 : 0;
+  a.deterministic = p->deterministic; a.max_eps = p->max_eps; a.env_index0 = p->env_index0; a.n_global = p->n_global;
+  a.n_eval_episodes = p->n_eval_episodes; a.theta = d_params; a.norm = d_norm_affine;
+  a.steps = p->d_steps; a.count = p->d_count; a.ep_return = p->d_ep_return; a.ep_length = p->d_ep_length; a.pending = p->d_pending;
+  // the kernel choice of rollout_policy_impl
+  const RolloutKernel which = tensor_cores ? kTensorCores
+      : (g_rollout_kernel_mode == 2 || (g_rollout_kernel_mode == 0 && e->n <= kWarpRolloutMaxEnvs)) ? kWarpPerEnv : kThreadPerEnv;
+  cudaStream_t st = (cudaStream_t)stream;
+  const bool randomized = (e->cfg.flags & DRONECU_RANDOMIZED) != 0;
+  int rc;
+  if (d_norm_affine) rc = randomized ? launch_policy_eval<true, true>(which, e->n, a, st) : launch_policy_eval<false, true>(which, e->n, a, st);
+  else rc = randomized ? launch_policy_eval<true, false>(which, e->n, a, st) : launch_policy_eval<false, false>(which, e->n, a, st);
+  if (rc != DRONECU_OK) return rc;
+  e->launches += 1;
+  CUDA_TRY(cudaGetLastError());
+  return DRONECU_OK;
 }
 
 // ------------------------------------------------------------------------------------------------

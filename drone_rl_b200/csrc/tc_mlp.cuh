@@ -331,6 +331,15 @@ __device__ __forceinline__ void forward(Smem& S, const float (&x)[kObs], uint32_
   value = v1[0];
 }
 
+// policy tower only (evaluation: ppo_eval.cuh); the same MMAs on the same operands as the pi tower of forward()
+__device__ __forceinline__ void forward_policy(Smem& S, const float (&x)[kObs], uint32_t& phase, float (&mean)[kAct]) {
+  float xv[16];
+#pragma unroll
+  for (int i = 0; i < kObs; ++i) xv[i] = to_tf32_fast(x[i]);
+  xv[15] = 1.0f;
+  tower<kAct>(S, 0, xv, phase, mean, nullptr, nullptr);
+}
+
 // value tower only (the GAE bootstrap after the last step)
 __device__ __forceinline__ float forward_value(Smem& S, const float (&x)[kObs], uint32_t& phase) {
   float xv[16], v1[1];

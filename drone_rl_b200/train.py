@@ -56,6 +56,16 @@ class RunLogger:
             self.keys = list(values)
             with open(self.csv_path, "w", newline="") as f:
                 csv.writer(f).writerow(["step"] + self.keys)
+        elif any(k not in self.keys for k in values):
+            # keys that first appear now (eval/* after the first evaluation): rewrite the header with the extended key set
+            # and pad the earlier rows, as SB3's CSV writer does
+            self.keys += [k for k in values if k not in self.keys]
+            with open(self.csv_path, newline="") as f:
+                old = list(csv.reader(f))[1:]
+            with open(self.csv_path, "w", newline="") as f:
+                w = csv.writer(f)
+                w.writerow(["step"] + self.keys)
+                w.writerows(row + [""] * (len(self.keys) + 1 - len(row)) for row in old)
         with open(self.csv_path, "a", newline="") as f:
             csv.writer(f).writerow([step] + [values.get(k, "") for k in self.keys])
         self.tb.add_scalars(values, step)
@@ -156,6 +166,11 @@ def main(argv=None):
     ap.add_argument("--norm-obs", action="store_true", help="normalise observations (SB3 VecNormalize norm_obs) in the rollout")
     ap.add_argument("--norm-reward", action="store_true", help="normalise rewards by the running std of the discounted return")
     ap.add_argument("--clip-obs", type=float, default=10.0, help="clip of the normalised observations")
+    ap.add_argument("--eval-freq", type=int, default=0,
+                    help="evaluate the policy every this many vec-env steps (SB3 EvalCallback; 0 = no evaluation)")
+    ap.add_argument("--n-eval-episodes", type=int, default=5)
+    ap.add_argument("--n-eval-envs", type=int, default=1, help="evaluation envs per GPU")
+    ap.add_argument("--eval-stochastic", action="store_true", help="evaluate with sampled actions instead of the mean")
     ap.add_argument("--tensorboard-root", default="./tensorboard")
     ap.add_argument("--save", default="ppo_drone_rel_obs_pos_reward")
     ap.add_argument("--quiet", action="store_true")
@@ -202,10 +217,26 @@ def main(argv=None):
         if model.normalizer is not None and model.normalizer.norm_obs:
             model.set_raw_obs_tap(cb.env_index)
 
+    eval_cb = None
+    if args.eval_freq > 0:
+        from .evaluation import EvalCallback
+        run_dirs = [logger.run_dir if rank == 0 else None]
+        if world > 1:
+            dist.broadcast_object_list(run_dirs, src=0)
+        eval_env = DroneBatch(args.n_eval_envs, EnvConfig.single(), device=local, seed=args.seed + 1,
+                              env_offset=rank * args.n_eval_envs)
+        eval_cb = EvalCallback(eval_env, n_eval_episodes=args.n_eval_episodes, eval_freq=args.eval_freq,
+                               deterministic=not args.eval_stochastic, log_path=run_dirs[0], best_model_save_path=run_dirs[0],
+                               verbose=int(rank == 0 and not args.quiet))
+
     def on_iteration(m):
+        if eval_cb is not None:
+            eval_cb(m)
         if rank == 0:
             cb(m)
             logger.dump(dict(m.logger_values), m.num_timesteps)
+        for k in [k for k in m.logger_values if k.startswith("eval/")]:      # SB3 records them for the evaluation's row only
+            del m.logger_values[k]
         return True
 
     # SB3 semantics (reset_num_timesteps=True): total_timesteps MORE steps, also after a resume (train.py:22-30, :63-68)

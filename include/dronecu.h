@@ -289,6 +289,37 @@ int dronecu_norm_reduce(int device, const double* d_partials, int64_t n_partials
 int dronecu_norm_combine(int device, double* d_stats, const double* d_moments, double epsilon, float clip_obs, float* d_affine,
                          void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Policy evaluation: SB3 evaluate_policy(model, VecMonitor(DummyVecEnv([DroneGymEnv] * N)), n_eval_episodes, deterministic)
+ * with the actor alone (csrc/ppo_eval.cuh, DESIGN.md section 10).  Env g (global index among the N = n_global evaluation envs)
+ * records target_g = (n_eval_episodes + g) / N episodes; all envs step in lockstep until every env has reached its target,
+ * T steps in all.  Step c of an env uses the noise index t0 + c, as dronecu_rollout_policy does.  The caller resets the envs
+ * first, then issues probe launches (each env runs until its target or step `limit`; *d_pending counts the envs still
+ * below target) until no env is pending, then ONE catch-up launch with limit = T = max(d_steps): every env has then been
+ * stepped exactly T times.  The env clock (dronecu_global_step) is not advanced: the caller sets it to t0 + T.
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct dronecu_eval_args {
+  int64_t t0;              /* env clock at the first step of the evaluation                                          */
+  int32_t limit;           /* probe: run up to this step (absolute, counted from the reset); catch-up: T              */
+  int32_t catch_up;        /* 0 = probe, 1 = catch-up                                                               */
+  int32_t deterministic;   /* != 0: action = clip(mean); else clip(mean + std * z), z from the rollout's noise stream */
+  int32_t max_eps;         /* row stride of d_ep_return / d_ep_length: >= ceil(n_eval_episodes / n_global)           */
+  int64_t env_index0;      /* global index of this handle's env 0 among the n_global evaluation envs                  */
+  int64_t n_global;
+  int64_t n_eval_episodes; /* >= 1                                                                                   */
+  int32_t* d_steps;        /* [n] steps taken since the reset (zero before the first launch), updated                 */
+  int32_t* d_count;        /* [n] episodes recorded (zero before the first launch), updated                           */
+  float* d_ep_return;      /* [n, max_eps] VecMonitor return of each recorded episode (float32, raw reward)           */
+  int32_t* d_ep_length;    /* [n, max_eps] its length                                                               */
+  int32_t* d_pending;      /* probe: += number of envs still below their target (zero it first)                       */
+} dronecu_eval_args;
+
+/* One launch (probe or catch-up).  d_norm_affine != NULL: the policy sees observations normalised with that record
+ * (nothing is updated).  tensor_cores != 0: the tcgen05 kernel (tf32), else the float32 kernel dronecu_set_rollout_kernel
+ * selects for dronecu_rollout_policy.  Needs the 15-dim observation and DRONECU_AUTORESET. */
+int dronecu_evaluate_policy(dronecu_env* env, const float* d_params, const float* d_norm_affine, int tensor_cores,
+                            const dronecu_eval_args* args, void* stream);
+
 typedef struct dronecu_ppo_config {
   float learning_rate; /* 3e-4  */
   float beta1, beta2;  /* 0.9, 0.999 */
