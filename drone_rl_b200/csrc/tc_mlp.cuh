@@ -15,7 +15,12 @@
 // latency of the others (round-1 ncu: the 256-column, both-towers-at-once variant left the SM at 40 %
 // issue utilisation with 8 resident warps).
 // Precision: tf32 products (10-bit mantissa), fp32 accumulation, tanh.approx.f32 (2^-11): outputs agree
-// with the fp32 CUDA-core path to ~2e-3; that path stays the parity reference (tests/test_gpu_ppo.py).
+// with the fp32 CUDA-core path to ~2e-3; that path stays the parity reference (tests/test_gpu_ppo.py).  The
+// per-element bound is derived in oracle/tc_bound.py.
+// Non-finite rows: +-inf, and values that round to inf in tf32, behave as in float32 torch (the first tanh
+// saturates).  A row holding NaN gives an unspecified, possibly finite, output: tanh.approx returns the canonical
+// NaN 0x7fffffff, which to_tf32_fast wraps to -0, so the NaN does not reach layer 2 (the fp32 path returns NaN).
+// The env can emit such rows (body rates that overflow never end the episode: the crash test looks at the position).
 #pragma once
 #include "ppo_common.cuh"
 

@@ -23,7 +23,9 @@ def check_rollout(obs0, actions, next_obs, reward, done, *, spec=do.SINGLE, seed
 
     ep_num0 / step0: episode number (default 2: constructor reset + reset()) and step counter
     (default 0) of every env before the first step.
-    Returns a dict with the worst error/bound ratio and the counts of borderline decisions.
+    Returns a dict with the worst error/bound ratio and the counts of borderline decisions; "terminated" counts the
+    recorded dones the oracle calls a crash (at the time limit too) away from the crash borderline, and
+    "terminated_slack" the recorded dones on the borderline, whose crash flag is not decided here.
     Raises AssertionError on a violation.
     """
     K, n = actions.shape[:2]
@@ -32,7 +34,7 @@ def check_rollout(obs0, actions, next_obs, reward, done, *, spec=do.SINGLE, seed
     ep_num = np.broadcast_to(np.asarray(2 if ep_num0 is None else ep_num0, dtype=np.int64), (n,)).copy()
     step = np.zeros(n, dtype=np.int64) if step0 is None else np.broadcast_to(np.asarray(step0, dtype=np.int64), (n,)).copy()
     prev = np.asarray(obs0, dtype=np.float32)
-    worst, borderline, n_done, n_sing = 0.0, 0, 0, 0
+    worst, borderline, n_done, n_sing, n_term, term_slack = 0.0, 0, 0, 0, 0, 0
     # the tolerance has a unit floor (1e-5 * max(|ref|, 1)); to make the floor visible also track the worst PURE relative
     # error |got - ref| / |ref| -- over all finite non-zero reference entries outside the near-singular rows, and over those
     # with |ref| >= 1e-3 (below that the quantity is a difference of O(1) terms and its relative error is cancellation)
@@ -52,6 +54,8 @@ def check_rollout(obs0, actions, next_obs, reward, done, *, spec=do.SINGLE, seed
             margin = ((np.abs(npos[:, 2]) > 1e-5) & (np.abs(rad - 50.0) > 1e-4)) | ~np.isfinite(rad)
             assert np.array_equal(d_got[margin], d_ref[margin]), f"done mismatch at step {k}"
             borderline += int((~margin).sum())
+            n_term += int((d_got & crashed & margin).sum())
+            term_slack += int((d_got & ~margin).sum())
             live = (~d_got & ~d_ref) if spec.auto_reset else (d_got == d_ref)
             ref_obs = do.build_obs(npos, nvel, neul, nom, target, D).astype(np.float64)
             got_obs = np.asarray(next_obs[k], dtype=np.float64)
@@ -117,8 +121,14 @@ def check_rollout(obs0, actions, next_obs, reward, done, *, spec=do.SINGLE, seed
                 # the CUDA env stores the target as float32, then forms target - pos in float32
                 rt32, rp32 = rt.astype(np.float32), rp.astype(np.float32)
                 ref_reset = np.concatenate([rp32, np.zeros((rows.size, 9), np.float32), rt32 - rp32], 1)
-                assert np.array_equal(np.asarray(next_obs[k])[rows], ref_reset[:, :D]), f"reset obs at step {k}"
+                got_reset = np.asarray(next_obs[k])[rows]
+                if not np.array_equal(got_reset, ref_reset[:, :D]):
+                    bad = np.flatnonzero((got_reset != ref_reset[:, :D]).any(1))
+                    i = rows[bad[0]]
+                    raise AssertionError(f"reset obs at step {k}: {bad.size} of {rows.size} rows differ; env id {env_ids[i]}, "
+                                         f"ep_num {ep_num[i]}: got {got_reset[bad[0]].tolist()} ref {ref_reset[bad[0], :D].tolist()}")
             prev = np.asarray(next_obs[k], dtype=np.float32)
     return {"worst_err_over_bound": worst, "borderline_done": borderline, "dones": n_done,
+            "terminated": n_term, "terminated_slack": term_slack,
             "near_singular_rows": n_sing, "transitions": K * n,
             "worst_pure_relative": {k: {"rel_err": v[0], "at_abs_ref": v[1]} for k, v in pure.items()}}

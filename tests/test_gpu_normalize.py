@@ -23,6 +23,7 @@ pytestmark = pytest.mark.gpu
 from oracle import drone_oracle as do  # noqa: E402
 from oracle import normalize_oracle as no  # noqa: E402
 from oracle import philox, ppo_oracle as po, verify  # noqa: E402
+from oracle.tc_bound import tc_forward_bound  # noqa: E402
 
 U = 2.0 ** -24
 OFFSETS = torch.tensor([1e3, -50, 20, 3, -2, 1, 0.5, 0, -0.3, 40, -40, 5, 0, 0, 7e3], dtype=torch.float64)
@@ -194,18 +195,30 @@ def test_rollout_with_normalised_towers(drl, rollout_kernel_mode, kernel):
     act = b.actions.cpu().numpy()
     ids = np.arange(77, 77 + n, dtype=np.uint64)
     std = np.exp(theta[-4:].numpy())
-    tol_a, tol_v, tol_lp = (2e-2, 2e-2, 5e-2) if tc else (2e-5, 2e-5, 1e-4)
+    tol_a, tol_v, tol_lp = 2e-5, 2e-5, 1e-4
+    th32 = theta.float().numpy()
     for k in range(K):
         mean, value, log_std = po.forward(theta, x_n[k].cpu().double())
         z = philox.noise_normals(seed, ids, t0 + k)
         ref_a = mean.numpy() + std * z
+        lp_got = b.logp[k].cpu().numpy()
+        v = b.value[k].cpu().double()
+        if tc:      # the tensor-core forward within its derived bound (oracle/tc_bound.py); logp from z alone
+            _, _, mb, vb = tc_forward_bound(th32, x_n[k].cpu().numpy())
+            bound_a = mb + 2.0 ** -20 * std * np.abs(z) + 2.0 ** -24 * np.abs(act[k])
+            assert (np.abs(act[k] - ref_a) <= bound_a).all(), f"action k={k}"
+            ref_lp = -0.5 * (z * z).sum(1) - th32[-4:].astype(np.float64).sum() - 2 * np.log(2 * np.pi)
+            assert (np.abs(lp_got - ref_lp) <= 2.0 ** -19 * (0.5 * (z * z).sum(1) + np.abs(th32[-4:]).sum() + 4)).all()
+            assert bool(((v - value).abs() <= torch.from_numpy(vb)).all()), f"value k={k}"
+            continue
         assert (np.abs(act[k] - ref_a) <= tol_a * np.maximum(np.abs(ref_a), 1)).all(), f"action k={k}"
         lp = po.log_prob(mean, log_std, torch.from_numpy(act[k]).double())
-        assert np.abs(b.logp[k].cpu().numpy() - lp.numpy()).max() < tol_lp
-        v = b.value[k].cpu().double()
+        assert np.abs(lp_got - lp.numpy()).max() < tol_lp
         assert bool(((v - value).abs() <= tol_v * value.abs().clamp(min=1)).all()), f"value k={k}"
     _, lv, _ = po.forward(theta, _affine_ref(last_obs, nz).cpu().double())
-    assert bool(((b.last_value.cpu().double() - lv).abs() <= tol_v * lv.abs().clamp(min=1)).all())
+    lv_bound = (torch.from_numpy(tc_forward_bound(th32, _affine_ref(last_obs, nz).cpu().numpy())[3]) if tc
+                else tol_v * lv.abs().clamp(min=1))
+    assert bool(((b.last_value.cpu().double() - lv).abs() <= lv_bound).all())
     # the env transitions, on the raw rows
     o = obs.cpu().numpy()
     nxt = np.concatenate([o[1:], last_obs.cpu().numpy()[None]], 0)

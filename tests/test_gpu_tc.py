@@ -3,7 +3,7 @@ path.  Stated tolerance: tf32 products (10-bit mantissa, inputs rounded to neare
 accumulation and tanh.approx.f32 (max rel error 2^-11):
     layer-1 pre-activations  |err| <= 2^-10 * sum_k |w_k x_k|   (each product carries two 2^-11 roundings)
     layer-2 pre-activations  |err| <= 1.5e-2 * max(1, |ref|)      (adds the layer-1 error through tanh)
-    mean / value             |err| <= 2e-2 * max(1, |ref|)
+    mean / value             per element within the bound of oracle/tc_bound.py
 PARITY UNPINNED for the same reason as tests/test_gpu_ppo.py (SB3 is not in the reference tree)."""
 import numpy as np
 import pytest
@@ -12,6 +12,7 @@ torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
 from oracle import ppo_oracle as po  # noqa: E402
+from oracle.tc_bound import tc_forward_bound  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -62,35 +63,17 @@ def test_tc_forward_matches_oracle(drl, B):
     assert (err1 <= 2.0 ** -10 * scale1 + 1e-6).all(), f"layer-1: worst err/bound {(err1 / (2.0 ** -10 * scale1 + 1e-6)).max():.3g}"
     e1 = (err1 / np.maximum(1.0, np.abs(z1.numpy()))).max()
     e2 = check(d2, z2, 1.5e-2, "layer-2 pre-activation")
-    em = check(mean, rm, 2e-2, "mean")
-    ev = check(value, rv, 2e-2, "value")
+    # mean and value: per element within the derived bound of oracle/tc_bound.py
+    rm_b, rv_b, mb, vb = tc_forward_bound(theta.float().numpy(), obs.numpy())
+    assert np.allclose(rm_b, rm.numpy(), rtol=1e-12, atol=1e-14) and np.allclose(rv_b, rv.numpy(), rtol=1e-12, atol=1e-14)
+    em = (np.abs(mean.cpu().double().numpy() - rm_b) / mb).max()
+    ev = (np.abs(value.cpu().double().numpy() - rv_b) / vb).max()
+    assert em <= 1.0 and ev <= 1.0, f"worst err/bound: mean {em:.3g}, value {ev:.3g}"
     # and against the fp32 CUDA-core kernel of the same library
     m32, v32 = model.policy_forward(obs.cuda())
     assert (mean - m32).abs().max().item() < 2e-2 and (value - v32).abs().max().item() < 4e-2
-    print(f"B={B}: scaled errors L1 {e1:.2e} L2 {e2:.2e} mean {em:.2e} value {ev:.2e}")
+    print(f"B={B}: scaled errors L1 {e1:.2e} L2 {e2:.2e}; err/bound mean {em:.2e} value {ev:.2e}")
     model.close()
-
-
-def test_tc_rollout_matches_fp32_rollout_statistically(drl):
-    """Same seed, same policy: the tf32 rollout's recorded values / log-probs agree with the fp32
-    kernel's wherever the two trajectories have not yet diverged (first step exactly comparable)."""
-    from drone_rl_b200.ppo import PPO
-    n, K = 4096, 8
-    outs = []
-    for prec in ("fp32", "tf32"):
-        m = PPO(drl.DroneBatch(n, drl.EnvConfig.single(), seed=5), n_steps=K, seed=5, rollout_precision=prec)
-        m.params.copy_(_params(7).float().cuda())
-        m.collect_rollouts()
-        torch.cuda.synchronize()
-        outs.append((m.buf.obs.clone(), m.buf.actions.clone(), m.buf.value.clone(), m.buf.logp.clone(), m.buf.adv.clone()))
-        m.close()
-    (o0, a0, v0, l0, adv0), (o1, a1, v1, l1, adv1) = outs
-    assert torch.equal(o0[0], o1[0])                                  # same reset observation
-    assert (a0[0] - a1[0]).abs().max().item() < 2e-2                  # same noise, mean within tf32 tolerance
-    assert (v0[0] - v1[0]).abs().max().item() < 4e-2
-    assert torch.equal(l0[0], l1[0])                                  # log-prob depends on the noise only
-    assert torch.isfinite(adv1).all()
-    assert (v0 - v1).abs().mean().item() < 2e-2
 
 
 # ------------------------------------------------------------------------------------------------------
