@@ -11,10 +11,7 @@
 
 namespace dronecu {
 
-#ifndef DRONECU_BLOCK
-#define DRONECU_BLOCK 256
-#endif
-constexpr int kBlock = DRONECU_BLOCK;
+constexpr int kBlock = 256;
 constexpr int kWarps = kBlock / 32;
 constexpr int kStatSlots = 128;   // episode statistics are spread over this many L2 lines
 
@@ -43,47 +40,20 @@ struct RolloutArgs {
   StatSlot* stats;             // [kStatSlots]
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) {
-  return (uint32_t)__cvta_generic_to_shared(p);
-}
-
-#ifndef DRONECU_EMIT_BULK
-#define DRONECU_EMIT_BULK 0
-#endif
-#ifndef DRONECU_PIPE_PHILOX
-#define DRONECU_PIPE_PHILOX 1   // issue the action Philox block one step ahead (A/B knob)
-#endif
-#ifndef DRONECU_MIN_BLOCKS
-#define DRONECU_MIN_BLOCKS 3   // <= 80 registers/thread, 3 CTAs of 256 threads per SM: no spills and no per-step
-                               // re-derivation of indices (at 64 registers ptxas did both); A/B in profiles/README.md
-#endif
+// <= 80 registers/thread, 3 CTAs of 256 threads per SM: no spills and no per-step re-derivation of indices (at 64
+// registers ptxas did both); A/B in profiles/README.md
+constexpr int kMinBlocks = 3;
 
 // One warp's 32 observations: registers -> per-warp smem tile (stride D words) -> global as
 // 128-bit coalesced stores (lane j moves quad j, j+32, ... of the 32*D contiguous floats).
-// profiles/README.md (round 1) has the ncu comparison with the cp.async.bulk variant
-// (-DDRONECU_EMIT_BULK=1): the kernel is issue-bound and the async-proxy fence + elect + UBLKCP
-// sequence costs more issue slots per warp-step than 4 LDS.128 + 4 STG.128.
+// A cp.async.bulk store of the tile measured no faster (profiles/README.md, round 1): the kernel is
+// issue-bound and the async-proxy fence + elect + UBLKCP sequence costs more issue slots per
+// warp-step than 4 LDS.128 + 4 STG.128.
 template <int OBS_DIM>
 __device__ __forceinline__ void emit_obs_rows(float* tile, float* gdst, const EnvState& s, int lane,
                                               int valid, bool active, bool fast) {
   float* const row = tile + lane * OBS_DIM;
   constexpr int kQuads = 32 * OBS_DIM / 4;
-#if DRONECU_EMIT_BULK
-  constexpr uint32_t kBytes = 32 * OBS_DIM * sizeof(float);
-  if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-  __syncwarp();
-  if (active) write_obs<OBS_DIM>(row, s);
-  if (fast) {
-    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-    __syncwarp();
-    if (lane == 0) {
-      asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;"
-                   :: "l"(gdst), "r"(smem_u32(tile)), "r"(kBytes) : "memory");
-      asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-    }
-    return;
-  }
-#else
   __syncwarp();     // the previous step's read-back of this tile is complete
   if (active) write_obs<OBS_DIM>(row, s);
   if (fast) {       // full warp, 16-byte aligned destination rows: 128-bit read-back + store
@@ -94,7 +64,6 @@ __device__ __forceinline__ void emit_obs_rows(float* tile, float* gdst, const En
     for (int j = lane; j < kQuads; j += 32) st_quad(g4 + j, t4[j]);
     return;
   }
-#endif
   __syncwarp();
   for (int j = lane; j < valid * OBS_DIM; j += 32) gdst[j] = tile[j];
   __syncwarp();
@@ -117,7 +86,7 @@ __device__ __forceinline__ bool emit_fast_ok(const float* base, int64_t warp_bas
 // per-step output bases are warp-uniform (k * n lives in the uniform datapath) so no per-thread running
 // pointers exist, and the episode statistics go straight to shared-memory atomics on the done path.
 template <int OBS_DIM, bool RANDOMIZED, bool AUTORESET, int ACT_MODE, bool RECORD>
-__global__ void __launch_bounds__(kBlock, DRONECU_MIN_BLOCKS) rollout_kernel(const __grid_constant__ RolloutArgs A) {
+__global__ void __launch_bounds__(kBlock, kMinBlocks) rollout_kernel(const __grid_constant__ RolloutArgs A) {
   __shared__ __align__(128) float tiles[kWarps][32 * OBS_DIM];
   __shared__ uint32_t blk_stats[3];      // episodes, terminated, length sum of this CTA (<= 256 * K each)
   __shared__ double blk_ret;
@@ -165,12 +134,8 @@ __global__ void __launch_bounds__(kBlock, DRONECU_MIN_BLOCKS) rollout_kernel(con
     if constexpr (ACT_MODE == 0) {
       if (active && k + 1 < A.K) act = ld_quad_nc(A.actions + koff + n + i);     // software prefetch of the next quad
     } else {
-#if DRONECU_PIPE_PHILOX
       const uint4 w = wnext;
       if (k + 1 < A.K) wnext = env_stream(P.keys, P.env_offset + (uint64_t)i, A.t0 + (uint64_t)(k + 1), STREAM_ACTION);
-#else
-      const uint4 w = env_stream(P.keys, P.env_offset + (uint64_t)i, A.t0 + (uint64_t)k, STREAM_ACTION);
-#endif
       f = make_float4((float)(w.x >> 8) * act_scale, (float)(w.y >> 8) * act_scale,
                       (float)(w.z >> 8) * act_scale, (float)(w.w >> 8) * act_scale);
     }
@@ -221,9 +186,6 @@ __global__ void __launch_bounds__(kBlock, DRONECU_MIN_BLOCKS) rollout_kernel(con
     atomicAdd(&slot->length_sum, (unsigned long long)blk_stats[2]);
     atomicAdd(&slot->return_sum, blk_ret);
   }
-#if DRONECU_EMIT_BULK
-  if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");   // tile must outlive the copy
-#endif
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -250,9 +212,6 @@ __global__ void __launch_bounds__(kBlock) reset_kernel(StatePlanes sp, const __g
   if (obs != nullptr && valid > 0)
     emit_obs_rows<OBS_DIM>(tiles[warp], obs + warp_base * OBS_DIM, s, lane, valid, active,
                            emit_fast_ok<OBS_DIM>(obs, warp_base, n, valid));
-#if DRONECU_EMIT_BULK
-  if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-#endif
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -21,10 +21,7 @@ constexpr float kHalfLog2Pi = 0.91893853320467274178f;   // 0.5 * ln(2 pi)
 // Packed float32 pairs (sm_100: FFMA2 / FMUL2 / FADD2 work on an aligned 64-bit register pair, and one operand may be a
 // scalar that is broadcast to both halves).  Each half is the IEEE fmaf / * / + it replaces -- results are bit-identical --
 // but a pair costs ONE issue slot: the fp32 towers and the elementwise phases of the tensor-core kernels are bound by
-// instruction issue (DESIGN.md section 4), not by the FMA pipe.  -DDRONECU_F32X2=0 compiles the scalar forms (A/B).
-#ifndef DRONECU_F32X2
-#define DRONECU_F32X2 1
-#endif
+// instruction issue (DESIGN.md section 4), not by the FMA pipe; the scalar forms measured slower.
 __device__ __forceinline__ uint64_t pk2(float lo, float hi) {
   uint64_t r;
   asm("mov.b64 %0, {%1, %2};" : "=l"(r) : "f"(lo), "f"(hi));
@@ -33,13 +30,9 @@ __device__ __forceinline__ uint64_t pk2(float lo, float hi) {
 __device__ __forceinline__ void upk2(uint64_t v, float& lo, float& hi) { asm("mov.b64 {%0, %1}, %2;" : "=f"(lo), "=f"(hi) : "l"(v)); }
 // (d0, d1) = (a0, a1) * (b0, b1) + (d0, d1)
 __device__ __forceinline__ void fma2(float& d0, float& d1, float a0, float a1, float b0, float b1) {
-#if DRONECU_F32X2
   uint64_t d;
   asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(pk2(a0, a1)), "l"(pk2(b0, b1)), "l"(pk2(d0, d1)));
   upk2(d, d0, d1);
-#else
-  d0 = fmaf(a0, b0, d0); d1 = fmaf(a1, b1, d1);
-#endif
 }
 // acc[0..3] = w * s + acc[0..3]: the inner step of every fp32 tower (four output units per LDS.128 of weights)
 __device__ __forceinline__ void fma4s(float* acc, const float4 w, const float s) {
@@ -48,31 +41,19 @@ __device__ __forceinline__ void fma4s(float* acc, const float4 w, const float s)
 }
 // (a, b) <- 1 - (a, b)^2
 __device__ __forceinline__ void one_minus_sq2(float a, float b, float& ra, float& rb) {
-#if DRONECU_F32X2
   uint64_t d;
   asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(pk2(-a, -b)), "l"(pk2(a, b)), "l"(pk2(1.f, 1.f)));
   upk2(d, ra, rb);
-#else
-  ra = fmaf(-a, a, 1.f); rb = fmaf(-b, b, 1.f);
-#endif
 }
 __device__ __forceinline__ void mul2(float& a, float& b, float x, float y) {           // (a, b) *= (x, y)
-#if DRONECU_F32X2
   uint64_t d;
   asm("mul.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(pk2(a, b)), "l"(pk2(x, y)));
   upk2(d, a, b);
-#else
-  a *= x; b *= y;
-#endif
 }
 __device__ __forceinline__ void add2(float& a, float& b, float x, float y) {           // (a, b) += (x, y)
-#if DRONECU_F32X2
   uint64_t d;
   asm("add.rn.f32x2 %0, %1, %2;" : "=l"(d) : "l"(pk2(a, b)), "l"(pk2(x, y)));
   upk2(d, a, b);
-#else
-  a += x; b += y;
-#endif
 }
 
 // tanh(x) = 1 - 2 / (exp(2x) + 1) with the MUFU ex2 / rcp approximations: absolute error of a few

@@ -51,6 +51,66 @@ struct UpdArgs {
   float* dbg;                // nullable (tensor-core kernel only): raw TMEM dump [2 gridDim.x, 128 lanes, 256 columns]
 };
 
+// SB3's PPO loss at the head, per sample -- one statement for the three gradient kernels (ppo_grad_kernel, ppo_grad_tc_kernel,
+// ppo_grad_bf16_kernel); each accumulates and stores the results its own way.
+
+// the advantage normalisation of the minibatch: adv = (adv_raw - mean) * inv_std
+__device__ __forceinline__ void adv_normalizer(const UpdArgs& A, float& mean, float& inv_std) {
+  mean = A.adv_mean;
+  inv_std = A.adv_inv_std;
+  if (A.adv_stats != nullptr && A.adv_stats[2] > 1.0) {   // SB3: (adv - adv.mean()) / (adv.std() + 1e-8), torch.std is unbiased
+    const double cnt = A.adv_stats[2], mu = A.adv_stats[0] / cnt;
+    const double var = (A.adv_stats[1] - A.adv_stats[0] * mu) / (cnt - 1.0);
+    mean = (float)mu;
+    inv_std = (float)(1.0 / (sqrt(fmax(var, 0.0)) + 1e-8));
+  } else if (A.adv_stats != nullptr) {   // SB3 normalises only `if len(advantages) > 1`: one sample keeps its raw advantage
+    mean = 0.f;
+    inv_std = 1.f;
+  }
+}
+
+struct PolicyHead {
+  float g_mean[kAct];        // d loss / d mean: clipped surrogate through the Gaussian log-probability
+  float g_logstd[kAct];      // d loss / d log_std: the same, plus the entropy term -ent_coef
+  float pg_loss;             // -min(s1, s2)
+  float kl;                  // (ratio - 1) - log ratio: SB3's approx_kl estimator
+  float clipped;             // 1 where |ratio - 1| > clip (clip fraction)
+};
+
+// `adv` is the normalised advantage, `mean` the policy head's output including its bias
+__device__ __forceinline__ PolicyHead policy_head(const float4 act, const float (&mean)[kAct], const float (&std_inv)[kAct],
+                                                  const float logstd_sum, const float old_logp, const float adv,
+                                                  const float clip, const float ent_coef) {
+  PolicyHead h;
+  const float av[4] = {act.x, act.y, act.z, act.w};
+  float z[kAct], sq = 0.f;
+#pragma unroll
+  for (int o = 0; o < kAct; ++o) { z[o] = (av[o] - mean[o]) * std_inv[o]; sq = fmaf(z[o], z[o], sq); }
+  const float logp = -0.5f * sq - logstd_sum - kAct * kHalfLog2Pi;
+  const float log_ratio = logp - old_logp;
+  const float ratio = expf(log_ratio);
+  const float lo = 1.0f - clip, hi = 1.0f + clip;
+  const float s1 = adv * ratio, s2 = adv * fminf(fmaxf(ratio, lo), hi);
+  const bool inside = (ratio >= lo) && (ratio <= hi);
+  const float dl_dlogp = (inside || s1 < s2) ? -adv * ratio : 0.f;     // d(-min(s1,s2)) / d logp
+#pragma unroll
+  for (int o = 0; o < kAct; ++o) {
+    h.g_mean[o] = dl_dlogp * z[o] * std_inv[o];
+    h.g_logstd[o] = dl_dlogp * (z[o] * z[o] - 1.0f) - ent_coef;
+  }
+  h.pg_loss = -fminf(s1, s2);
+  h.kl = (ratio - 1.0f) - log_ratio;
+  h.clipped = (fabsf(ratio - 1.0f) > clip) ? 1.0f : 0.f;
+  return h;
+}
+
+// value head: returns d(vf_coef * (ret - v)^2) / dv, and the squared error for the value-loss statistic
+__device__ __forceinline__ float value_head(const float v, const float ret, const float vf_coef, float& sq_err) {
+  const float diff = v - ret;
+  sq_err = diff * diff;
+  return 2.0f * vf_coef * diff;
+}
+
 // forward of one tower keeping what the backward pass needs: h1 -> bufA row, h2 -> bufB row
 template <int NOUT>
 __device__ __forceinline__ void tower_forward_keep(const MlpSmem& S, const int t, const float (&x)[kObs],
@@ -249,16 +309,8 @@ __global__ void __launch_bounds__(kUpdBlock, 1) ppo_grad_kernel(const __grid_con
   float std_inv[kAct], logstd_sum = 0.f;
 #pragma unroll
   for (int o = 0; o < kAct; ++o) { std_inv[o] = expf(-U.fwd.log_std[o]); logstd_sum += U.fwd.log_std[o]; }
-  float adv_mean = A.adv_mean, adv_inv_std = A.adv_inv_std;
-  if (A.adv_stats != nullptr && A.adv_stats[2] > 1.0) {   // SB3: (adv - adv.mean()) / (adv.std() + 1e-8), torch.std is unbiased
-    const double cnt = A.adv_stats[2], mu = A.adv_stats[0] / cnt;
-    const double var = (A.adv_stats[1] - A.adv_stats[0] * mu) / (cnt - 1.0);
-    adv_mean = (float)mu;
-    adv_inv_std = (float)(1.0 / (sqrt(fmax(var, 0.0)) + 1e-8));
-  } else if (A.adv_stats != nullptr) {   // SB3 normalises only `if len(advantages) > 1`: one sample keeps its raw advantage
-    adv_mean = 0.f;
-    adv_inv_std = 1.f;
-  }
+  float adv_mean, adv_inv_std;
+  adv_normalizer(A, adv_mean, adv_inv_std);
 
   const int64_t n_tiles = (A.m + kUpdBlock - 1) / kUpdBlock;
   for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -278,35 +330,14 @@ __global__ void __launch_bounds__(kUpdBlock, 1) ppo_grad_kernel(const __grid_con
     // ---------------- policy tower ----------------
     float mean[kAct];
     tower_forward_keep<kAct>(U.fwd, 0, x, U.bufA[tid], U.bufB[tid], mean);
-    float g_pi[kAct] = {0.f, 0.f, 0.f, 0.f}, g_ls[kAct] = {0.f, 0.f, 0.f, 0.f};
-    float st_pl = 0.f, st_kl = 0.f, st_cf = 0.f;
-    if (live) {
-      const float4 a = A.actions[row];
-      const float av[4] = {a.x, a.y, a.z, a.w};
-      float z[kAct], sq = 0.f;
-#pragma unroll
-      for (int o = 0; o < kAct; ++o) { z[o] = (av[o] - mean[o]) * std_inv[o]; sq = fmaf(z[o], z[o], sq); }
-      const float logp = -0.5f * sq - logstd_sum - kAct * kHalfLog2Pi;
-      const float log_ratio = logp - A.old_logp[row];
-      const float ratio = expf(log_ratio);
-      const float adv = (A.adv[row] - adv_mean) * adv_inv_std;
-      const float lo = 1.0f - A.clip, hi = 1.0f + A.clip;
-      const float s1 = adv * ratio, s2 = adv * fminf(fmaxf(ratio, lo), hi);
-      const bool inside = (ratio >= lo) && (ratio <= hi);
-      const float dl_dlogp = (inside || s1 < s2) ? -adv * ratio : 0.f;     // d(-min(s1,s2)) / d logp
-#pragma unroll
-      for (int o = 0; o < kAct; ++o) {
-        g_pi[o] = dl_dlogp * z[o] * std_inv[o];
-        g_ls[o] = dl_dlogp * (z[o] * z[o] - 1.0f) - A.ent_coef;
-      }
-      st_pl = -fminf(s1, s2);
-      st_kl = (ratio - 1.0f) - log_ratio;
-      st_cf = (fabsf(ratio - 1.0f) > A.clip) ? 1.0f : 0.f;
-    }
-    reinterpret_cast<float4*>(U.g3[tid])[0] = make_float4(g_pi[0], g_pi[1], g_pi[2], g_pi[3]);
+    PolicyHead h = {};
+    if (live)
+      h = policy_head(A.actions[row], mean, std_inv, logstd_sum, A.old_logp[row], (A.adv[row] - adv_mean) * adv_inv_std,
+                      A.clip, A.ent_coef);
+    reinterpret_cast<float4*>(U.g3[tid])[0] = make_float4(h.g_mean[0], h.g_mean[1], h.g_mean[2], h.g_mean[3]);
     // log_std gradient + statistics: warp sums -> smem -> fixed-order sum over the 4 warps (deterministic)
     {
-      float v[7] = {g_ls[0], g_ls[1], g_ls[2], g_ls[3], st_pl, st_kl, st_cf};
+      float v[7] = {h.g_logstd[0], h.g_logstd[1], h.g_logstd[2], h.g_logstd[3], h.pg_loss, h.kl, h.clipped};
 #pragma unroll
       for (int q = 0; q < 7; ++q) v[q] = warp_sum(v[q]);
       if (lane == 0) {
@@ -323,7 +354,7 @@ __global__ void __launch_bounds__(kUpdBlock, 1) ppo_grad_kernel(const __grid_con
     wgrad_head<kAct>(U, O_PI_W3, O_PI_B3, rows);
     __syncthreads();                                   // dW3 has consumed h2
     float d1[kHid];
-    tower_backward<kAct>(U, 0, g_pi, U.bufA[tid], U.bufB[tid], d1);
+    tower_backward<kAct>(U, 0, h.g_mean, U.bufA[tid], U.bufB[tid], d1);
     __syncthreads();                                   // delta2 rows complete
     wgrad_hidden(U, O_PI_W2, O_PI_B2, rows);
     __syncthreads();                                   // dW2 has consumed h1
@@ -338,11 +369,7 @@ __global__ void __launch_bounds__(kUpdBlock, 1) ppo_grad_kernel(const __grid_con
     float val[1];
     tower_forward_keep<1>(U.fwd, 1, x, U.bufA[tid], U.bufB[tid], val);
     float g_v[1] = {0.f}, st_vl = 0.f;
-    if (live) {
-      const float diff = val[0] - A.ret[row];
-      g_v[0] = 2.0f * A.vf_coef * diff;                 // d(vf_coef * (ret - v)^2) / dv
-      st_vl = diff * diff;
-    }
+    if (live) g_v[0] = value_head(val[0], A.ret[row], A.vf_coef, st_vl);
     U.g3[tid][0] = g_v[0];
     {
       const float v0 = warp_sum(st_vl), v1 = warp_sum(live ? 1.0f : 0.f);

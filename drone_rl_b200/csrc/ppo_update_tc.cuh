@@ -359,16 +359,8 @@ __global__ void __launch_bounds__(tcu::kThreads, 1) ppo_grad_tc_kernel(const __g
     float std_inv[kAct], logstd_sum = 0.f;
 #pragma unroll
     for (int o = 0; o < kAct; ++o) { std_inv[o] = expf(-S.log_std[o]); logstd_sum += S.log_std[o]; }
-    float adv_mean = A.adv_mean, adv_inv_std = A.adv_inv_std;
-    if (A.adv_stats != nullptr && A.adv_stats[2] > 1.0) {   // SB3: (adv - adv.mean()) / (adv.std() + 1e-8), torch.std is unbiased
-      const double cnt = A.adv_stats[2], mu = A.adv_stats[0] / cnt;
-      const double var = (A.adv_stats[1] - A.adv_stats[0] * mu) / (cnt - 1.0);
-      adv_mean = (float)mu;
-      adv_inv_std = (float)(1.0 / (sqrt(fmax(var, 0.0)) + 1e-8));
-    } else if (A.adv_stats != nullptr) {   // SB3 normalises only `if len(advantages) > 1`: one sample keeps its raw advantage
-      adv_mean = 0.f;
-      adv_inv_std = 1.f;
-    }
+    float adv_mean, adv_inv_std;
+    adv_normalizer(A, adv_mean, adv_inv_std);
 
     unsigned char* const bufA = S.bufA[wg];
     unsigned char* const bufB = S.bufB[wg];
@@ -516,34 +508,27 @@ __global__ void __launch_bounds__(tcu::kThreads, 1) ppo_grad_tc_kernel(const __g
       float g3[kAct] = {0.f, 0.f, 0.f, 0.f};
       if (tw == 0) {
         if (live) {
-          const float av[4] = {act.x, act.y, act.z, act.w};
-          float z[kAct], sq = 0.f;
+          float mean[kAct];
 #pragma unroll
-          for (int o = 0; o < kAct; ++o) { z[o] = (av[o] - (out[o] + S.b3[o])) * std_inv[o]; sq = fmaf(z[o], z[o], sq); }
-          const float logp = -0.5f * sq - logstd_sum - kAct * kHalfLog2Pi;
-          const float log_ratio = logp - old_logp;
-          const float ratio = expf(log_ratio);
-          const float adv = (adv_raw - adv_mean) * adv_inv_std;
-          const float lo = 1.0f - A.clip, hi = 1.0f + A.clip;
-          const float s1 = adv * ratio, s2 = adv * fminf(fmaxf(ratio, lo), hi);
-          const bool inside = (ratio >= lo) && (ratio <= hi);
-          const float dl_dlogp = (inside || s1 < s2) ? -adv * ratio : 0.f;     // d(-min(s1,s2)) / d logp
+          for (int o = 0; o < kAct; ++o) mean[o] = out[o] + S.b3[o];
+          const PolicyHead h = policy_head(act, mean, std_inv, logstd_sum, old_logp, (adv_raw - adv_mean) * adv_inv_std,
+                                           A.clip, A.ent_coef);
 #pragma unroll
           for (int o = 0; o < kAct; ++o) {
-            g3[o] = dl_dlogp * z[o] * std_inv[o];
-            accs[o] += dl_dlogp * (z[o] * z[o] - 1.0f) - A.ent_coef;
+            g3[o] = h.g_mean[o];
+            accs[o] += h.g_logstd[o];
             accs[4 + o] += g3[o];
           }
-          accs[8] += -fminf(s1, s2);
-          accs[9] += (ratio - 1.0f) - log_ratio;
-          accs[10] += (fabsf(ratio - 1.0f) > A.clip) ? 1.0f : 0.f;
+          accs[8] += h.pg_loss;
+          accs[9] += h.kl;
+          accs[10] += h.clipped;
         }
       } else {
         if (live) {
-          const float diff = (out[0] + S.b3[0]) - ret;
-          g3[0] = 2.0f * A.vf_coef * diff;                   // d(vf_coef * (ret - v)^2) / dv
+          float sq_err;
+          g3[0] = value_head(out[0] + S.b3[0], ret, A.vf_coef, sq_err);
           accs[0] += g3[0];
-          accs[1] += diff * diff;
+          accs[1] += sq_err;
           accs[2] += 1.0f;
         }
       }

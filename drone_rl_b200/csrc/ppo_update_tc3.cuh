@@ -21,14 +21,15 @@
 //     (S1..S3) need no order at all: every warpgroup has its OWN private-step issuer warp (512 threads per CTA).  r02:
 //     before, one shared private-step issuer warp walked a global order, which made every warpgroup's S1 wait for
 //     another warpgroup's tanh phase -- 1.9k idle cycles per tile in the in-kernel timeline; issuing from warp 0 of the
-//     warpgroup instead (-DDRONECU_PRIVATE_ISSUER_WARPS=0) cost 9 %: that warp sits in the MMA issue for ~1k cycles when
-//     the tensor queue is full and becomes the straggler of its warpgroup;
+//     warpgroup instead cost 9 %: that warp sits in the MMA issue for ~1k cycles when the tensor queue is full and
+//     becomes the straggler of its warpgroup;
 //   * the observation rows of the next tile are fetched a tile ahead in four parts spread over the tile; with 64-byte rows
 //     in the rollout buffer (template PADDED) a row is four LDG.128 by four lanes and is staged with vector stores; the tf32
 //     X tile is staged over the dead bufB (never over memory another warp still reads: the r02 race);
 //   * tanh'(layer 1) = 1 - H1^2 is stashed per sample as bf16 (2^-9 relative) next to the operands, because H1 itself
 //     survives only as a bf16 operand (1 - h^2 from a rounded h would lose the saturated units); tanh'(layer 2) uses
-//     the fp32 H2 still in TMEM.  The stash uses the [8-feature chunk][sample][16 B] layout of the operand buffers;
+//     the fp32 H2 still in TMEM.  The stash uses the [8-feature chunk][sample][16 B] layout of the operand buffers
+//     (swizzled 128-byte rows per sample measured slower);
 //   * the elementwise phases work on the register pairs tcgen05.ld delivers with packed fp32 instructions (FFMA2 / FMUL2 /
 //     FADD2, ppo_common.cuh): ~1,180 instructions per thread and tile instead of ~1,400, bit-identical results.
 // Steps per tile (S1..S6 as in ppo_update_tc.cuh): S1 D1 = X.W1^T | S2 D2 = H1.W2^T | S3 D3 = H2.W3p^T |
@@ -37,27 +38,6 @@
 #pragma once
 #include "ppo_update_tc.cuh"
 
-// A-operand activations written to TMEM (H1, H2, dZ2): 1 = round to nearest tf32 first (one integer add per value),
-// 0 = leave the fp32 bits, the tensor core drops the low 13 mantissa bits itself.  Truncation measured 2 % faster, but its
-// error is a coherent bias: the largest block error grew with the minibatch (4.5e-3 at 38k samples, 6.9e-3 at 114k).
-#ifndef DRONECU_TF32_ROUND
-#define DRONECU_TF32_ROUND 1
-#endif
-
-// A/B knobs of the accumulating issuer (r02 race hunt): software-pipelined service order, interleaved S5 products
-#ifndef DRONECU_ACC_PIPELINED
-#define DRONECU_ACC_PIPELINED 1
-#endif
-#ifndef DRONECU_S5_INTERLEAVE
-#define DRONECU_S5_INTERLEAVE 1
-#endif
-#ifndef DRONECU_ACC_DYNAMIC
-#define DRONECU_ACC_DYNAMIC 0       // accumulating issuer serves whichever warpgroup is ready, per-accumulator tile order kept (measured 24 % slower)
-#endif
-#ifndef DRONECU_S5_SPLIT
-#define DRONECU_S5_SPLIT 0          // S5: dH1 committed on its own, the weight-gradient half signals a second barrier (measured 4.5 % slower)
-#endif
-
 namespace dronecu {
 namespace tcb {
 
@@ -65,10 +45,7 @@ using namespace tcu;            // descriptors, TMEM ld / st helpers, elect_one,
 
 constexpr int kWG3 = 3;
 constexpr int kComputeThreads3 = 128 * kWG3;
-#ifndef DRONECU_PRIVATE_ISSUER_WARPS
-#define DRONECU_PRIVATE_ISSUER_WARPS 1   // 1: one private-step issuer warp per warpgroup (512 threads); 0: warp 0 of the warpgroup issues them (416 threads)
-#endif
-constexpr int kIssuerWarps3 = DRONECU_PRIVATE_ISSUER_WARPS ? kWG3 + 1 : 1;
+constexpr int kIssuerWarps3 = kWG3 + 1;                // one private-step issuer warp per warpgroup + the accumulating issuer
 constexpr int kThreads3 = kComputeThreads3 + 32 * kIssuerWarps3;   // compute warpgroups + issuer warps (the LAST one is the accumulating issuer: S4..S6)
 constexpr int kGrp = 128 * 16;                         // one 8-feature group of a bf16 MN-major operand: [128 samples][16 B]
 constexpr int kWgCols = 136;                           // P 64 | Q 64 | G 8
@@ -92,11 +69,10 @@ struct alignas(1024) Smem3 {
   float b3[kAct];
   float log_std[kAct];
   float wsum[kWG3][4][kNS];
-  alignas(8) unsigned long long full[kWG3];     // operands of S1 / S2 / S3 staged (served by issuer warp 0)
-  alignas(8) unsigned long long fullA[kWG3];    // operands of S4 / S5 / S6 staged (served by issuer warp 1, fixed order)
-  alignas(8) unsigned long long done[kWG3];     // S1 / S2 / S3 completed (commit of issuer warp 0)
-  alignas(8) unsigned long long doneA[kWG3];    // S4 / S5 / S6 completed (commit of issuer warp 1)
-  alignas(8) unsigned long long doneW[kWG3];    // DRONECU_S5_SPLIT: the weight-gradient half of S5 completed (bufA / bufB free)
+  alignas(8) unsigned long long full[kWG3];     // operands of S1 / S2 / S3 staged (served by the warpgroup's private-step issuer)
+  alignas(8) unsigned long long fullA[kWG3];    // operands of S4 / S5 / S6 staged (served by the accumulating issuer, fixed order)
+  alignas(8) unsigned long long done[kWG3];     // S1 / S2 / S3 completed (commit of the private-step issuer)
+  alignas(8) unsigned long long doneA[kWG3];    // S4 / S5 / S6 completed (commit of the accumulating issuer)
   uint32_t tmem_base, pad1[3];
 };
 
@@ -121,20 +97,6 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
 }
 __device__ __forceinline__ float bf16_lo(uint32_t w) { return __uint_as_float(w << 16); }
 __device__ __forceinline__ float bf16_hi(uint32_t w) { return __uint_as_float(w & 0xffff0000u); }
-
-// A/B knobs of the elementwise phases (r02, profiles/README.md)
-#ifndef DRONECU_STASH_GROUPS
-#define DRONECU_STASH_GROUPS 1      // tanh' stash in the [chunk][sample][16 B] layout of bufA instead of swizzled 128-byte rows
-#endif
-#ifndef DRONECU_S5_BF16MUL
-#define DRONECU_S5_BF16MUL 0        // dZ1 = bf16(dH1) * stash as one HMUL2.BF16 per pair (two roundings) instead of fp32 products
-#endif
-__device__ __forceinline__ uint32_t mul_bf16x2(uint32_t a, uint32_t b) {
-  uint32_t r;
-  asm("mul.rn.bf16x2 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(b));
-  return r;
-}
-
 
 __device__ __forceinline__ void setup3(Smem3& S, const float* __restrict__ theta, const int tw) {
   const int tid = threadIdx.x;
@@ -164,7 +126,7 @@ __device__ __forceinline__ void setup3(Smem3& S, const float* __restrict__ theta
     S.log_std[tid] = theta[O_LOGSTD + tid];
   }
   if (tid == 0) {
-    for (int w = 0; w < kWG3; ++w) { mbar_init(&S.full[w], 128); mbar_init(&S.fullA[w], 128); mbar_init(&S.done[w], 1); mbar_init(&S.doneA[w], 1); mbar_init(&S.doneW[w], 1); }
+    for (int w = 0; w < kWG3; ++w) { mbar_init(&S.full[w], 128); mbar_init(&S.fullA[w], 128); mbar_init(&S.done[w], 1); mbar_init(&S.doneA[w], 1); }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncwarp();
@@ -186,7 +148,8 @@ constexpr uint64_t kStrA = (9 * kGrp) >> 4, kStrB = (8 * kGrp) >> 4, kStrXn = (4
 constexpr uint64_t kBumpW = 256 >> 4, kBumpXs = (2 * kXsLbo) >> 4, kBumpIl = 256 >> 4;      // per-slice bumps of the start-address field
 
 // Private steps S1, S2, S3 of warpgroup w: they write only the warpgroup's private TMEM columns, so there is nothing to
-// order against the other warpgroups.  Called by warp 0 of the warpgroup after every thread of it has arrived on `full`.
+// order against the other warpgroups.  Called by the warpgroup's private-step issuer warp; waits until every thread of the
+// warpgroup has arrived on `full`.
 // `dA` = descriptor of the step's shared-memory A operand (S1: the X tile) -- unused for S2 / S3 (A in TMEM); `dB` = its weights.
 template <int STEP>
 __device__ __forceinline__ void issue_private(unsigned long long* full, unsigned long long* done, const uint32_t tmem,
@@ -214,15 +177,17 @@ __device__ __forceinline__ void issue_private(unsigned long long* full, unsigned
 // j = 3 r + w (round r, warpgroup w); the existing ones are a prefix j = 0 .. n_cta - 1 of that sequence.  Each shared
 // accumulator (dW3 by S4, dW2 | db2 by S5, dW1 | db1 by S6) must receive the tiles in order of j; the services are
 // software-pipelined over consecutive tiles -- S4(0) S5(0) | S4(j) S6(j-1) S5(j) | ... | S6(n-1) -- so that between the two
-// services of one warpgroup that are separated by its dZ2 / dZ1 phases the issuer serves another warpgroup.
+// services of one warpgroup that are separated by its dZ2 / dZ1 phases the issuer serves another warpgroup.  The fixed order
+// is also what staggers the three warpgroups: the sequential S4(j) S5(j) S6(j) measured 1.625 vs 1.619 ms, and serving
+// whichever warpgroup is ready 24 % slower (served eagerly they fall into step and queue on the same phases; profiles/README.md).
 __device__ __forceinline__ void issuer_accum(Smem3& S, const int n_cta, long long* tlog) {
   const uint64_t dW2T = desc_w(smem_addr(S.W2T), kHid, 0), dW3k = desc_w(smem_addr(S.W3k), 8, 0);
   const uint64_t dA0 = desc_il(smem_addr(S.bufA[0]), 0), dB0 = desc_il(smem_addr(S.bufB[0]), 0), dXn0 = desc_il(smem_addr(S.XN[0][0]), 0);
   const uint32_t tbase = S.tmem_base;
   uint32_t ph_mask = 0;                                // bit w: parity of warpgroup w's `fullA` barrier
-  auto serve = [&](const int j, const int step, const bool ready = false) __attribute__((always_inline)) {      // step 3, 4, 5 = S4, S5, S6 of tile j
+  auto serve = [&](const int j, const int step) __attribute__((always_inline)) {      // step 3, 4, 5 = S4, S5, S6 of tile j
     const int w = j % kWG3, r = j / kWG3;
-    if (!ready) mbar_wait(&S.fullA[w], (ph_mask >> w) & 1u);
+    mbar_wait(&S.fullA[w], (ph_mask >> w) & 1u);
     ph_mask ^= 1u << w;
     fence_after();
     if (w == 0) TSTAMP(tlog, r, 2 * step);
@@ -237,84 +202,30 @@ __device__ __forceinline__ void issuer_accum(Smem3& S, const int n_cta, long lon
         for (int s = 0; s < 8; ++s) mma_bf16_ss(tbase + kAcc3, dH + kBumpIl * s, dG + kBumpIl * s, idesc_bf16(64, 8, 1, 1), first | (s > 0));
       } else if (step == 4) {     // S5: dH1 = dZ2 . W2 (tf32, A = dZ2 in TMEM) ; dW2 | db2 += dZ2^T . [H1 | G] (bf16, N = 72)
         const uint64_t dZ = dB0 + kStrB * uw, dHG = dA0 + kStrA * uw;
-#if DRONECU_S5_SPLIT
-        // the compute warps only need dH1 to go on: commit the activation-gradient product on its own; the weight-gradient
-        // product (it reads bufA / bufB, which the dZ1 phase overwrites) signals doneW
+        // The two products are independent: interleave them in the pipe.  Issued one after the other they keep the tensor
+        // pipe waiting on shared-memory operands (1.633 vs 1.619 ms); so does committing dH1 on its own so that the dZ1
+        // phase starts earlier (+4.5 %, more than the earlier wake-up gains).
 #pragma unroll
-        for (int s = 0; s < 8; ++s) mma_tf32_ts(tmem + kCP, tmem + kCQ + 8 * s, dW2T + kBumpW * s, idesc(128, 64, 0, 0), s > 0);
-        mma_commit(&S.doneA[w]);
-#pragma unroll
-        for (int s = 0; s < 8; ++s) mma_bf16_ss(tbase + kAcc2, dZ + kBumpIl * s, dHG + kBumpIl * s, idesc_bf16(64, 72, 1, 1), first | (s > 0));
-        mma_commit(&S.doneW[w]);
-#elif DRONECU_S5_INTERLEAVE
-#pragma unroll
-        for (int s = 0; s < 8; ++s) {                  // the two products are independent: interleave them in the pipe
+        for (int s = 0; s < 8; ++s) {
           mma_tf32_ts(tmem + kCP, tmem + kCQ + 8 * s, dW2T + kBumpW * s, idesc(128, 64, 0, 0), s > 0);
           mma_bf16_ss(tbase + kAcc2, dZ + kBumpIl * s, dHG + kBumpIl * s, idesc_bf16(64, 72, 1, 1), first | (s > 0));
         }
-#else
-#pragma unroll
-        for (int s = 0; s < 8; ++s) mma_tf32_ts(tmem + kCP, tmem + kCQ + 8 * s, dW2T + kBumpW * s, idesc(128, 64, 0, 0), s > 0);
-#pragma unroll
-        for (int s = 0; s < 8; ++s) mma_bf16_ss(tbase + kAcc2, dZ + kBumpIl * s, dHG + kBumpIl * s, idesc_bf16(64, 72, 1, 1), first | (s > 0));
-#endif
       } else {                    // S6: dW1 | db1 += dZ1^T . [X | 1] (bf16, N = 16)
         const uint64_t dZ = dA0 + kStrA * uw, dX = dXn0 + kStrXn * uw + kParXn * (uint64_t)(r & 1);
 #pragma unroll
         for (int s = 0; s < 8; ++s) mma_bf16_ss(tbase + kAcc1, dZ + kBumpIl * s, dX + kBumpIl * s, idesc_bf16(64, 16, 1, 1), first | (s > 0));
       }
-      if (!(DRONECU_S5_SPLIT && step == 4)) mma_commit(&S.doneA[w]);
+      mma_commit(&S.doneA[w]);
     }
     __syncwarp();
     if (w == 0) TSTAMP(tlog, r, 2 * step + 1);
   };
-#if DRONECU_ACC_DYNAMIC
-  // Whoever is ready, within the order every accumulator needs: S4 / S5 / S6 each take the tiles in order of j (dW3, dW2 | db2,
-  // dW1 | db1 accumulate in that order: the sums stay bit-identical to the fixed schedule), but a ready S4 of the next warpgroup
-  // no longer waits behind a not-yet-ready S5 of this one.
-  int nx4 = 0, nx5 = 0, nx6 = 0;                       // the next tile of each step
-  uint32_t stp = 0;                                    // 2 bits per warpgroup: the step (0, 1, 2 = S4, S5, S6) it hands over next
-  int r0 = 0, r1 = 0, r2 = 0;                          // ... of the tile of this round
-  int left = 3 * n_cta, w = 0;
-#pragma unroll 1
-  while (left > 0) {
-    const int r = (w == 0) ? r0 : (w == 1) ? r1 : r2;
-    const int j = kWG3 * r + w;
-    const int st = (int)((stp >> (2 * w)) & 3u);
-    const int nx = (st == 0) ? nx4 : (st == 1) ? nx5 : nx6;
-    bool served = false;
-    if (j < n_cta && nx == j) {
-      uint32_t ok;
-      asm volatile("{\n\t.reg .pred p;\n\tmbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}\n"
-                   : "=r"(ok) : "r"(smem_addr(&S.fullA[w])), "r"((ph_mask >> w) & 1u) : "memory");
-      if (ok) {
-        if (st == 0) { serve(j, 3, true); nx4 = j + 1; }
-        else if (st == 1) { serve(j, 4, true); nx5 = j + 1; }
-        else { serve(j, 5, true); nx6 = j + 1; }
-        stp = (stp & ~(3u << (2 * w))) | ((st == 2 ? 0u : (uint32_t)(st + 1)) << (2 * w));
-        if (st == 2) { if (w == 0) ++r0; else if (w == 1) ++r1; else ++r2; }
-        --left;
-        served = true;
-      }
-    }
-    w = (w == kWG3 - 1) ? 0 : w + 1;
-    if (!served && w == 0) __nanosleep(32);            // a full round without work: leave the issue slots to the compute warps
-  }
-#elif DRONECU_ACC_PIPELINED
 #pragma unroll 1
   for (int j = 0; j <= n_cta; ++j) {
     if (j < n_cta) serve(j, 3);
     if (j > 0) serve(j - 1, 5);
     if (j < n_cta) serve(j, 4);
   }
-#else
-#pragma unroll 1
-  for (int j = 0; j < n_cta; ++j) {
-    serve(j, 3);
-    serve(j, 4);
-    serve(j, 5);
-  }
-#endif
 }
 
 }  // namespace tcb
@@ -370,48 +281,23 @@ __global__ void __launch_bounds__(tcb::kThreads3, 1) ppo_grad_bf16_kernel(const 
     float std_inv[kAct], logstd_sum = 0.f;
 #pragma unroll
     for (int o = 0; o < kAct; ++o) { std_inv[o] = expf(-S.log_std[o]); logstd_sum += S.log_std[o]; }
-    float adv_mean = A.adv_mean, adv_inv_std = A.adv_inv_std;
-    if (A.adv_stats != nullptr && A.adv_stats[2] > 1.0) {   // SB3: (adv - adv.mean()) / (adv.std() + 1e-8), torch.std is unbiased
-      const double cnt = A.adv_stats[2], mu = A.adv_stats[0] / cnt;
-      const double var = (A.adv_stats[1] - A.adv_stats[0] * mu) / (cnt - 1.0);
-      adv_mean = (float)mu;
-      adv_inv_std = (float)(1.0 / (sqrt(fmax(var, 0.0)) + 1e-8));
-    } else if (A.adv_stats != nullptr) {   // SB3 normalises only `if len(advantages) > 1`: one sample keeps its raw advantage
-      adv_mean = 0.f;
-      adv_inv_std = 1.f;
-    }
+    float adv_mean, adv_inv_std;
+    adv_normalizer(A, adv_mean, adv_inv_std);
 
     unsigned char* const rowA = S.bufA[wg] + r * 16;       // + g * kGrp: this sample's 16 bytes of feature group g
     unsigned char* const rowB = S.bufB[wg] + r * 16;
     unsigned char* const XN0 = S.XN[wg][0];
     // tf32 X tile (A operand of S1, 9216 B): staged over the DEAD bufB of the previous tile (dZ2: read only by the tensor core,
     // S5 has completed) -- no thread ever reads that region.  r01 staged it over the tanh' stash, whose rows other warps of the
-    // warpgroup still read in their dZ1 phase: with the private steps issued by warp 0 that aliasing produced one garbage
-    // 8-feature block of dW1 per ~1500 launches at the c5 size (scratch/stress_determinism.py).
+    // warpgroup still read in their dZ1 phase: that aliasing produced one garbage 8-feature block of dW1 per ~1500 launches at
+    // the c5 size (scratch/stress_determinism.py).
     unsigned char* const XS = S.bufB[wg];
-#if DRONECU_STASH_GROUPS
     unsigned char* const rowG1 = S.XG[wg] + r * 16;        // chunk c of this sample at c * kGrp (the layout of bufA: conflict-free, immediate offsets)
-#define STASH_OFF(c) ((c) * kGrp)
-#else
-    unsigned char* const rowG1 = S.XG[wg] + r * 128;       // 8 chunks of 16 B, chunk c at ((c ^ (r & 7)) << 4)
-    const int sw = r & 7;
-#define STASH_OFF(c) (((c) ^ sw) << 4)
-#endif
     unsigned long long* const full = &S.full[wg];
     unsigned long long* const fullA = &S.fullA[wg];
     unsigned long long* const done = &S.done[wg];
     unsigned long long* const doneA = &S.doneA[wg];
-#if DRONECU_S5_SPLIT
-    unsigned long long* const doneW = &S.doneW[wg];
-    uint32_t phW = 0;
-#endif
     uint32_t phA = 0;
-#if !DRONECU_PRIVATE_ISSUER_WARPS
-    uint32_t phf = 0;
-    // descriptors of the private steps (issued by warp 0 of the warpgroup)
-    const uint64_t dXs = make_desc(smem_addr(S.bufB[wg]), kXsLbo, kXsSbo, 0), dW1 = desc_w(smem_addr(S.W1), 16, 0);
-    const uint64_t dW2 = desc_w(smem_addr(S.W2), kHid, 0), dW3p = desc_w(smem_addr(S.W3p), kHid, 0);
-#endif
     const uint32_t tmem = S.tmem_base + wg * kWgCols;
     const uint32_t tL = tmem + ((uint32_t)(wq * 32) << 16);
     uint32_t ph = 0;
@@ -512,9 +398,6 @@ __global__ void __launch_bounds__(tcb::kThreads3, 1) ppo_grad_bf16_kernel(const 
         }
       }
       hand_over(full);
-#if !DRONECU_PRIVATE_ISSUER_WARPS
-      if (wq == 0) issue_private<0>(full, done, tmem, dXs, dW1, phf);
-#endif
       TSTAMP(tlog, it, 2);
       const int row_nn = row_of(tile + 2 * stride);       // the tile after the next: its row numbers are needed a tile from now
       gather_rows(row_nxt, cur, 0);
@@ -543,27 +426,21 @@ __global__ void __launch_bounds__(tcb::kThreads3, 1) ppo_grad_bf16_kernel(const 
             float t[8];
 #pragma unroll
             for (int i = 0; i < 8; i += 2) one_minus_sq2(h[i], h[i + 1], t[i], t[i + 1]);
-            *reinterpret_cast<uint4*>(rowG1 + STASH_OFF(2 * c + j)) =
+            *reinterpret_cast<uint4*>(rowG1 + (2 * c + j) * kGrp) =
                 make_uint4(pack_bf16(t[0], t[1]), pack_bf16(t[2], t[3]), pack_bf16(t[4], t[5]), pack_bf16(t[6], t[7]));
           }
-#if DRONECU_TF32_ROUND
+          // A operands written to TMEM (H1, H2, dZ2) are rounded to nearest tf32 first (one integer add per value) rather
+          // than left for the tensor core to truncate: truncation measured 2 % faster, but its error is a coherent bias --
+          // the largest block error grew with the minibatch (4.5e-3 at 38k samples, 6.9e-3 at 114k).
 #pragma unroll
           for (int i = 0; i < 16; ++i) v[i] = to_tf32_fast(v[i]);
-#endif
           st16(tL + kCP + 16 * c, v);
           if (c < 3) ld_fence(w);
         }
       }
       wait_st();
       hand_over(full);
-      // warp 0 issues this step's MMAs (it can sit in the issue for ~1k cycles when the tensor pipe's queue is full): it takes
-      // its second and third part of the gather after the S4 / S5 hand-overs instead, where the accumulating issuer issues
-#if DRONECU_PRIVATE_ISSUER_WARPS
       gather_rows(row_nxt, cur, 4);
-#else
-      if (wq == 0) issue_private<1>(full, done, tmem, 0, dW2, phf);
-      else gather_rows(row_nxt, cur, 4);
-#endif
       TSTAMP(tlog, it, 5);
 
       // ---------------- S2 done: H2 = tanh(D2 + b2) -> Q (tf32, A of S3; fp32-accurate copy for tanh'), bufB (bf16) ----------------
@@ -592,22 +469,15 @@ __global__ void __launch_bounds__(tcb::kThreads3, 1) ppo_grad_bf16_kernel(const 
             *reinterpret_cast<uint4*>(rowB + (2 * c + j) * kGrp) =
                 make_uint4(pack_bf16(h[0], h[1]), pack_bf16(h[2], h[3]), pack_bf16(h[4], h[5]), pack_bf16(h[6], h[7]));
           }
-#if DRONECU_TF32_ROUND
 #pragma unroll
           for (int i = 0; i < 16; ++i) v[i] = to_tf32_fast(v[i]);
-#endif
           st16(tL + kCQ + 16 * c, v);
           if (c < 3) ld_fence(w);
         }
       }
       wait_st();
       hand_over(full);
-#if DRONECU_PRIVATE_ISSUER_WARPS
       gather_rows(row_nxt, cur, 8);
-#else
-      if (wq == 0) issue_private<2>(full, done, tmem, 0, dW3p, phf);
-      else gather_rows(row_nxt, cur, 8);
-#endif
       TSTAMP(tlog, it, 7);
 
       // ---------------- S3 done: head outputs -> loss gradient at the head ----------------
@@ -618,34 +488,27 @@ __global__ void __launch_bounds__(tcb::kThreads3, 1) ppo_grad_bf16_kernel(const 
       float g3[kAct] = {0.f, 0.f, 0.f, 0.f};
       if (tw == 0) {
         if (live) {
-          const float av[4] = {act.x, act.y, act.z, act.w};
-          float z[kAct], sq = 0.f;
+          float mean[kAct];
 #pragma unroll
-          for (int o = 0; o < kAct; ++o) { z[o] = (av[o] - (out[o] + S.b3[o])) * std_inv[o]; sq = fmaf(z[o], z[o], sq); }
-          const float logp = -0.5f * sq - logstd_sum - kAct * kHalfLog2Pi;
-          const float log_ratio = logp - old_logp;
-          const float ratio = expf(log_ratio);
-          const float adv = (adv_raw - adv_mean) * adv_inv_std;
-          const float lo = 1.0f - A.clip, hi = 1.0f + A.clip;
-          const float s1 = adv * ratio, s2 = adv * fminf(fmaxf(ratio, lo), hi);
-          const bool inside = (ratio >= lo) && (ratio <= hi);
-          const float dl_dlogp = (inside || s1 < s2) ? -adv * ratio : 0.f;     // d(-min(s1,s2)) / d logp
+          for (int o = 0; o < kAct; ++o) mean[o] = out[o] + S.b3[o];
+          const PolicyHead h = policy_head(act, mean, std_inv, logstd_sum, old_logp, (adv_raw - adv_mean) * adv_inv_std,
+                                           A.clip, A.ent_coef);
 #pragma unroll
           for (int o = 0; o < kAct; ++o) {
-            g3[o] = dl_dlogp * z[o] * std_inv[o];
-            accs[o] += dl_dlogp * (z[o] * z[o] - 1.0f) - A.ent_coef;
+            g3[o] = h.g_mean[o];
+            accs[o] += h.g_logstd[o];
             accs[4 + o] += g3[o];
           }
-          accs[8] += -fminf(s1, s2);
-          accs[9] += (ratio - 1.0f) - log_ratio;
-          accs[10] += (fabsf(ratio - 1.0f) > A.clip) ? 1.0f : 0.f;
+          accs[8] += h.pg_loss;
+          accs[9] += h.kl;
+          accs[10] += h.clipped;
         }
       } else {
         if (live) {
-          const float diff = (out[0] + S.b3[0]) - ret;
-          g3[0] = 2.0f * A.vf_coef * diff;                   // d(vf_coef * (ret - v)^2) / dv
+          float sq_err;
+          g3[0] = value_head(out[0] + S.b3[0], ret, A.vf_coef, sq_err);
           accs[0] += g3[0];
-          accs[1] += diff * diff;
+          accs[1] += sq_err;
           accs[2] += 1.0f;
         }
       }
@@ -659,9 +522,6 @@ __global__ void __launch_bounds__(tcb::kThreads3, 1) ppo_grad_bf16_kernel(const 
       wait_st();
       hand_over(fullA);
       gather_rows(row_nxt, cur, 12);
-#if !DRONECU_PRIVATE_ISSUER_WARPS
-      if (wq == 0) gather_rows(row_nxt, cur, 4);
-#endif
       gather_scalars(row_nxt, cur);                        // this tile's act / old_logp / adv / ret live in locals since the top
       TSTAMP(tlog, it, 9);
 
@@ -687,24 +547,19 @@ __global__ void __launch_bounds__(tcb::kThreads3, 1) ppo_grad_bf16_kernel(const 
           *reinterpret_cast<uint4*>(rowB + (2 * c + j) * kGrp) =
               make_uint4(pack_bf16(z[0], z[1]), pack_bf16(z[2], z[3]), pack_bf16(z[4], z[5]), pack_bf16(z[6], z[7]));
         }
-#if DRONECU_TF32_ROUND
 #pragma unroll
         for (int i = 0; i < 16; ++i) d[i] = to_tf32_fast(d[i]);
-#endif
         st16(tL + kCQ + 16 * c, d);
       }
       wait_st();
       hand_over(fullA);
-#if !DRONECU_PRIVATE_ISSUER_WARPS
-      if (wq == 0) gather_rows(row_nxt, cur, 8);
-#endif
       TSTAMP(tlog, it, 11);
 
       // ---------------- S5 done: dZ1 = dH1 * (1 - H1^2) -> bufA (bf16, A of S6) ----------------
       {
         uint4 g1[8];                              // the stash does not depend on S5: read it while S5 runs
 #pragma unroll
-        for (int c = 0; c < 8; ++c) g1[c] = *reinterpret_cast<const uint4*>(rowG1 + STASH_OFF(c));
+        for (int c = 0; c < 8; ++c) g1[c] = *reinterpret_cast<const uint4*>(rowG1 + c * kGrp);
         mbar_wait(doneA, phA); phA ^= 1; fence_after();
         TSTAMP(tlog, it, 12);
         float va[16], vb[16];
@@ -719,22 +574,13 @@ __global__ void __launch_bounds__(tcb::kThreads3, 1) ppo_grad_bf16_kernel(const 
           for (int j = 0; j < 2; ++j) {
             const uint4 g = g1[2 * c + j];
             float* z = v + 8 * j;
-#if DRONECU_S5_BF16MUL
-            *reinterpret_cast<uint4*>(rowA + (2 * c + j) * kGrp) =
-                make_uint4(mul_bf16x2(pack_bf16(z[0], z[1]), g.x), mul_bf16x2(pack_bf16(z[2], z[3]), g.y),
-                           mul_bf16x2(pack_bf16(z[4], z[5]), g.z), mul_bf16x2(pack_bf16(z[6], z[7]), g.w));
-            continue;
-#endif
+            // fp32 products, one rounding to bf16 (a bf16 product of bf16(dH1) and the stash measured slower and less accurate)
             mul2(z[0], z[1], bf16_lo(g.x), bf16_hi(g.x));
             mul2(z[2], z[3], bf16_lo(g.y), bf16_hi(g.y));
             mul2(z[4], z[5], bf16_lo(g.z), bf16_hi(g.z));
             mul2(z[6], z[7], bf16_lo(g.w), bf16_hi(g.w));
-            const uint4 pk = make_uint4(pack_bf16(z[0], z[1]), pack_bf16(z[2], z[3]), pack_bf16(z[4], z[5]), pack_bf16(z[6], z[7]));
-#if DRONECU_S5_SPLIT
-            // dZ1 goes over H1 in bufA: wait (as late as possible) until the weight-gradient half of S5 has read it
-            if (c == 0 && j == 0) { mbar_wait(doneW, phW); phW ^= 1; fence_after(); }
-#endif
-            *reinterpret_cast<uint4*>(rowA + (2 * c + j) * kGrp) = pk;
+            *reinterpret_cast<uint4*>(rowA + (2 * c + j) * kGrp) =
+                make_uint4(pack_bf16(z[0], z[1]), pack_bf16(z[2], z[3]), pack_bf16(z[4], z[5]), pack_bf16(z[6], z[7]));
           }
           if (c < 3) ld_fence(w);
         }

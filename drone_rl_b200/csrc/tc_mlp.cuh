@@ -65,38 +65,12 @@ __device__ __forceinline__ float tanh_mufu(float x) {
   return y;
 }
 
-// Experiment (VERDICT r01 item 6; profiles/README.md): the rollout kernel is bound by the MUFU pipe (256 tanh per env-step at
-// 16 / clk / SM), so a share of the activations can be evaluated on the FMA pipe instead: odd minimax polynomial
-// x q(x^2) of degree 17 on [-3.75, 3.75] (input clamped; max abs error 5.9e-4, the size of tanh.approx's own 2^-11), two
-// activations per packed instruction: 4 FMNMX + 10 FFMA2 / FMUL2 per pair.  DRONECU_TANH_POLY_PAIRS = pairs per 16-wide chunk
-// that take this route (0 = all MUFU).
-#ifndef DRONECU_TANH_POLY_PAIRS
-#define DRONECU_TANH_POLY_PAIRS 0
-#endif
-__device__ __forceinline__ void tanh_poly2(float& x0, float& x1) {
-  constexpr float L = 3.75f;
-  const float a = fminf(fmaxf(x0, -L), L), b = fminf(fmaxf(x1, -L), L);
-  float t0 = a, t1 = b;
-  mul2(t0, t1, a, b);
-  float q0 = 1.370740944e-08f, q1 = 1.370740944e-08f;
-  constexpr float c[8] = {9.968600950e-01f, -3.149698032e-01f, 1.002266090e-01f, -2.373800408e-02f, 3.820229060e-03f,
-                          -3.979489950e-04f, 2.547277998e-05f, -9.067762226e-07f};
-#pragma unroll
-  for (int k = 7; k >= 0; --k) {                 // q = q * t + c[k]
-    uint64_t d;
-    asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(d) : "l"(pk2(q0, q1)), "l"(pk2(t0, t1)), "l"(pk2(c[k], c[k])));
-    upk2(d, q0, q1);
-  }
-  mul2(q0, q1, a, b);
-  x0 = q0; x1 = q1;
-}
-// tanh of a 16-wide chunk in place: the first DRONECU_TANH_POLY_PAIRS pairs on the FMA pipe, the rest on MUFU
+// tanh of a 16-wide chunk in place on the MUFU pipe.  Evaluating a share of the activations as a packed odd polynomial on the
+// FMA pipe instead measured no faster (profiles/README.md): the MUFU pipe is not what a warp waits for, and the polynomial's
+// 7 issue slots per activation (against 1) push the rollout kernel to the issue limit.
 __device__ __forceinline__ void tanh_chunk16(float (&v)[16]) {
 #pragma unroll
-  for (int i = 0; i < 16; i += 2) {
-    if (i < 2 * DRONECU_TANH_POLY_PAIRS) tanh_poly2(v[i], v[i + 1]);
-    else { v[i] = tanh_mufu(v[i]); v[i + 1] = tanh_mufu(v[i + 1]); }
-  }
+  for (int i = 0; i < 16; ++i) v[i] = tanh_mufu(v[i]);
 }
 
 // byte offset of element (n, k) of an [N x K] K-major operand in the canonical no-swizzle layout

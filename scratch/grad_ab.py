@@ -1,5 +1,6 @@
-"""A/B of gradient-kernel builds at the c5 size: time per 8.4M-sample minibatch (CUDA events, 5 rounds x 4 minibatches after a
-warm-up round), a hash of the gradient bits, the error against the fp32 CUDA-core kernel.
+"""A/B of gradient-kernel builds at the c5 size: time of the bf16 kernel per 8.4M-sample minibatch (CUDA events, 5 rounds x 4
+minibatches after a warm-up round), a hash of the gradient bits of each update precision (fp32, tf32, bf16), the error of the
+bf16 kernel against the fp32 CUDA-core kernel.
 usage: DRONECU_LIB=path/to/lib.so python scratch/grad_ab.py [n_envs] [K] [minibatches]"""
 import sys, os, hashlib, ctypes as C, numpy as np, torch
 sys.path.insert(0, '.')
@@ -25,13 +26,16 @@ for rnd in range(6):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(); launch(k, "bf16"); e1.record(); torch.cuda.synchronize()
         if rnd: times.append(e0.elapsed_time(e1))
-h = hashlib.sha256()
+hs = {p: hashlib.sha256() for p in ("fp32", "tf32", "bf16")}
 errs = []
 for k in range(mb):
-    launch(k, "bf16"); torch.cuda.synchronize(); g16 = g.cpu().numpy().copy()
-    launch(k, "fp32"); torch.cuda.synchronize(); g32 = g.cpu().numpy().copy()
-    h.update(g16.tobytes())
-    errs.append(float(np.abs(g16[:10697] - g32[:10697]).max() / np.abs(g32[:10697]).max()))
+    gk = {}
+    for p, h in hs.items():
+        launch(k, p); torch.cuda.synchronize(); gk[p] = g.cpu().numpy().copy()
+        h.update(gk[p].tobytes())
+    g16, g32 = gk["bf16"][:10697], gk["fp32"][:10697]
+    errs.append(float(np.abs(g16 - g32).max() / np.abs(g32).max()))
 t = np.array(times)
 print(f"{os.environ.get('DRONECU_LIB', 'libdronecu.so'):44s} grad+reduce {t.mean():.4f} ms (min {t.min():.4f}, max {t.max():.4f}) per {m} samples | "
-      f"sha256 {h.hexdigest()[:16]} | max err vs fp32 / max|g| {max(errs):.2e}", flush=True)
+      + " | ".join(f"sha256 {p} {h.hexdigest()[:16]}" for p, h in hs.items())
+      + f" | max err vs fp32 / max|g| {max(errs):.2e}", flush=True)
