@@ -21,7 +21,7 @@ arithmetic is float64, only the observation is cast to float32 (drone.py:79).
 """
 from __future__ import annotations
 
-from dataclasses import dataclass
+from dataclasses import dataclass, replace
 
 import numpy as np
 
@@ -55,20 +55,74 @@ SINGLE = Spec("single", 15, 200, 0.05, True, True, False, True)
 VECTOR = Spec("vector", 12, 1000, 1.0, False, False, True, False)
 
 
+@dataclass(frozen=True)
+class Params:
+    """Every constant of the env, field for field as ``EnvConfig`` (drone_rl_b200/core.py) holds them; the defaults are
+    the reference's literals (drone.py:21-43, :57-73, :147-156) and ``SINGLE``'s epilogue.  ``randomized`` selects the
+    Philox start with the curriculum target (drone.py:57-73) over ``fixed_start`` / ``fixed_target``
+    (vectorized_drone.py:30,50); ``auto_reset`` the DummyVecEnv reset on done."""
+    dt: float = DT
+    mass: float = MASS
+    gravity: float = GRAVITY
+    inertia: tuple = tuple(INERTIA.tolist())
+    arm_length: float = ARM_LENGTH
+    k_yaw: float = K_YAW
+    reward_scale: float = 0.01
+    bonus_radius: float = 0.05
+    bonus: float = 1.0
+    z_floor: float = 0.0
+    r_max: float = 50.0
+    fixed_target: tuple = (0.0, 0.0, 10.0)
+    fixed_start: tuple = (0.1, 0.1, 0.1)
+    start_z: float = 1.0
+    target_z: float = 1.0
+    curriculum_step: float = 0.1
+    curriculum_period: int = 2000
+    max_steps: int = 200
+    obs_dim: int = 15
+    randomized: bool = True
+    auto_reset: bool = True
+
+    @property
+    def motor_max(self):
+        return 3 * self.mass * self.gravity / 4.0      # drone.py:263
+
+    @classmethod
+    def of(cls, spec=None, **kw):
+        """A ``Params`` as it is, or the one of a ``Spec`` (default constants), with ``kw`` replaced."""
+        if spec is None:
+            spec = SINGLE
+        if isinstance(spec, Params):
+            return replace(spec, **kw) if kw else spec
+        base = dict(obs_dim=spec.obs_dim, max_steps=spec.max_steps, bonus_radius=spec.bonus_radius,
+                    randomized=spec.random_start, auto_reset=spec.auto_reset)
+        base.update(kw)
+        return cls(**base)
+
+    @classmethod
+    def from_config(cls, cfg):
+        """The record of an ``EnvConfig`` (any object with its attribute names)."""
+        return cls(**{f: (tuple(getattr(cfg, f)) if isinstance(getattr(cfg, f), (tuple, list)) else getattr(cfg, f))
+                      for f in cls.__dataclass_fields__})
+
+
+DEFAULT = Params()
+
+
 # ----------------------------------------------------------------------------------------
 # physics: one batched Euler step
 # ----------------------------------------------------------------------------------------
-def rotor_mix(action):
+def rotor_mix(action, p=DEFAULT):
     """Thrust and body torques from the four motor forces.
 
     drone.py:106-117 / vectorized_drone.py:154-166.  ``action`` float64 [B,4].
     """
     f1, f2, f3, f4 = action[:, 0], action[:, 1], action[:, 2], action[:, 3]
     thrust = np.sum(action, axis=1)
-    lever = ARM_LENGTH / np.sqrt(2)
+    lever = p.arm_length / np.sqrt(2)
     tau_roll = lever * (f1 + f2 - f3 - f4)
     tau_pitch = lever * (-f1 + f2 + f3 - f4)
-    tau_yaw = K_YAW * (f1 - f2 + f3 - f4)
+    tau_yaw = p.k_yaw * (f1 - f2 + f3 - f4)
     return thrust, tau_roll, tau_pitch, tau_yaw
 
 
@@ -112,22 +166,24 @@ def euler_rates(euler, omega):
     return np.einsum("bij,bj->bi", tm, omega)
 
 
-def dynamics_step(pos, vel, euler, omega, action, dt=DT):
+def dynamics_step(pos, vel, euler, omega, action, dt=None, p=DEFAULT):
     """One step of the reference integrator; returns NEW arrays (inputs untouched).
 
     Order (drone.py:119-139 / vectorized_drone.py:168-197): acceleration from the OLD
     attitude; v += a dt; p += v_new dt (semi-implicit); euler += T(old euler) old_omega dt;
-    omega += omega_dot(old omega) dt.
+    omega += omega_dot(old omega) dt.  ``dt`` (default ``p.dt``) overrides the record's step.
     """
+    dt = p.dt if dt is None else dt
+    inertia = np.asarray(p.inertia, dtype=np.float64)
     action = np.asarray(action, dtype=np.float64)
-    thrust, tau_roll, tau_pitch, tau_yaw = rotor_mix(action)
+    thrust, tau_roll, tau_pitch, tau_yaw = rotor_mix(action, p)
     n = action.shape[0]
 
     rot = body_to_inertial(euler)
     thrust_body = np.zeros((n, 3))
     thrust_body[:, 2] = thrust
     thrust_world = np.einsum("bij,bj->bi", rot, thrust_body)
-    accel = np.tile(np.array([0, 0, -GRAVITY]), (n, 1)) + (thrust_world / MASS)
+    accel = np.tile(np.array([0, 0, -p.gravity]), (n, 1)) + (thrust_world / p.mass)
 
     vel = vel + accel * dt
     pos = pos + vel * dt
@@ -135,23 +191,24 @@ def dynamics_step(pos, vel, euler, omega, action, dt=DT):
     new_euler = euler + euler_rates(euler, omega) * dt
 
     wdot = np.empty_like(omega)
-    wdot[:, 0] = (tau_roll - (INERTIA[1] - INERTIA[2]) * omega[:, 1] * omega[:, 2]) / INERTIA[0]
-    wdot[:, 1] = (tau_pitch - (INERTIA[2] - INERTIA[0]) * omega[:, 0] * omega[:, 2]) / INERTIA[1]
-    wdot[:, 2] = (tau_yaw - (INERTIA[0] - INERTIA[1]) * omega[:, 0] * omega[:, 1]) / INERTIA[2]
+    wdot[:, 0] = (tau_roll - (inertia[1] - inertia[2]) * omega[:, 1] * omega[:, 2]) / inertia[0]
+    wdot[:, 1] = (tau_pitch - (inertia[2] - inertia[0]) * omega[:, 0] * omega[:, 2]) / inertia[1]
+    wdot[:, 2] = (tau_yaw - (inertia[0] - inertia[1]) * omega[:, 0] * omega[:, 1]) / inertia[2]
     new_omega = omega + wdot * dt
     return pos, vel, new_euler, new_omega
 
 
-def reward_and_crash(pos, target, bonus_radius):
+def reward_and_crash(pos, target, bonus_radius, p=DEFAULT):
     """reward (float64 [B]) and the crash/out-of-range flag (bool [B]).
 
     drone.py:142-148,154 / vectorized_drone.py:204-207,211.  NaN position -> both
-    comparisons False -> not crashed.
+    comparisons False -> not crashed.  ``bonus_radius`` overrides ``p.bonus_radius`` (None: the record's).
     """
+    bonus_radius = p.bonus_radius if bonus_radius is None else bonus_radius
     dist = np.linalg.norm(pos - target, axis=1)
-    reward = -0.01 * dist
-    reward[dist < bonus_radius] += 1
-    crashed = (pos[:, 2] < 0) | (np.linalg.norm(pos, axis=1) > 50)
+    reward = -p.reward_scale * dist
+    reward[dist < bonus_radius] += p.bonus
+    crashed = (pos[:, 2] < p.z_floor) | (np.linalg.norm(pos, axis=1) > p.r_max)
     return reward, crashed
 
 
@@ -163,18 +220,33 @@ def build_obs(pos, vel, euler, omega, target, obs_dim):
     return np.concatenate(parts, axis=1).astype(np.float32)
 
 
-def curriculum_eps(ep_num):
+def curriculum_eps(ep_num, period=2000, step=0.1):
     """eps after the reset that made the episode counter ``ep_num`` (drone.py:61,68-70).
 
     The reference accumulates ``eps += 0.1`` each time ep_num hits a multiple of 2000, in
     float64 (0.1, 0.2, 0.30000000000000004, ...): reproduce the accumulation, not 0.1*n.
+    One sequential float64 sum up to the largest bump count, read off at every distinct count
+    (an ep_num of 2^31 - 1 at period 1 takes 2^31 additions).
     """
     ep_num = np.asarray(ep_num)
-    bumps = ep_num // 2000
+    bumps = ep_num // period
     out = np.zeros(ep_num.shape, dtype=np.float64)
-    for k in range(int(bumps.max()) if bumps.size else 0):
-        out = np.where(bumps > k, out + 0.1, out)
+    eps, done = 0.0, 0
+    for b in np.unique(bumps):
+        eps, done = _accumulate(eps, step, int(b) - done), int(b)
+        out[bumps == b] = eps
     return out
+
+
+def _accumulate(eps, step, count, chunk=1 << 22):
+    """((eps + step) + step) + ... with ``count`` float64 additions in order (ufunc.accumulate is sequential)."""
+    while count > 0:
+        m = min(count, chunk)
+        a = np.full(m + 1, step, dtype=np.float64)
+        a[0] = eps
+        eps = float(np.add.accumulate(a)[-1])
+        count -= m
+    return eps
 
 
 # ----------------------------------------------------------------------------------------
@@ -188,14 +260,16 @@ class BatchedDroneOracle:
     the Philox stream keyed by (seed, global id, ep_num) -- see oracle/philox.py.
     """
 
-    def __init__(self, n_envs, spec=SINGLE, seed=0, env_offset=0, dt=DT):
-        self.n, self.spec, self.seed, self.dt = int(n_envs), spec, int(seed), dt
+    def __init__(self, n_envs, spec=SINGLE, seed=0, env_offset=0, dt=None):
+        """``spec``: a ``Spec`` (the reference's constants) or a ``Params`` record; ``dt`` overrides its step."""
+        self.p = Params.of(spec) if dt is None else Params.of(spec, dt=dt)
+        self.n, self.spec, self.seed, self.dt = int(n_envs), spec, int(seed), self.p.dt
         self.env_ids = np.arange(env_offset, env_offset + self.n, dtype=np.uint64)
         self.pos = np.zeros((self.n, 3))
         self.vel = np.zeros((self.n, 3))
         self.euler = np.zeros((self.n, 3))
         self.omega = np.zeros((self.n, 3))
-        self.target = np.tile(np.array([0.0, 0.0, 10.0]), (self.n, 1))  # vectorized_drone.py:30
+        self.target = np.tile(np.array(self.p.fixed_target, dtype=np.float64), (self.n, 1))  # vectorized_drone.py:30
         self.step_count = np.zeros(self.n, dtype=np.int64)
         self.ep_num = np.zeros(self.n, dtype=np.int64)
         # VecMonitor accumulators (SURVEY.md appendix C)
@@ -213,19 +287,19 @@ class BatchedDroneOracle:
         self.omega[rows] = 0.0
         self.ep_num[rows] += 1
         self.step_count[rows] = 0
-        if self.spec.random_start:
+        p = self.p
+        if p.randomized:
             u = philox.reset_uniforms(self.seed, self.env_ids[rows], self.ep_num[rows])
             self.pos[rows, 0] = u[0] - 0.5
             self.pos[rows, 1] = u[1] - 0.5
-            self.pos[rows, 2] = 1.0
-        else:
-            self.pos[rows] = np.array([0.1, 0.1, 0.1])
-        if self.spec.curriculum:
-            eps = curriculum_eps(self.ep_num[rows])
+            self.pos[rows, 2] = p.start_z
+            eps = curriculum_eps(self.ep_num[rows], p.curriculum_period, p.curriculum_step)
             self.target[rows, 0] = eps * u[2]
             self.target[rows, 1] = eps * u[3]
-            self.target[rows, 2] = eps * u[4] + 1.0 + 0
-        # VECTOR: target stays [0,0,10]
+            self.target[rows, 2] = eps * u[4] + p.target_z + 0
+        else:
+            self.pos[rows] = np.array(p.fixed_start, dtype=np.float64)
+            self.target[rows] = np.array(p.fixed_target, dtype=np.float64)   # VECTOR: [0,0,10]
 
     def reset(self, mask=None):
         rows = np.arange(self.n) if mask is None else np.flatnonzero(np.asarray(mask))
@@ -235,7 +309,7 @@ class BatchedDroneOracle:
         return self.obs()
 
     def obs(self):
-        return build_obs(self.pos, self.vel, self.euler, self.omega, self.target, self.spec.obs_dim)
+        return build_obs(self.pos, self.vel, self.euler, self.omega, self.target, self.p.obs_dim)
 
     # -- state injection for teacher-forced tests ---------------------------------------------
     def set_state(self, pos=None, vel=None, euler=None, omega=None, target=None,
@@ -259,10 +333,10 @@ class BatchedDroneOracle:
         """
         with np.errstate(all="ignore"):
             self.pos, self.vel, self.euler, self.omega = dynamics_step(
-                self.pos, self.vel, self.euler, self.omega, action, self.dt)
-            reward, crashed = reward_and_crash(self.pos, self.target, self.spec.bonus_radius)
+                self.pos, self.vel, self.euler, self.omega, action, self.dt, self.p)
+            reward, crashed = reward_and_crash(self.pos, self.target, None, self.p)
             self.step_count += 1                                   # drone.py:155 / vec :200
-            timeout = self.step_count >= self.spec.max_steps        # drone.py:156 / vec :212
+            timeout = self.step_count >= self.p.max_steps           # drone.py:156 / vec :212
             done = crashed | timeout
             obs = self.obs()
         info = {"terminated": crashed.copy(), "truncated": timeout & ~crashed,
@@ -272,11 +346,11 @@ class BatchedDroneOracle:
         self.ep_length += 1
         info["episode_r"] = self.ep_return.copy()
         info["episode_l"] = self.ep_length.copy()
-        if self.spec.auto_reset:
-            rows = np.flatnonzero(done)
-            if rows.size:
-                self._reset_rows(rows)
-                self.ep_return[rows] = 0.0
-                self.ep_length[rows] = 0
-                obs = self.obs()
+        # VecMonitor zeroes its accumulators on every done, whether or not the env resets
+        rows = np.flatnonzero(done)
+        self.ep_return[rows] = 0.0
+        self.ep_length[rows] = 0
+        if self.p.auto_reset and rows.size:
+            self._reset_rows(rows)
+            obs = self.obs()
         return obs, reward, done, info

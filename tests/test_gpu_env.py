@@ -424,26 +424,35 @@ def test_full_size_rollout_properties(drl):
 
 def test_chunked_host_step_equals_device_step(drl):
     """dronecu_step_host cuts large batches into 1M-env chunks on two streams (H2D / kernel / D2H
-    overlap); the result must be bit-identical to the single device-pointer launch, ragged tail included."""
+    overlap); the result must be bit-identical to the single device-pointer launch, ragged tail included.
+    Both specs, the 15-dim auto-resetting one and the 12-dim fixed-start one, 2 steps short of their time
+    limit, so the chunks carry timeouts with and without a reset."""
     n = (1 << 21) + 1000
     rng = np.random.default_rng(3)
     acts = rng.uniform(0, 7.3575, (n, 4)).astype(np.float32)
-    venv = drl.DroneVecEnv(n, seed=9, info_mode="arrays", copy=False)
-    ref = drl.DroneBatch(n, drl.EnvConfig.single(), seed=9)
-    o_h = venv.reset().copy()
-    o_d = ref.reset()
-    assert np.array_equal(o_h, o_d.cpu().numpy())
     a_dev = torch.from_numpy(acts).cuda()
-    for _ in range(3):
-        obs, rew, done, info = venv.step(acts)
-        out = ref.step(a_dev, want_truncated=True)
-        assert np.array_equal(obs, out["obs"].cpu().numpy())
-        assert np.array_equal(rew, out["reward"].cpu().numpy())
-        assert np.array_equal(done, out["done"].cpu().numpy().astype(bool))
-        assert np.array_equal(info["truncated"], out["truncated"].cpu().numpy().astype(bool))
-    assert venv.batch.global_step == ref.global_step == 3
-    assert venv.episode_stats()["env_steps"] == 3 * n
-    venv.close(); ref.close()
+    for cfg in (drl.EnvConfig.single(), drl.EnvConfig.vector()):
+        venv = drl.DroneVecEnv(n, seed=9, info_mode="arrays", copy=False, config=cfg)
+        ref = drl.DroneBatch(n, cfg, seed=9)
+        o_h = venv.reset().copy()
+        o_d = ref.reset()
+        assert np.array_equal(o_h, o_d.cpu().numpy())
+        for b in (venv.batch, ref):
+            b.set_state(step=np.full(n, cfg.max_steps - 2, np.int32))
+        n_done = 0
+        for _ in range(3):
+            obs, rew, done, info = venv.step(acts)
+            out = ref.step(a_dev, want_truncated=True)
+            assert np.array_equal(obs, out["obs"].cpu().numpy())
+            assert np.array_equal(rew, out["reward"].cpu().numpy())
+            assert np.array_equal(done, out["done"].cpu().numpy().astype(bool))
+            assert np.array_equal(info["truncated"], out["truncated"].cpu().numpy().astype(bool))
+            n_done += int(done.sum())
+        assert n_done > 0
+        assert venv.batch.global_step == ref.global_step == 3
+        assert venv.episode_stats()["env_steps"] == 3 * n
+        assert venv.episode_stats()["episodes"] == ref.episode_stats()["episodes"] == n_done
+        venv.close(); ref.close()
 
 
 @pytest.mark.parametrize("scale", [1.0, 50.0, 3e3, 1.0e5, 1.056e5, 1.0e7, 5.0e8, 1.05e9, 3.0e9, 1.0e15])
