@@ -191,8 +191,8 @@ extern "C" int dronecu_norm_pass(int device, const dronecu_norm_pass_args* p, vo
   if (p->d_obs && p->obs_stride == 16 && (reinterpret_cast<uintptr_t>(p->d_obs) & 15))
     return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: padded d_obs must be 16-byte aligned");
   if (p->d_obs && !p->d_affine) return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: d_obs needs d_affine");
-  if (p->d_reward && (!p->d_done || !p->d_stats || (p->update && !p->d_returns)))
-    return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: d_reward needs d_done, d_stats and (update) d_returns");
+  if (p->d_reward && (!p->d_done || !p->d_stats || !p->d_returns))
+    return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: d_reward needs d_done, d_stats and d_returns");
   if (p->update && (!p->d_stats || !p->d_partials)) return fail(DRONECU_ERR_INVALID, "dronecu_norm_pass: update needs d_stats and d_partials");
   DeviceGuard guard(device);
   NormPassArgs a;

@@ -28,9 +28,13 @@ constexpr int kNormBlock = 256;               // envs per CTA of the pass (one p
 constexpr int kNormReduceThreads = 1024;
 
 // THE normalisation of one observation value: every rollout kernel and the pass call this, with explicit round-to-nearest
-// subtract and multiply so that no call site can contract them into an FMA and round differently.
+// subtract and multiply so that no call site can contract them into an FMA and round differently.  The clip is np.clip's:
+// NaN stays NaN (max.NaN / min.NaN; fmaxf / fminf would return the other operand, -clip), +-inf goes to +-clip.
 __device__ __forceinline__ float norm_obs1(float x, float mean, float rstd, float clip) {
-  return fminf(fmaxf(__fmul_rn(__fsub_rn(x, mean), rstd), -clip), clip);
+  float y = __fmul_rn(__fsub_rn(x, mean), rstd);
+  asm("max.NaN.f32 %0, %0, %1;" : "+f"(y) : "f"(-clip));
+  asm("min.NaN.f32 %0, %0, %1;" : "+f"(y) : "f"(clip));
+  return y;
 }
 
 // a [31]-float affine record staged in shared memory (s) applied to an observation row in registers.  Volatile reads: the
@@ -83,7 +87,7 @@ __global__ void __launch_bounds__(kNormBlock, 2) obs_norm_pass_kernel(const __gr
   if (active) {
     const size_t n = (size_t)A.n;
     const double rden = do_rew ? sqrt(A.stats[2 * kObs + 2] + A.epsilon) : 1.0;
-    double ret = (do_rew && upd) ? A.returns[i] : 0.0;
+    double ret = do_rew ? A.returns[i] : 0.0;
     for (int k = 0; k < A.K; ++k) {
       const size_t row = (size_t)k * n + (size_t)i;
       if (do_obs) {
@@ -123,11 +127,12 @@ __global__ void __launch_bounds__(kNormBlock, 2) obs_norm_pass_kernel(const __gr
           const double d = ret - s_c[kObs];
           r1 += d; r2 = fma(d, d, r2);
         }
-        A.reward[row] = (float)fmin(fmax(r / rden, -A.clip_reward), A.clip_reward);
-        if (A.done[row]) ret = 0.0;
+        const double q = r / rden;                   // np.clip: NaN stays NaN (fmax / fmin would return the bound)
+        A.reward[row] = (float)(q != q ? q : fmin(fmax(q, -A.clip_reward), A.clip_reward));
+        if (A.done[row]) ret = 0.0;                  // SB3 step_wait: returns[dones] = 0, training or not
       }
     }
-    if (do_rew && upd) A.returns[i] = ret;
+    if (do_rew) A.returns[i] = ret;
   }
   if (!upd) return;
   // warp shuffle -> CTA (fixed order) -> one partial record per CTA
@@ -179,7 +184,8 @@ __global__ void __launch_bounds__(kNormReduceThreads) obs_norm_reduce_kernel(con
 // sums s1 = sum(x - c), s2 = sum((x - c)^2) over cb values, c == mean (the shift the pass read)
 __device__ __forceinline__ void rms_combine(double& mean, double& var, const double count, double s1, double s2, double cb) {
   const double delta = s1 / cb;                                    // batch_mean - mean
-  const double var_b = fmax(s2 / cb - delta * delta, 0.0);         // population variance of the batch
+  const double v = s2 / cb - delta * delta;                        // population variance of the batch, clamped at 0 but
+  const double var_b = v < 0.0 ? 0.0 : v;                          // kept NaN (inf - inf) as np.var's NaN (fmax: 0)
   const double tot = count + cb;
   const double m2 = var * count + var_b * cb + delta * delta * count * cb / tot;
   mean = mean + delta * cb / tot;

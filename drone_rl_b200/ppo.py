@@ -278,7 +278,8 @@ class PPO:
 
     @property
     def training(self) -> bool:
-        """False (evaluation): the rollout keeps normalising but leaves the statistics and per-env returns unchanged."""
+        """False (evaluation): the rollout keeps normalising but leaves the statistics unchanged and does not advance the
+        per-env returns; as in SB3, a return is still zeroed where its episode ends."""
         return True if self.normalizer is None else self.normalizer.training
 
     @training.setter

@@ -247,7 +247,8 @@ int dronecu_gae(int device, int K, int64_t n, const float* d_reward, const float
  *   dronecu_norm_combine                         parallel-variance update of the statistics, next affine record
  * Layouts (device memory):
  *   affine  float32 [31]: mean_f[15] | rstd_f[15] | clip_obs;  x_norm = min(max((x - mean_f) * rstd_f, -clip), clip) with
- *           a round-to-nearest subtract and multiply (no FMA), rstd_f = (float)(1 / sqrt(var + epsilon))
+ *           a round-to-nearest subtract and multiply (no FMA), rstd_f = (float)(1 / sqrt(var + epsilon)); the clip keeps
+ *           NaN (np.clip), for the observations and the rewards alike
  *   stats   float64 [34]: obs_mean[15] | obs_var[15] | obs_count | ret_mean | ret_var | ret_count  (SB3 RunningMeanStd;
  *           initial state mean 0, var 1, count 1e-4)
  *   moments float64 [34]: sum(x - c)[15] | sum((x - c)^2)[15] | obs count | sum(ret - c_r) | sum((ret - c_r)^2) | return
@@ -272,11 +273,12 @@ typedef struct dronecu_norm_pass_args {
   int64_t n;
   const float* d_affine;    /* [31] the record the rollout used (required with d_obs)                                       */
   float* d_reward;          /* [K,n] raw in, out clip(r / sqrt(ret_var + epsilon), +-clip_reward) (float64, then cast); NULL: off */
-  const uint8_t* d_done;    /* [K,n] the per-env return restarts after done                                                 */
-  double* d_returns;        /* [n] per-env discounted return ret = ret * gamma + r, persistent across rollouts                */
+  const uint8_t* d_done;    /* [K,n] the per-env return restarts after done (in both modes, as SB3's returns[dones] = 0)     */
+  double* d_returns;        /* [n] per-env discounted return ret = ret * gamma + r, persistent across rollouts (required with d_reward) */
   const double* d_stats;    /* [34] running statistics (moment shift, reward scale)                                         */
   double gamma, epsilon, clip_reward;
-  int32_t update;           /* != 0 (training): returns advance, d_partials written; 0 (evaluation): statistics untouched   */
+  int32_t update;           /* != 0 (training): returns advance, d_partials written; 0 (evaluation): statistics untouched,
+                               returns only zeroed at dones                                                                 */
   int32_t side_env;         /* >= 0 with d_side_obs: copy that env's raw rows to d_side_obs [K,15] before normalising       */
   float* d_side_obs;
   double* d_partials;       /* [ceil(n / DRONECU_NORM_BLOCK), DRONECU_NORM_MOMENTS] scratch, one record per CTA (update != 0) */

@@ -63,6 +63,119 @@ def normalize_obs_f32(obs, rms: RunningMeanStd, clip_obs: float = 10.0, epsilon:
     return np.clip(y.astype(np.float32), np.float32(-clip_obs), np.float32(clip_obs))
 
 
+def normalize_reward_f32(rew, ret_var, clip_reward: float = 10.0, epsilon: float = 1e-8) -> np.ndarray:
+    """The pass's reward: float32(clip(float64(r) / sqrt(ret_var + eps), +-clip_reward)).  Double sqrt and / are correctly
+    rounded, so the kernel and numpy agree bit for bit; np.clip keeps NaN."""
+    q = np.asarray(rew, np.float32).astype(np.float64) / np.sqrt(np.float64(ret_var) + np.float64(epsilon))
+    return np.clip(q, -clip_reward, clip_reward).astype(np.float32)
+
+
+REDUCE_GROUPS = 30      # obs_norm_reduce_kernel: 1024 threads // 34 columns
+
+
+def reduce_partials(partials) -> np.ndarray:
+    """obs_norm_reduce_kernel's fixed order restated: group g sums the records p = g, g + 30, ... in that order (from 0.0),
+    then the 30 group sums are added in order.  Plain float64 additions: bit-identical to the kernel."""
+    p = np.asarray(partials, np.float64)
+    groups = np.zeros((REDUCE_GROUPS, p.shape[1]))
+    for q0 in range(0, p.shape[0], REDUCE_GROUPS):
+        blk = p[q0:q0 + REDUCE_GROUPS]
+        groups[:blk.shape[0]] = groups[:blk.shape[0]] + blk
+    out = np.zeros(p.shape[1])
+    for g in range(REDUCE_GROUPS):
+        out = out + groups[g]
+    return out
+
+
+U64 = 2.0 ** -53
+
+
+def gamma_n(k) -> float:
+    """Higham's gamma_k = k u / (1 - k u): the relative error bound of k float64 roundings in a row."""
+    return k * U64 / (1.0 - k * U64)
+
+
+def combine_bound(mean, var, count, s1, s2, cb):
+    """Bound on |kernel - SB3 update_from_moments| for the (mean, var) after merging one batch given by its shifted sums
+    s1 = sum(x - mean), s2 = sum((x - mean)^2) over cb values.  SB3's side receives batch_mean = mean + s1 / cb and
+    batch_var = s2 / cb - (s1 / cb)^2; the kernel uses delta = s1 / cb directly and nvcc may contract its products and sums
+    into FMAs.  Both evaluations are within the forward error of the exact result, so the bound is twice that:
+        delta:  |e_d| <= u (|mean| + 3 |delta|)                (SB3's batch_mean - mean round trip; the kernel's is u |delta|)
+        delta^2:      <= 2 |delta| e_d + 3 u delta^2
+        mean'   = mean + delta cb / tot:      gamma_4 (|mean| + |delta|) + e_d
+        var'    = (T1 + T2 + T3) / tot, T1 = var count, T2 = var_b cb, T3 = delta^2 count cb / tot:
+                  [gamma_6 (T1 + T2 + T3 + s2) + (cb + count cb / tot) e_d2] / tot
+    Returns (bound on mean', bound on var'), elementwise."""
+    mean, var, s1, s2 = (np.asarray(a, np.float64) for a in (mean, var, s1, s2))
+    delta = s1 / cb
+    var_b = np.maximum(s2 / cb - delta * delta, 0.0)
+    tot = count + cb
+    e_d = U64 * (np.abs(mean) + 3 * np.abs(delta))
+    e_d2 = 2 * np.abs(delta) * e_d + 3 * U64 * delta * delta
+    b_mean = gamma_n(4) * (np.abs(mean) + np.abs(delta)) + e_d
+    t1, t2, t3 = var * count, var_b * cb, delta * delta * count * cb / tot
+    b_var = (gamma_n(6) * (t1 + t2 + t3 + s2) + (cb + count * cb / tot) * e_d2) / tot
+    return 2 * b_mean, 2 * b_var
+
+
+def combine_sb3(rms: RunningMeanStd, s1, s2, cb):
+    """SB3 update_from_moments fed with the batch moments of the shifted sums (shift = rms.mean)."""
+    delta = np.asarray(s1, np.float64) / cb
+    rms.update_from_moments(rms.mean + delta, np.maximum(np.asarray(s2, np.float64) / cb - delta * delta, 0.0), cb)
+
+
+def two_pass_moments(x):
+    """(batch mean, population variance) of the rows of x in two passes, as np.mean / np.var take them, but summed in
+    extended precision along a contiguous axis (numpy's pairwise summation): np.mean(axis=0) of a C-ordered [N, F] array
+    adds the N rows one after another, an error of N float64 roundings that would swamp the kernel's.  What is left is
+    the final rounding to float64 plus ~(log2 N + 20) roundings of the extended type (ref_depth)."""
+    x = np.asarray(x, np.float64)
+    n = x.shape[0]
+    xt = np.ascontiguousarray(x.reshape(n, -1).T).astype(np.longdouble)
+    m = xt.sum(axis=1) / n
+    v = np.square(xt - m[:, None]).sum(axis=1) / n
+    shape = x.shape[1:]
+    return m.astype(np.float64).reshape(shape), v.astype(np.float64).reshape(shape)
+
+
+def ref_depth(cb) -> float:
+    """two_pass_moments' own error in float64 roundings (the pairwise blocks of 128, then log2 levels, in long double)"""
+    return 1 + (np.log2(max(cb, 2.0)) + 20) * float(np.finfo(np.longdouble).eps) / (2 * U64)
+
+
+def one_pass_bound(mean, var, count, s2, cb, depth: int):
+    """Bound on |kernel - SB3 update_from_moments(two_pass_moments(data))| for the (mean, var) after one rollout: the
+    kernel's batch moments come from one pass of shifted sums.  Each of the cb shifted values d = x - c carries one
+    rounding; s1 and s2 are sums of depth = K + 5 + 8 + ceil(P / 30) + 30 additions deep at most (each env's K steps, the
+    warp shuffle tree, the 8-warp fold, then the reduce's P / 30 records per group and its 30 groups), so
+        |e_s2| <= gamma_{depth + 3} s2,  |e_s1| <= gamma_{depth + 1} sum|d| <= gamma_{depth + 1} sqrt(cb s2)
+    and the shifted one-pass formula var_b = s2 / cb - delta^2 inherits
+        |e_var_b| <= gamma_{depth + 4} (s2 / cb) + 2 |delta| |e_delta| <= gamma_{depth + 4} (2 s2 / cb + delta^2)
+    (Cauchy-Schwarz: sum|d| / cb <= sqrt(s2 / cb); 2 a b <= a^2 + b^2).  This is relative to the spread about the shift,
+    not to var_b: with the initial statistics (shift 0) and features far from zero it is the cancellation of the one-pass
+    formula, |e_var_b| ~ gamma (s2 / cb + delta^2).  The reference's batch mean is rounded to float64 and SB3 subtracts
+    the running mean from it (the |mean| term of e_delta); its own summation error adds ref_depth(cb) roundings.
+    Propagated through the combine (var_b enters with weight cb / tot, delta^2 with count cb / tot^2, delta with
+    cb / tot), plus the combine's own rounding (combine_bound), with |delta| <= sqrt(s2 / cb) throughout.  Returns
+    (bound on mean', bound on var')."""
+    mean, var, s2 = (np.asarray(a, np.float64) for a in (mean, var, s2))
+    g = gamma_n(depth + 4 + ref_depth(cb))
+    d_max = np.sqrt(s2 / cb)                            # |delta| <= sqrt(s2 / cb): the batch mean lies inside the spread
+    e_delta = g * (d_max + np.abs(mean))
+    e_d2 = (2 * d_max + e_delta) * e_delta              # |(delta + e)^2 - delta^2|: a constant column has s2 = 0, but
+    e_var_b = g * (2 * s2 / cb + d_max * d_max) + e_d2  # its float64 batch mean minus the shift need not be 0
+    tot = count + cb
+    c_mean, c_var = combine_bound(mean, var, count, d_max * cb, s2, cb)
+    return (e_delta * cb / tot + c_mean,
+            (e_var_b * cb + e_d2 * count * cb / tot) / tot + c_var)
+
+
+def pass_depth(K: int, n: int) -> int:
+    """The deepest chain of additions behind one moment: K steps, 5 shuffle levels, the 8-warp fold, the reduce."""
+    P = -(-n // 256)
+    return K + 5 + 8 + -(-P // REDUCE_GROUPS) + REDUCE_GROUPS
+
+
 class FrozenVecNormalize:
     """VecNormalize with the statistics frozen per rollout.  ``apply(obs, rew, done)`` takes one rollout's RAW [K,n,15]
     observations (the rows the policy acted on), [K,n] rewards and dones; returns the normalised observations and rewards

@@ -268,7 +268,7 @@ def _spy(model):
     return raw
 
 
-def test_ppo_statistics_follow_the_oracle(drl, tmp_path):
+def test_ppo_statistics_and_evaluation_returns_follow_the_oracle(drl, tmp_path):
     from drone_rl_b200.ppo import PPO
     n, K = 256, 32
     model = PPO(drl.DroneBatch(n, drl.EnvConfig.single(), seed=2), n_steps=K, batch_size=2048, n_epochs=2, seed=2,
@@ -291,11 +291,14 @@ def test_ppo_statistics_follow_the_oracle(drl, tmp_path):
         model.train()
         l0 = model.launches
     assert model.obs_rms.count == pytest.approx(3 * n * K + 1e-4)
-    # evaluation: statistics and per-env returns unchanged
+    # evaluation: statistics unchanged, per-env returns not advanced but zeroed where an episode ended (SB3 step_wait)
     model.training = False
     before = (model.normalizer.stats.clone(), model.normalizer.returns.clone())
     model.collect_rollouts()
-    assert torch.equal(before[0], model.normalizer.stats) and torch.equal(before[1], model.normalizer.returns)
+    ended = model.buf.done.bool().any(0)
+    assert bool(ended.any())
+    assert torch.equal(before[0], model.normalizer.stats)
+    assert torch.equal(model.normalizer.returns, torch.where(ended, torch.zeros_like(before[1]), before[1]))
     model.training = True
     # checkpoints: statistics, per-env returns (same shard), identical predict
     obs = np.random.default_rng(0).normal(0, 5, (64, 15)).astype(np.float32)

@@ -64,6 +64,9 @@ def test_frozen_vec_normalize_uses_previous_statistics():
     before = (vn.obs_rms.mean.copy(), vn.ret_rms.var, vn.returns.copy())
     vn.apply(obs, rew, done)
     assert np.array_equal(before[0], vn.obs_rms.mean) and before[1] == vn.ret_rms.var
+    # evaluation: the returns are not advanced, but an env whose episode ended restarts from 0 (SB3 step_wait)
+    assert done.any(0).any()
+    assert np.array_equal(vn.returns, np.where(done.any(0), 0.0, before[2]))
 
 
 def test_norm_pass_args_mirror_matches_header(tmp_path):
@@ -88,3 +91,107 @@ def test_ppo_loop_oracle_normalisation_is_opt_in():
     b.train()                                          # the update runs on the normalised buffer
     # the buffer holds normalised observations (positions of up to 50 m clipped at 10)
     assert float(b.buf[0].abs().max()) <= 10.0 < float(a.buf[0].abs().max())
+
+
+def test_reward_formula_is_float64_then_float32_with_np_clip():
+    import math
+    rng = np.random.default_rng(5)
+    r = np.concatenate([rng.normal(0, 0.3, 200), [np.nan, np.inf, -np.inf, 3.4028235e38, -0.0]]).astype(np.float32)
+    got = no.normalize_reward_f32(r, 0.0123, clip_reward=2.0, epsilon=1e-3)
+    for x, y in zip(r, got):
+        q = float(x) / math.sqrt(0.0123 + 1e-3)
+        want = q if math.isnan(q) else min(max(q, -2.0), 2.0)
+        assert (math.isnan(want) and math.isnan(y)) or np.float32(want).tobytes() == y.tobytes()
+    assert got.dtype == np.float32 and np.isnan(got[200]) and got[201] == 2 and got[202] == -2
+
+
+@pytest.mark.parametrize("P", [1, 29, 30, 31, 4097])
+def test_reduce_order_restates_the_kernel_loop(P):
+    rng = np.random.default_rng(P)
+    parts = rng.normal(0, 1, (P, 34)) * 10.0 ** rng.integers(-8, 8, (P, 34))
+    got = no.reduce_partials(parts)
+    for j in (0, 17, 33):               # thread (g, j): p = g, g + 30, ...; then the 30 group sums in order, from 0.0
+        groups = []
+        for g in range(30):
+            t = 0.0
+            for p in range(g, P, 30):
+                t += float(parts[p, j])
+            groups.append(t)
+        t = 0.0
+        for v in groups:
+            t += v
+        assert got[j] == t
+
+
+def _exact_combine(mean, var, count, xs):
+    """SB3 update with the batch's exact mean and population variance, in rational arithmetic"""
+    from fractions import Fraction as F
+    xs = [F(float(x)) for x in xs]
+    cb = len(xs)
+    bm = sum(xs) / cb
+    bv = sum((x - bm) ** 2 for x in xs) / cb
+    m, v, c = F(float(mean)), F(float(var)), F(float(count))
+    d = bm - m
+    tot = c + cb
+    return float(m + d * cb / tot), float((v * c + bv * cb + d * d * c * cb / tot) / tot)
+
+
+@pytest.mark.parametrize("shift,count", [(0.0, 1e-4), (0.9, 50.0), (0.0, 1e12), (1.0, 3.0)])
+def test_combine_and_one_pass_bounds_hold(shift, count):
+    """The float64 one-pass shifted evaluation (the kernel's) and SB3's combine on two_pass_moments, each within half the
+    stated bound of the exact rational result; the initial statistics put the shift far from data at 7e3 +- 1."""
+    rng = np.random.default_rng(int(count) % 97)
+    xs = 7e3 + rng.normal(0, 1, 2000)
+    mean, var = shift * 7e3, 4.0
+    exact_m, exact_v = _exact_combine(mean, var, count, xs)
+    d = xs - mean
+    s1, s2 = 0.0, 0.0
+    for v in d:                                      # sequential: depth = cb
+        s1 += v
+        s2 += v * v
+    cb = float(len(xs))
+    bm, bv = no.combine_bound(mean, var, count, s1, s2, cb)
+    r = no.RunningMeanStd(())
+    r.mean, r.var, r.count = np.float64(mean), np.float64(var), count
+    no.combine_sb3(r, s1, s2, cb)
+    om, ov = no.one_pass_bound(mean, var, count, s2, cb, depth=len(xs))
+    assert abs(r.mean - exact_m) <= om / 2 + bm / 2 and abs(r.var - exact_v) <= ov / 2 + bv / 2
+    r2 = no.RunningMeanStd(())
+    r2.mean, r2.var, r2.count = np.float64(mean), np.float64(var), count
+    r2.update_from_moments(*no.two_pass_moments(xs), cb)
+    assert abs(r2.mean - exact_m) <= om / 2 and abs(r2.var - exact_v) <= ov / 2
+    if shift == 0.0 and count < 1:   # the one-pass cancellation is visible, and the bound is not a relative one
+        assert abs(r.var - exact_v) > 1e-15 * exact_v
+
+
+def _lib_or_skip():
+    from drone_rl_b200 import _lib
+    try:
+        return _lib, _lib.load()
+    except Exception as e:          # noqa: BLE001  (no built library: the build step reports that)
+        pytest.skip(f"libdronecu.so not loadable: {e}")
+
+
+def test_norm_entry_points_reject_bad_arguments_without_launching():
+    """Every check runs before the device is touched, so these return DRONECU_ERR_INVALID with or without a GPU."""
+    _lib, lib = _lib_or_skip()
+    P = lambda v: C.c_void_p(v)
+
+    def args(**kw):
+        a = _lib.NormPassArgs()
+        a.d_obs, a.obs_stride, a.K, a.n, a.d_affine = 4096, 16, 4, 100, 8192
+        a.d_reward, a.d_done, a.d_returns, a.d_stats = 12288, 16384, 20480, 24576
+        a.update, a.d_partials, a.side_env, a.epsilon, a.clip_reward = 1, 28672, -1, 1e-8, 10.0
+        for k, v in kw.items():
+            setattr(a, k, v)
+        return a
+    bad = [dict(obs_stride=14), dict(obs_stride=16, d_obs=4100), dict(d_done=None), dict(d_stats=None),
+           dict(d_returns=None), dict(d_returns=None, update=0), dict(d_partials=None), dict(n=0), dict(n=-3),
+           dict(K=0), dict(K=-1), dict(d_affine=None)]
+    for kw in bad:
+        assert lib.dronecu_norm_pass(0, C.byref(args(**kw)), None) == -1, kw
+    assert lib.dronecu_norm_pass(0, None, None) == -1
+    for npart in (0, -1):
+        assert lib.dronecu_norm_reduce(0, P(4096), npart, P(8192), None) == -1
+    for eps, clip in ((-1e-8, 10.0), (float("nan"), 10.0), (1e-8, 0.0), (1e-8, -1.0), (1e-8, float("nan"))):
+        assert lib.dronecu_norm_combine(0, P(4096), None, eps, clip, P(8192), None) == -1, (eps, clip)
