@@ -77,6 +77,82 @@ def episodes_from_transitions(reward, done, n_eval_episodes: int):
     return returns, lengths, T
 
 
+def shard_targets(n_eval_episodes: int, env_index0: int, n_global: int, n: int):
+    """the targets of the n envs of one shard: env i is env ``env_index0 + i`` of the ``n_global`` evaluation envs"""
+    return (int(n_eval_episodes) + int(env_index0) + np.arange(n, dtype=np.int64)) // int(n_global)
+
+
+def launch_sequence(reward, done, targets, launches, max_eps: int, ep_ret0=None, ep_len0=None):
+    """The launch contract of ``dronecu_evaluate_policy`` (csrc/ppo_eval.cuh) restated over a record: ``reward`` float32
+    [T, n] and ``done`` bool [T, n] of the n envs stepped from the evaluation's first step, ``targets`` [n],
+    ``launches`` a list of (limit, catch_up), ``ep_ret0`` / ``ep_len0`` the running return and length of every env at
+    the first step (default 0: a fresh reset).
+
+    One launch steps env i from ``steps[i]`` while ``steps[i] < limit`` and (catch-up or ``count[i] < target[i]``);
+    step c adds reward[c] to the float32 running return and 1 to the length, and on done[c] records (return, length) in
+    slot ``count[i]`` if ``count[i] < target[i]`` (then ``count[i] += 1``) and zeroes both.  A probe adds to ``pending``
+    the envs still below target; a catch-up leaves it alone.
+
+    Returns ``(after, ep_return, ep_length, written)``: ``after`` one dict of ``steps``, ``count`` and ``pending`` (None
+    for a catch-up) per launch; ``ep_return`` float32 / ``ep_length`` int [n, max_eps] with ``written`` [n, max_eps] bool
+    the slots the launches wrote.  ValueError if a launch needs a step past the end of the record."""
+    reward, done = np.asarray(reward, np.float32), np.asarray(done, bool)
+    T, n = reward.shape
+    targets = np.asarray(targets, np.int64)
+    ret = np.zeros(n, np.float32) if ep_ret0 is None else np.asarray(ep_ret0, np.float32).copy()
+    length = np.zeros(n, np.int64) if ep_len0 is None else np.asarray(ep_len0, np.int64).copy()
+    steps, count = np.zeros(n, np.int64), np.zeros(n, np.int64)
+    ep_return, ep_length = np.zeros((n, max_eps), np.float32), np.zeros((n, max_eps), np.int64)
+    written = np.zeros((n, max_eps), bool)
+    after = []
+    for limit, catch_up in launches:
+        lo = int(steps.min()) if n else 0
+        for c in range(lo, max(lo, int(limit))):
+            going = bool(catch_up) | (count < targets)
+            if not (going & (steps >= c)).any():
+                break
+            live = going & (steps == c)
+            if not live.any():
+                continue
+            if c >= T:
+                raise ValueError(f"launch to step {limit} needs step {c}, past the end of the record ({T} steps)")
+            ret[live] = (ret[live] + reward[c, live]).astype(np.float32)
+            length[live] += 1
+            end = live & done[c]
+            rec = np.flatnonzero(end & (count < targets))
+            ep_return[rec, count[rec]] = ret[rec]
+            ep_length[rec, count[rec]] = length[rec]
+            written[rec, count[rec]] = True
+            count[rec] += 1
+            ret[end], length[end] = 0.0, 0
+            steps[live] += 1
+        after.append({"steps": steps.copy(), "count": count.copy(),
+                      "pending": None if catch_up else int((count < targets).sum())})
+    return after, ep_return, ep_length, written
+
+
+def episode_lists(count, ep_return, ep_length, env_index0: int = 0, ep_len0=None):
+    """The rows of a shard's slots as ``evaluation.evaluate_policy`` forms them: (step of completion, global env index,
+    return, length) of every recorded episode, env by env.  ``ep_len0``: the running lengths at the first step (default
+    0); slots past ``count`` are not read."""
+    count = np.asarray(count, np.int64)
+    n, max_eps = np.shape(ep_length)
+    len0 = np.zeros(n, np.int64) if ep_len0 is None else np.asarray(ep_len0, np.int64)
+    env = np.repeat(np.arange(n), count)
+    j = np.arange(env.size) - np.repeat(np.cumsum(count) - count, count)
+    ln = np.where(np.arange(max_eps) < count[:, None], np.asarray(ep_length, np.int64), 0)
+    done_at = np.cumsum(ln, axis=1)[env, j] - len0[env]
+    return (done_at.tolist(), (env + int(env_index0)).tolist(), np.asarray(ep_return, np.float32)[env, j].tolist(),
+            ln[env, j].tolist())
+
+
+def sb3_order(*shard_rows):
+    """SB3's lists from the rows of every shard: by step of completion, then by global env index"""
+    rows = [[x for r in shard_rows for x in r[k]] for k in range(4)]
+    order = np.lexsort((np.asarray(rows[1], np.int64), np.asarray(rows[0], np.int64)))
+    return [rows[2][j] for j in order], [int(rows[3][j]) for j in order]
+
+
 class OracleDroneGymEnv:
     """One float64 oracle env with the legacy gym API of ``DroneGymEnv`` (no auto-reset: DummyVecEnv resets it), global id
     ``env_id`` of the Philox streams.  The constructor resets once, as ``DroneGymEnv.__init__`` does."""

@@ -1,12 +1,8 @@
-"""GPU tests of policy evaluation (csrc/ppo_eval.cuh, drone_rl_b200/evaluation.py).
-
-Each evaluation kernel is checked against its rollout counterpart: two envs with the same seed, offset and clock; one is
-evaluated, the other runs dronecu_rollout_policy[_tc|_norm] for the same T steps recording rewards and done flags, whose
-transitions go through the SB3 bookkeeping of oracle/eval_oracle.py.  Same arithmetic on the same operands, so the
-episode returns must agree bit for bit as float32, the lengths and T exactly, and both envs must end in bit-identical
-states at the same clock.
+"""GPU tests of policy evaluation (csrc/ppo_eval.cuh, drone_rl_b200/evaluation.py) as the training loop uses it: the
+model, its normaliser and its env are left untouched, EvalCallback inside PPO.learn, the train.py driver's eval keys,
+the argument checks, and two ranks against one.  Every evaluation kernel against its rollout twin and float64, over
+launch shapes, splits, probe chunks and configs: tests/test_gpu_eval_parity.py.
 """
-import ctypes as C
 import os
 import socket
 
@@ -16,10 +12,9 @@ import pytest
 torch = pytest.importorskip("torch")
 pytestmark = pytest.mark.gpu
 
-from oracle import eval_oracle as eo  # noqa: E402
 from oracle import ppo_oracle as po  # noqa: E402
 
-SEED, OFFSET = 13, 5
+SEED = 13
 
 
 @pytest.fixture(scope="module")
@@ -29,14 +24,6 @@ def drl():
     import drone_rl_b200
     import drone_rl_b200.ppo  # noqa: F401
     return drone_rl_b200
-
-
-@pytest.fixture
-def rollout_kernel_mode():
-    from drone_rl_b200 import _lib
-    lib = _lib.load()
-    yield lambda mode: _lib.check(lib.dronecu_set_rollout_kernel(mode))
-    lib.dronecu_set_rollout_kernel(0)
 
 
 def _model(drl, precision="fp32", norm=False, device=0):
@@ -57,72 +44,6 @@ def _model(drl, precision="fp32", norm=False, device=0):
         model.normalizer.stats.copy_(s)
         model.normalizer._combine(None)
     return model
-
-
-def _rollout_record(drl, model, env, T, deterministic):
-    """T steps of the same-flavour rollout kernel on `env`: reward and done [T, n]."""
-    from drone_rl_b200 import _lib
-    n = env.n
-    rew = torch.empty(T, n, device="cuda")
-    done = torch.empty(T, n, dtype=torch.uint8, device="cuda")
-    out = _lib.PolicyOut(None, None, None, None, rew.data_ptr(), done.data_ptr(), None, None, 0, 0)
-    tc = int(model.rollout_precision == "tf32" and n > model.tc_min_envs)
-    aff = model.normalizer.affine_ptr() if model.normalizer is not None else None
-    _lib.check(model.lib.dronecu_rollout_policy_norm(env._h, T, C.c_void_p(model.params.data_ptr()), int(deterministic),
-                                                     C.byref(out), aff, tc, None))
-    torch.cuda.synchronize()
-    return rew.cpu().numpy(), done.cpu().numpy().astype(bool)
-
-
-def _check_against_rollout(drl, model, n, n_eval, deterministic):
-    from drone_rl_b200.evaluation import evaluate_policy
-    ev = drl.DroneBatch(n, drl.EnvConfig.single(), seed=SEED, env_offset=OFFSET)
-    ro = drl.DroneBatch(n, drl.EnvConfig.single(), seed=SEED, env_offset=OFFSET)
-    for b in (ev, ro):           # same, non-zero clock
-        b.global_step = 1000
-    t0 = ev.global_step
-    rewards, lengths = evaluate_policy(model, ev, n_eval, deterministic=deterministic, return_episode_rewards=True)
-    T = ev.global_step - t0
-    assert len(rewards) == n_eval and T > 0
-    ro.reset()
-    rew, done = _rollout_record(drl, model, ro, T, deterministic)
-    ref_r, ref_l, ref_T = eo.episodes_from_transitions(rew, done, n_eval)
-    assert ref_T == T
-    assert np.array_equal(np.array(rewards, np.float32), np.array(ref_r, np.float32)) and rewards == ref_r
-    assert lengths == ref_l
-    assert ro.global_step == ev.global_step
-    sa, sb = ev.get_state(), ro.get_state()
-    for k in sa:
-        assert np.array_equal(sa[k].view(np.uint32) if sa[k].dtype == np.float32 else sa[k],
-                              sb[k].view(np.uint32) if sb[k].dtype == np.float32 else sb[k]), k
-    mean, std = evaluate_policy(model, ro, n_eval, deterministic=deterministic)
-    assert np.isfinite(mean) and std >= 0
-    ev.close(); ro.close()
-    return rewards, lengths, T
-
-
-@pytest.mark.parametrize("norm", [False, True])
-@pytest.mark.parametrize("deterministic", [True, False])
-@pytest.mark.parametrize("kernel", ["thread_per_env", "warp_per_env", "tensor_cores"])
-def test_eval_equals_rollout(drl, rollout_kernel_mode, kernel, deterministic, norm):
-    tc = kernel == "tensor_cores"
-    if not tc:
-        rollout_kernel_mode({"thread_per_env": 1, "warp_per_env": 2}[kernel])
-    # tensor cores: 1500 envs = 11 full tiles and a partial one; 2000 episodes = targets of 1 and 2
-    n, n_eval = (1500, 2000) if tc else (300, 450)
-    model = _model(drl, "tf32" if tc else "fp32", norm)
-    _check_against_rollout(drl, model, n, n_eval, deterministic)
-    model.close()
-
-
-@pytest.mark.parametrize("n,n_eval", [(1, 7), (64, 10), (64, 64), (64, 100)])
-def test_eval_targets_and_chunks(drl, monkeypatch, n, n_eval):
-    from drone_rl_b200 import evaluation
-    monkeypatch.setattr(evaluation, "PROBE_CHUNK", 50)        # several probe launches per evaluation
-    model = _model(drl)
-    _, lengths, T = _check_against_rollout(drl, model, n, n_eval, True)
-    assert T > 50 or n > 1
-    model.close()
 
 
 def test_eval_leaves_the_model_untouched(drl):

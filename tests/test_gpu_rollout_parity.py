@@ -1,7 +1,8 @@
 """Every in-kernel policy rollout kernel -- thread per env, warp per env, tensor cores (csrc/ppo_rollout.cuh,
-csrc/ppo_rollout_tc.cuh) -- teacher-forced against float64 over a covering design of launch shapes, start states,
-clocks, modes, normalisation, row layouts and policies.  Every level of every factor appears, and every level of
-every other factor appears with every kernel.
+csrc/ppo_rollout_tc.cuh), each instantiated for RANDOMIZED x NORM -- teacher-forced against float64 over a covering
+design of launch shapes, start states, clocks, modes, normalisation, row layouts, policies, env constants and start
+kinds (Philox or fixed).  Every level of every factor appears, and every level of every other factor appears with every
+kernel.
 
 Checked at every (step, env):
   env transition      obs / reward / done / last_obs / auto-resets through oracle/verify.check_rollout (clipped actions)
@@ -32,9 +33,9 @@ from oracle import philox, ppo_oracle as po, verify  # noqa: E402
 from oracle.tc_bound import tc_forward_bound  # noqa: E402
 
 SEED = 21
-MOTOR_MAX = np.float32(7.3575)
 HALF_LOG_2PI = np.float32(0.91893853320467274178)
 KERNELS = ("thread", "warp", "tc")
+CONFIGS = ("single", "A", "B")                  # the constant sets of tests/test_gpu_env_parity.py
 NS = (1, 31, 33, 127, 129, 1000, 1025, 2049, 4097, 8193)
 
 
@@ -55,16 +56,24 @@ def rollout_kernel_mode():
     lib.dronecu_set_rollout_kernel(0)
 
 
-def _policy(kind):
+def make_config(drl, name, randomized=True):
+    from tests.test_gpu_env_parity import CONFIG_KW
+    return drl.EnvConfig.single(**CONFIG_KW[name], obs_dim=15, randomized=randomized, auto_reset=True)
+
+
+def _policy(kind, motor_max=do.MOTOR_MAX):
     """hover: the policy of tests/test_gpu_ppo.py (mean near hover thrust); wide: three times its perturbation and a
-    positive log_std, so sampled actions cross both clip limits."""
+    positive log_std, so sampled actions cross both clip limits.  Under other constants the action bias and the std
+    scale with motor_max (hover thrust is motor_max / 3 in every config); the default constants give the same bits."""
     g = torch.Generator().manual_seed(5)
     flat = po.init_params(5, dtype=torch.float64) + (0.03 if kind == "hover" else 0.09) * torch.randn(
         po.N_PARAMS, generator=g, dtype=torch.float64)
+    scale = motor_max / do.MOTOR_MAX
     off = po.offsets()["pi.b3"][0]
-    flat[off:off + 4] = 2.45 if kind == "hover" else 3.5
+    flat[off:off + 4] = (2.45 if kind == "hover" else 3.5) * scale
     off = po.offsets()["log_std"][0]
-    flat[off:off + 4] = torch.tensor([-0.5, -0.2, 0.1, -1.0] if kind == "hover" else [0.5, 0.7, 0.4, 0.6], dtype=torch.float64)
+    flat[off:off + 4] = torch.tensor([-0.5, -0.2, 0.1, -1.0] if kind == "hover" else [0.5, 0.7, 0.4, 0.6],
+                                     dtype=torch.float64) + np.log(scale)
     return flat.float().numpy()
 
 
@@ -121,10 +130,11 @@ def _launch(batch, kernel, K, theta_dev, det, stride, affine, set_mode):
 
 
 def _mid_episode(batch, rng):
-    """late steps (timeouts within 15 steps) and episode counters just below several curriculum bumps"""
-    n = batch.n
-    step = rng.integers(185, 200, n).astype(np.int32)
-    ep_num = rng.choice([5, 1999, 3999, 5998, 19999, 40001], n).astype(np.int32)
+    """late steps (timeouts within 15 steps) and episode counters just below several curriculum bumps of the config"""
+    n, cfg = batch.n, batch.config
+    ms, per = cfg.max_steps, cfg.curriculum_period
+    step = rng.integers(max(0, ms - 15), ms, n).astype(np.int32)
+    ep_num = rng.choice([5, per - 1, 2 * per - 1, 3 * per - 2, 10 * per - 1, 20 * per + 1], n).astype(np.int32)
     ep_ret = (-rng.uniform(0, 3, n)).astype(np.float32)
     batch.set_state(step=step, ep_num=ep_num, ep_len=step, ep_ret=ep_ret)
 
@@ -152,9 +162,31 @@ def _ratio(err, bound):
     return float(np.max(err / bound)) if err.size else 0.0
 
 
+def _same(a, b, what):
+    """bit-identical float32 tensors, except that any NaN matches any NaN"""
+    nan_a, nan_b = torch.isnan(a), torch.isnan(b)
+    bad = (nan_a != nan_b) | (~nan_a & ~nan_b & (a.view(torch.int32) != b.view(torch.int32)))
+    assert not bool(bad.any()), f"{what}: {int(bad.sum())} of {a.numel()} elements differ, first at flat index " \
+                                f"{int(torch.nonzero(bad.reshape(-1))[0])}"
+
+
+def _same_f32(a, b):
+    """numpy float32 arrays bit-identical, except that any NaN matches any NaN (NaN payloads differ between the device
+    and numpy)"""
+    a, b = np.asarray(a, np.float32), np.asarray(b, np.float32)
+    return a.shape == b.shape and bool(((a.view(np.uint32) == b.view(np.uint32)) | (np.isnan(a) & np.isnan(b))).all())
+
+
 def _check_record(batch, rec, theta, theta_dev, kernel, det, nz, st0, t0, cols=None):
-    """Every check of the module docstring on the envs `cols` (None = all).  Returns the worst err/bound per check."""
+    """Every check of the module docstring on the envs `cols` (None = all), under the constants of the batch's config.
+    Returns the worst err/bound per check.
+
+    A body left spinning without bound (large dt |dI / I| w^2 under wide actions) makes the env emit rows with huge,
+    inf or NaN features before its time limit (test_env_emits_non_finite_rows).  The comparisons with float64 skip the
+    rows the tower sees outside F32_SAFE (verify.py counts the same rows on the env side); on every row the fp32 kernels
+    still match policy_forward bit for bit (a NaN matching a NaN), and so do the tensor cores on rows without a NaN."""
     n = batch.n
+    spec = do.Params.from_config(batch.config)
     idx = torch.arange(n, device="cuda") if cols is None else cols
     g = lambda t: t[:, idx] if t.dim() >= 2 else t[idx]
     obs_d, act_d = g(rec["obs"]), g(rec["actions"])
@@ -166,33 +198,42 @@ def _check_record(batch, rec, theta, theta_dev, kernel, det, nz, st0, t0, cols=N
     pm, pv = _forward(theta_dev, xn, tc)
     _, plv = _forward(theta_dev, last_xn, tc)
     value, last_value = g(rec["value"]).reshape(-1), rec["last_value"][idx]
+    ok = (xn.abs() <= verify.F32_SAFE).all(1)              # NaN fails the test too
+    last_ok = (last_xn.abs() <= verify.F32_SAFE).all(1)
     worst = {}
     # mean and value against policy_forward
     if kernel == "warp":
-        worst["value_vs_forward"] = max(float((value - pv).abs().max()), float((last_value - plv).abs().max())) / 1e-5
+        worst["value_vs_forward"] = max(float((value - pv)[ok].abs().max()) if ok.any() else 0.0,
+                                        float((last_value - plv)[last_ok].abs().max()) if last_ok.any() else 0.0) / 1e-5
         assert worst["value_vs_forward"] <= 1.0
         if det:
-            worst["mean_vs_forward"] = float((act_d.reshape(-1, 4) - pm).abs().max()) / 1e-5
+            worst["mean_vs_forward"] = (float((act_d.reshape(-1, 4) - pm)[ok].abs().max()) if ok.any() else 0.0) / 1e-5
             assert worst["mean_vs_forward"] <= 1.0
     else:
-        assert torch.equal(value, pv) and torch.equal(last_value, plv), "value differs from policy_forward"
+        rows = ~torch.isnan(xn).any(1) if tc else torch.ones_like(ok)        # tc_mlp.cuh: NaN rows are unspecified
+        last_rows = ~torch.isnan(last_xn).any(1) if tc else torch.ones_like(last_ok)
+        _same(value[rows], pv[rows], "value vs policy_forward")
+        _same(last_value[last_rows], plv[last_rows], "last value vs policy_forward")
         if det:
-            assert torch.equal(act_d.reshape(-1, 4), pm), "deterministic action differs from policy_forward"
-    # policy_forward against the oracle
-    x64 = xn.cpu().numpy()
+            _same(act_d.reshape(-1, 4)[rows], pm[rows], "deterministic action vs policy_forward")
+    # policy_forward against the oracle, on the rows in float32 range
+    okh, last_okh = ok.cpu().numpy(), last_ok.cpu().numpy()
+    x64 = xn.cpu().numpy()[okh]
     pm_h, pv_h = pm.cpu().double().numpy(), pv.cpu().double().numpy()
+    last64 = last_xn.cpu().numpy()[last_okh]
     if tc:
-        m_ref, v_ref, mb, vb = tc_forward_bound(theta, x64)
-        _, lv_ref, _, lvb = tc_forward_bound(theta, last_xn.cpu().numpy())
+        bound = lambda x: tc_forward_bound(theta, x) if len(x) else (np.zeros((0, 4)), np.zeros(0), np.zeros((0, 4)), np.zeros(0))
+        m_ref, v_ref, mb, vb = bound(x64)
+        _, lv_ref, _, lvb = bound(last64)
     else:
         th64 = torch.from_numpy(theta).double()
         m_ref, v_ref, _ = (t.numpy() for t in po.forward(th64, torch.from_numpy(x64).double()))
-        _, lv_ref, _ = (t.numpy() for t in po.forward(th64, last_xn.cpu().double()))
+        _, lv_ref, _ = (t.numpy() for t in po.forward(th64, torch.from_numpy(last64).double()))
         mb, vb, lvb = 2e-5 * np.maximum(1, np.abs(m_ref)), 2e-5 * np.maximum(1, np.abs(v_ref)), 2e-5 * np.maximum(1, np.abs(lv_ref))
-    worst["forward_vs_oracle"] = max(_ratio(np.abs(pm_h - m_ref), mb), _ratio(np.abs(pv_h - v_ref), vb),
-                                     _ratio(np.abs(plv.cpu().double().numpy() - lv_ref), lvb))
+    worst["forward_vs_oracle"] = max(_ratio(np.abs(pm_h[okh] - m_ref), mb), _ratio(np.abs(pv_h[okh] - v_ref), vb),
+                                     _ratio(np.abs(plv.cpu().double().numpy()[last_okh] - lv_ref), lvb))
     if kernel != "tc":      # the fp32 kernels' own record against the oracle as well
-        worst["fp32_value_vs_oracle"] = _ratio(np.abs(value.cpu().double().numpy() - v_ref), vb)
+        worst["fp32_value_vs_oracle"] = _ratio(np.abs(value.cpu().double().numpy()[okh] - v_ref), vb)
         assert worst["fp32_value_vs_oracle"] <= 1.0
     assert worst["forward_vs_oracle"] <= 1.0, f"policy_forward vs oracle: {worst['forward_vs_oracle']:.3g}"
     # action and log-prob
@@ -207,17 +248,18 @@ def _check_record(batch, rec, theta, theta_dev, kernel, det, nz, st0, t0, cols=N
     else:
         ids = batch.env_offset + idx.cpu().numpy().astype(np.uint64)
         std = np.exp(ls32.astype(np.float64))
-        mean_k = pm_h.reshape(K, m, 4)
+        mean_k, ok_k = pm_h.reshape(K, m, 4), okh.reshape(K, m)
         slack = 1e-5 if kernel == "warp" else 0.0
         wa, wl = 0.0, 0.0
         for k in range(K):
             z = philox.noise_normals(SEED, ids, t0 + k)
             ref_a = mean_k[k] + std * z
             ba = 2.0 ** -20 * std * np.abs(z) + 2.0 ** -24 * np.abs(act[k]) + slack + 1e-30
-            wa = max(wa, _ratio(np.abs(act[k] - ref_a), ba))
+            r = ok_k[k]
+            wa = max(wa, _ratio(np.abs(act[k] - ref_a)[r], ba[r]))
             ref_lp = -0.5 * (z * z).sum(1) - ls32.astype(np.float64).sum() - 2 * np.log(2 * np.pi)
             bl = 2.0 ** -19 * (0.5 * (z * z).sum(1) + np.abs(ls32).sum() + 4)
-            wl = max(wl, _ratio(np.abs(logp[k] - ref_lp), bl))
+            wl = max(wl, _ratio(np.abs(logp[k] - ref_lp)[r], bl[r]))
         worst["action"], worst["logp"] = wa, wl
         assert wa <= 1.0 and wl <= 1.0, f"action {wa:.3g} logp {wl:.3g}"
     # env transitions under the clipped actions
@@ -225,15 +267,16 @@ def _check_record(batch, rec, theta, theta_dev, kernel, det, nz, st0, t0, cols=N
     nxt = np.concatenate([o[1:], rec["last_obs"][idx].cpu().numpy()[None]], 0)
     reward, done = g(rec["reward"]).cpu().numpy(), g(rec["done"]).cpu().numpy().astype(bool)
     sub = {k: v[idx.cpu().numpy()] for k, v in st0.items()}
-    rep = verify.check_rollout(o[0], np.clip(act, 0, MOTOR_MAX), nxt, reward, done, spec=do.SINGLE, seed=SEED,
+    clipped = np.fmin(np.fmax(act, np.float32(0)), np.float32(spec.motor_max))     # fminf / fmaxf: a NaN action clips to 0
+    rep = verify.check_rollout(o[0], clipped, nxt, reward, done, spec=spec, seed=SEED,
                                env_ids=batch.env_offset + idx.cpu().numpy().astype(np.uint64),
-                               ep_num0=sub["ep_num"], step0=sub["step"])
+                               ep_num0=sub["ep_num"], step0=sub["step"], target0=sub["target"])
     worst["env"] = rep["worst_err_over_bound"]
     # state after the launch
     st1 = {k: v[idx.cpu().numpy()] for k, v in batch.get_state("step", "ep_num", "ep_len", "ep_ret").items()}
     step, ep_num, ep_len, ep_ret, rets, length_sum = _expected_after(sub, done, reward)
     assert np.array_equal(st1["step"], step) and np.array_equal(st1["ep_num"], ep_num) and np.array_equal(st1["ep_len"], ep_len)
-    assert np.array_equal(st1["ep_ret"].view(np.uint32), ep_ret.view(np.uint32)), "ep_ret is not the float32 replay"
+    assert _same_f32(st1["ep_ret"], ep_ret), "ep_ret is not the float32 replay"
     return worst, rep, done, rets, length_sum
 
 
@@ -249,14 +292,18 @@ def _check_stats(stats, done, rets, length_sum, rep):
     assert stats["truncated"] == stats["episodes"] - stats["terminated"]
     flat = [r for env in rets for r in env]
     ref = float(np.sum(np.asarray(flat, np.float64)))
+    if not np.isfinite(ref):            # a non-finite return: the same inf, or NaN, in any order
+        assert stats["return_sum"] == ref or (np.isnan(ref) and np.isnan(stats["return_sum"])), (stats["return_sum"], ref)
+        return
     tol = sum(max(len(env) - 1, 0) * 2.0 ** -24 * 1.01 * float(np.abs(np.asarray(env, np.float64)).sum()) for env in rets)
     tol += 1e-12 * (float(np.abs(np.asarray(flat, np.float64)).sum()) + 1.0)
     assert abs(stats["return_sum"] - ref) <= tol, f"return_sum {stats['return_sum']!r} vs {ref!r} (tol {tol:.3g})"
 
 
-def _design():
+def design():
     """10 cases per kernel, one per n; the other factors cycle with periods <= 4 from a per-kernel offset, so each
-    kernel meets every level of every factor."""
+    kernel meets every level of every factor, and each of its four RANDOMIZED x NORM instantiations runs at least
+    twice."""
     cases = []
     for ki, kernel in enumerate(KERNELS):
         for j, n in enumerate(NS):
@@ -264,18 +311,20 @@ def _design():
             K = (1, 40, 230)[r % 3]
             if n * K > 1_100_000:
                 K = 40
-            cases.append(pytest.param(kernel, n, K, ("fresh", "mid")[r % 2], (0, 12345)[(r // 2) % 2],
-                                      (0, 7 << 23)[((r + 1) // 2) % 2], (r % 4) in (1, 2), (r % 4) >= 2,
-                                      16 if r % 3 == 1 else 15, "wide" if r % 4 == 3 else "hover",
-                                      id=f"{kernel}-n{n}-K{K}-{('fresh', 'mid')[r % 2]}-gs{(0, 12345)[(r // 2) % 2]}"
-                                         f"-off{(0, 7 << 23)[((r + 1) // 2) % 2]}-{'det' if (r % 4) in (1, 2) else 'stoch'}"
-                                         f"-{'norm' if (r % 4) >= 2 else 'raw'}-s{16 if r % 3 == 1 else 15}"
-                                         f"-{'wide' if r % 4 == 3 else 'hover'}"))
+            cases.append(dict(kernel=kernel, n=n, K=K, start=("fresh", "mid")[r % 2], gs=(0, 12345)[(r // 2) % 2],
+                              off=(0, 7 << 23)[((r + 1) // 2) % 2], det=(r % 4) in (1, 2), norm=(r % 4) >= 2,
+                              stride=16 if r % 3 == 1 else 15, policy="wide" if r % 4 == 3 else "hover",
+                              cfg=CONFIGS[(j // 2 + ki) % 3], randomized=(r + r // 4) % 2 == 0))
     return cases
 
 
-def _setup(drl, n, start, gs, off, rng):
-    b = drl.DroneBatch(n, drl.EnvConfig.single(), seed=SEED, env_offset=off)
+def _case_id(c):
+    return (f"{c['kernel']}-n{c['n']}-K{c['K']}-{c['start']}-gs{c['gs']}-off{c['off']}-{'det' if c['det'] else 'stoch'}"
+            f"-{'norm' if c['norm'] else 'raw'}-s{c['stride']}-{c['policy']}-{c['cfg']}-{'rand' if c['randomized'] else 'fixed'}")
+
+
+def _setup(drl, n, start, gs, off, rng, cfg=None):
+    b = drl.DroneBatch(n, cfg or drl.EnvConfig.single(), seed=SEED, env_offset=off)
     b.reset()
     if start == "mid":
         _mid_episode(b, rng)
@@ -284,13 +333,16 @@ def _setup(drl, n, start, gs, off, rng):
     return b
 
 
-@pytest.mark.parametrize("kernel,n,K,start,gs,off,det,norm,stride,policy", _design())
-def test_rollout_parity(drl, rollout_kernel_mode, kernel, n, K, start, gs, off, det, norm, stride, policy):
+@pytest.mark.parametrize("case", design(), ids=_case_id)
+def test_rollout_parity(drl, rollout_kernel_mode, case):
+    kernel, n, K, start, gs, off, det, norm, stride, policy = (case[k] for k in (
+        "kernel", "n", "K", "start", "gs", "off", "det", "norm", "stride", "policy"))
+    cfg = make_config(drl, case["cfg"], case["randomized"])
     rng = np.random.default_rng(n * 7 + K)
-    theta = _policy(policy)
+    theta = _policy(policy, cfg.motor_max)
     theta_dev = torch.from_numpy(theta).cuda()
     nz = _norm_affine(n) if norm else None
-    b = _setup(drl, n, start, gs, off, rng)
+    b = _setup(drl, n, start, gs, off, rng, cfg)
     st0 = b.get_state()
     rec = _launch(b, kernel, K, theta_dev, det, stride, None if nz is None else nz.affine, rollout_kernel_mode)
     stats = b.episode_stats(reset=True)
@@ -299,11 +351,12 @@ def test_rollout_parity(drl, rollout_kernel_mode, kernel, n, K, start, gs, off, 
     _check_stats(stats, done, rets, length_sum, rep)
     if policy == "wide" and not det and n * K >= 1000:
         a = rec["actions"]
-        assert bool((a < 0).any()) and bool((a > float(MOTOR_MAX)).any()), "the wide policy must cross both clip limits"
+        assert bool((a < 0).any()) and bool((a > float(np.float32(cfg.motor_max))).any()), \
+            "the wide policy must cross both clip limits"
     if start == "mid" and K >= 15:
         assert rep["dones"] >= n, "every env reaches its time limit"
-    if K == 230:
-        assert (done.any(0)).all(), "every env ends an episode in 230 steps"
+    if K >= cfg.max_steps:
+        assert (done.any(0)).all(), f"every env ends an episode in {K} steps"
     if stride == 16:
         assert bool((rec["obs_store"][..., 15] == 1.0).all())
         # the packed run from the same state and clock: identical record
@@ -312,7 +365,7 @@ def test_rollout_parity(drl, rollout_kernel_mode, kernel, n, K, start, gs, off, 
         packed = _launch(b, kernel, K, theta_dev, det, 15, None if nz is None else nz.affine, rollout_kernel_mode)
         for key in ("obs", "actions", "logp", "value", "reward", "done", "last_value", "last_obs"):
             assert torch.equal(rec[key], packed[key]), key
-    print(f"{kernel} n={n} K={K}: worst err/bound " + ", ".join(f"{k} {v:.3g}" for k, v in worst.items())
+    print(f"{_case_id(case)}: worst err/bound " + ", ".join(f"{k} {v:.3g}" for k, v in worst.items())
           + f"; dones {rep['dones']}, terminated {stats['terminated']}, borderline {rep['borderline_done']}")
     b.close()
 
