@@ -82,6 +82,11 @@ class EvalArgs(C.Structure):
                 ("d_pending", C.c_void_p)]
 
 
+class TimeoutBuf(C.Structure):
+    """Mirror of ``dronecu_timeout_buf`` (include/dronecu.h)."""
+    _fields_ = [("d_obs", C.c_void_p), ("d_row", C.c_void_p), ("slots_per_env", C.c_int32)]
+
+
 NORM_AFFINE = 31
 NORM_STATS = 34
 NORM_MOMENTS = 34
@@ -129,6 +134,9 @@ _SIGNATURES = {
     "dronecu_rollout_policy_tc": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(PolicyOut), _P]),
     "dronecu_policy_forward_tc": (C.c_int, [C.c_int, C.c_int64, _P, _P, _P, _P, _P, _P, _P]),
     "dronecu_rollout_policy_norm": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(PolicyOut), _P, C.c_int, _P]),
+    "dronecu_rollout_policy_timeouts": (C.c_int, [_P, C.c_int, _P, C.c_int, C.POINTER(PolicyOut), _P, C.c_int,
+                                                  C.POINTER(TimeoutBuf), _P]),
+    "dronecu_bootstrap_timeouts": (C.c_int, [C.c_int, _P, C.POINTER(TimeoutBuf), C.c_int64, _P, C.c_float, _P, _P]),
     "dronecu_evaluate_policy": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(EvalArgs), _P]),
     "dronecu_norm_pass": (C.c_int, [C.c_int, C.POINTER(NormPassArgs), _P]),
     "dronecu_norm_reduce": (C.c_int, [C.c_int, _P, C.c_int64, _P, _P]),

@@ -12,6 +12,7 @@
 #include "env_handle.h"
 #include "ppo_update.cuh"
 #include "ppo_rollout_tc.cuh"
+#include "ppo_timeout.cuh"
 #include "ppo_eval.cuh"
 #include "ppo_update_tc.cuh"
 #include "ppo_update_tc3.cuh"
@@ -55,29 +56,50 @@ extern "C" int dronecu_set_rollout_kernel(int mode) {
 
 enum RolloutKernel { kThreadPerEnv, kWarpPerEnv, kTensorCores };
 
-template <bool RANDOMIZED, bool NORM>
+template <bool RANDOMIZED, bool NORM, bool TIMEOUT>
 static int launch_policy_rollout(RolloutKernel which, int64_t n, const PolicyArgs& a, cudaStream_t st) {
   if (which == kTensorCores) {
     static_assert(tc::kTile == kPolBlock, "tile size");
-    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_tc_kernel<RANDOMIZED, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem));
-    policy_rollout_tc_kernel<RANDOMIZED, NORM><<<(unsigned)((n + kPolBlock - 1) / kPolBlock), tc::kTile, kTcSmem, st>>>(a);
+    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_tc_kernel<RANDOMIZED, NORM, TIMEOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kTcSmem));
+    policy_rollout_tc_kernel<RANDOMIZED, NORM, TIMEOUT><<<(unsigned)((n + kPolBlock - 1) / kPolBlock), tc::kTile, kTcSmem, st>>>(a);
   } else if (which == kWarpPerEnv) {
-    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_warp_kernel<RANDOMIZED, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmallSmem));
-    policy_rollout_warp_kernel<RANDOMIZED, NORM><<<(unsigned)((n + kSmallWarps - 1) / kSmallWarps), 32 * kSmallWarps, kPolicySmallSmem, st>>>(a);
+    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_warp_kernel<RANDOMIZED, NORM, TIMEOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmallSmem));
+    policy_rollout_warp_kernel<RANDOMIZED, NORM, TIMEOUT><<<(unsigned)((n + kSmallWarps - 1) / kSmallWarps), 32 * kSmallWarps, kPolicySmallSmem, st>>>(a);
   } else {
-    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_kernel<RANDOMIZED, NORM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmem));
-    policy_rollout_kernel<RANDOMIZED, NORM><<<(unsigned)((n + kPolBlock - 1) / kPolBlock), kPolBlock, kPolicySmem, st>>>(a);
+    CUDA_TRY(cudaFuncSetAttribute(policy_rollout_kernel<RANDOMIZED, NORM, TIMEOUT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolicySmem));
+    policy_rollout_kernel<RANDOMIZED, NORM, TIMEOUT><<<(unsigned)((n + kPolBlock - 1) / kPolBlock), kPolBlock, kPolicySmem, st>>>(a);
   }
+  return DRONECU_OK;
+}
+
+template <bool TIMEOUT>
+static int launch_policy_rollout(RolloutKernel which, bool randomized, bool norm, int64_t n, const PolicyArgs& a, cudaStream_t st) {
+  if (norm) return randomized ? launch_policy_rollout<true, true, TIMEOUT>(which, n, a, st) : launch_policy_rollout<false, true, TIMEOUT>(which, n, a, st);
+  return randomized ? launch_policy_rollout<true, false, TIMEOUT>(which, n, a, st) : launch_policy_rollout<false, false, TIMEOUT>(which, n, a, st);
+}
+
+// the side buffer of the time-limit bootstrap: slots_per_env slots per env, 16-byte aligned 64-byte rows
+static int check_timeout_buf(const dronecu_timeout_buf* tb, const char* what) {
+  if (!tb || !tb->d_obs || !tb->d_row) return fail(DRONECU_ERR_INVALID, std::string(what) + ": null timeout buffer");
+  if (reinterpret_cast<uintptr_t>(tb->d_obs) & 15) return fail(DRONECU_ERR_INVALID, std::string(what) + ": timeout d_obs must be 16-byte aligned");
+  if (tb->slots_per_env <= 0) return fail(DRONECU_ERR_INVALID, std::string(what) + ": slots_per_env must be positive");
   return DRONECU_OK;
 }
 
 static int rollout_policy_impl(dronecu_env* e, int K, const float* d_params, int deterministic,
                                const dronecu_policy_out* out, void* stream, bool tensor_cores,
-                               const float* d_norm_affine = nullptr) {
+                               const float* d_norm_affine = nullptr, const dronecu_timeout_buf* tb = nullptr) {
   if (!e || !d_params) return fail(DRONECU_ERR_INVALID, "dronecu_rollout_policy: null argument");
   if (K <= 0) return fail(DRONECU_ERR_INVALID, "K must be positive");
   if (e->cfg.obs_dim != 15 || !(e->cfg.flags & DRONECU_AUTORESET))
     return fail(DRONECU_ERR_UNSUPPORTED, "policy rollout needs the 15-dim observation and DRONECU_AUTORESET");
+  if (tb) {
+    // an env truncates at most 1 + floor((K - 1) / max_steps) = ceil(K / max_steps) times in K steps, whatever its clock
+    if ((int64_t)tb->slots_per_env < ((int64_t)K + e->cfg.max_steps - 1) / e->cfg.max_steps)
+      return fail(DRONECU_ERR_INVALID, "dronecu_rollout_policy_timeouts: slots_per_env is below ceil(K / max_steps)");
+    if ((int64_t)K * e->n > INT32_MAX || (int64_t)tb->slots_per_env * e->n > INT32_MAX)
+      return fail(DRONECU_ERR_INVALID, "dronecu_rollout_policy_timeouts: K * n and slots_per_env * n must fit in int32");
+  }
   if (out && out->d_actions && (reinterpret_cast<uintptr_t>(out->d_actions) & 15))
     return fail(DRONECU_ERR_INVALID, "out->d_actions must be 16-byte aligned");
   if (out && out->obs_padded && out->d_obs && (reinterpret_cast<uintptr_t>(out->d_obs) & 15))
@@ -94,14 +116,14 @@ static int rollout_policy_impl(dronecu_env* e, int K, const float* d_params, int
     a.value = out->d_value; a.reward = out->d_reward; a.done = out->d_done; a.last_value = out->d_last_value;
     a.last_obs = out->d_last_obs;
   }
+  if (tb) { a.term_obs = tb->d_obs; a.term_row = tb->d_row; a.term_slots = tb->slots_per_env; }
   // small batches: one warp per env (ppo_rollout.cuh)
   const RolloutKernel which = tensor_cores ? kTensorCores
       : (g_rollout_kernel_mode == 2 || (g_rollout_kernel_mode == 0 && e->n <= kWarpRolloutMaxEnvs)) ? kWarpPerEnv : kThreadPerEnv;
   cudaStream_t st = (cudaStream_t)stream;
   const bool randomized = (e->cfg.flags & DRONECU_RANDOMIZED) != 0;
-  int rc;
-  if (d_norm_affine) rc = randomized ? launch_policy_rollout<true, true>(which, e->n, a, st) : launch_policy_rollout<false, true>(which, e->n, a, st);
-  else rc = randomized ? launch_policy_rollout<true, false>(which, e->n, a, st) : launch_policy_rollout<false, false>(which, e->n, a, st);
+  const int rc = tb ? launch_policy_rollout<true>(which, randomized, d_norm_affine != nullptr, e->n, a, st)
+                    : launch_policy_rollout<false>(which, randomized, d_norm_affine != nullptr, e->n, a, st);
   if (rc != DRONECU_OK) return rc;
   e->launches += 1;
   CUDA_TRY(cudaGetLastError());
@@ -124,6 +146,35 @@ extern "C" int dronecu_rollout_policy_norm(dronecu_env* e, int K, const float* d
                                            const dronecu_policy_out* out, const float* d_norm_affine, int tensor_cores,
                                            void* stream) {
   return rollout_policy_impl(e, K, d_params, deterministic, out, stream, tensor_cores != 0, d_norm_affine);
+}
+
+extern "C" int dronecu_rollout_policy_timeouts(dronecu_env* e, int K, const float* d_params, int deterministic,
+                                               const dronecu_policy_out* out, const float* d_norm_affine, int tensor_cores,
+                                               const dronecu_timeout_buf* tb, void* stream) {
+  const int rc = check_timeout_buf(tb, "dronecu_rollout_policy_timeouts");
+  if (rc != DRONECU_OK) return rc;
+  return rollout_policy_impl(e, K, d_params, deterministic, out, stream, tensor_cores != 0, d_norm_affine, tb);
+}
+
+extern "C" int dronecu_bootstrap_timeouts(int device, const float* d_params, const dronecu_timeout_buf* tb, int64_t n,
+                                          const float* d_norm_affine, float gamma, float* d_reward, void* stream) {
+  if (!d_params || !d_reward || n <= 0) return fail(DRONECU_ERR_INVALID, "dronecu_bootstrap_timeouts: bad argument");
+  const int rc = check_timeout_buf(tb, "dronecu_bootstrap_timeouts");
+  if (rc != DRONECU_OK) return rc;
+  DeviceGuard guard(device);
+  const int64_t slots = (int64_t)tb->slots_per_env * n;
+  const unsigned grid = (unsigned)std::min<int64_t>((slots + kPolBlock - 1) / kPolBlock, 148 * 4);
+  const float4* obs = reinterpret_cast<const float4*>(tb->d_obs);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (d_norm_affine) {
+    CUDA_TRY(cudaFuncSetAttribute(timeout_bootstrap_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(MlpSmem)));
+    timeout_bootstrap_kernel<true><<<grid, kPolBlock, sizeof(MlpSmem), st>>>(d_params, obs, tb->d_row, slots, d_norm_affine, gamma, d_reward);
+  } else {
+    CUDA_TRY(cudaFuncSetAttribute(timeout_bootstrap_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(MlpSmem)));
+    timeout_bootstrap_kernel<false><<<grid, kPolBlock, sizeof(MlpSmem), st>>>(d_params, obs, tb->d_row, slots, nullptr, gamma, d_reward);
+  }
+  CUDA_TRY(cudaGetLastError());
+  return DRONECU_OK;
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -133,11 +133,40 @@ struct PolicyArgs {
   float* last_obs;        // [n,15]
   StatSlot* stats;
   const float* norm;      // [31] float32 affine record (obs_norm.cuh): read only by the NORM instantiations
+  // read only by the TIMEOUT instantiations (DESIGN.md section 11): env i's j-th time-limit truncation of the launch goes to
+  // slot j * n + i; term_slots >= ceil(K / max_steps) (checked by the host) always suffices
+  float* term_obs;        // [T,n,16] raw pre-reset observation of the truncated step (info["terminal_observation"]), 16th = 1.0
+  int32_t* term_row;      // [T,n]    its rollout-buffer row k * n + i; -1 in every slot the launch did not fill
+  int32_t term_slots;     // T
 };
 
+// TIMEOUT: a step that ended by the time limit alone (timeout && !crashed: Gymnasium's truncated), recorded after step_env
+// and before reset_env -- the observation SB3 keeps as info["terminal_observation"].  j counts this env's truncations.
+__device__ __forceinline__ void record_truncation(const PolicyArgs& A, const EnvState& s, const int64_t i, const int k,
+                                                  int32_t& j, const bool writer) {
+  if (writer && j < A.term_slots) {
+    float x[kObs];
+    write_obs<kObs>(x, s);
+    const size_t slot = (size_t)j * (size_t)A.n + (size_t)i;
+    float4* d = reinterpret_cast<float4*>(A.term_obs + slot * 16);
+    st_quad(d, make_float4(x[0], x[1], x[2], x[3]));
+    st_quad(d + 1, make_float4(x[4], x[5], x[6], x[7]));
+    st_quad(d + 2, make_float4(x[8], x[9], x[10], x[11]));
+    st_quad(d + 3, make_float4(x[12], x[13], x[14], 1.0f));
+    A.term_row[slot] = (int32_t)((int64_t)k * A.n + i);
+  }
+  ++j;
+}
+
+// TIMEOUT: the slots env i did not fill read -1, so the side buffer is fully defined after every launch
+__device__ __forceinline__ void close_truncation_slots(const PolicyArgs& A, const int64_t i, int32_t j) {
+  for (; j < A.term_slots; ++j) A.term_row[(size_t)j * (size_t)A.n + (size_t)i] = -1;
+}
+
 // NORM: the towers see norm_obs_row(x) (obs_norm.cuh) -- the buffer still receives the raw row, obs_norm_pass_kernel
-// normalises it afterwards with the same function and the same record
-template <bool RANDOMIZED, bool NORM = false>
+// normalises it afterwards with the same function and the same record.  TIMEOUT: truncated steps are recorded
+// (record_truncation) for timeout_bootstrap_kernel (ppo_timeout.cuh); nothing else changes.
+template <bool RANDOMIZED, bool NORM = false, bool TIMEOUT = false>
 __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_constant__ PolicyArgs A) {
   extern __shared__ __align__(128) unsigned char smem_raw[];      // > 48 KB: dynamic shared memory
   MlpSmem& S = *reinterpret_cast<MlpSmem*>(smem_raw);
@@ -171,6 +200,7 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
 
   uint32_t n_done = 0, n_term = 0, len_sum = 0;
   float ret_sum = 0.f;
+  int32_t n_trunc = 0;
   float4* p_act = A.actions + i;
   float* p_logp = A.logp + i;
   float* p_val = A.value + i;
@@ -226,6 +256,7 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
         n_term += r.crashed ? 1 : 0;
         len_sum += (uint32_t)s.ep_len;
         ret_sum += s.ep_ret;
+        if constexpr (TIMEOUT) { if (!r.crashed) record_truncation(A, s, i, k, n_trunc, true); }
         reset_env<RANDOMIZED>(s, P, env_id);       // the PPO path always auto-resets (DummyVecEnv)
       }
     }
@@ -246,6 +277,7 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
                           emit_fast_ok<kObs>(A.last_obs, warp_base, n, valid));
   }
   if (active) store_state(A.state, i, s);
+  if constexpr (TIMEOUT) { if (active) close_truncation_slots(A, i, n_trunc); }
 
   if (__ballot_sync(0xffffffffu, n_done != 0)) {
     n_done = __reduce_add_sync(0xffffffffu, n_done);
@@ -321,7 +353,7 @@ __device__ __forceinline__ void tower_forward_warp(const MlpSmem& S, float* __re
   }
 }
 
-template <bool RANDOMIZED, bool NORM = false>
+template <bool RANDOMIZED, bool NORM = false, bool TIMEOUT = false>
 __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(const __grid_constant__ PolicyArgs A) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   MlpSmem& S = *reinterpret_cast<MlpSmem*>(smem_raw);
@@ -350,6 +382,7 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(c
   for (int o = 0; o < kAct; ++o) { std_[o] = expf(S.log_std[o]); logstd_sum += S.log_std[o]; }
   uint32_t n_done = 0, n_term = 0, len_sum = 0;
   float ret_sum = 0.f;
+  int32_t n_trunc = 0;
 
   for (int k = 0; k < A.K; ++k) {
     float x[kObs];
@@ -397,6 +430,7 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(c
       n_term += r.crashed ? 1 : 0;
       len_sum += (uint32_t)s.ep_len;
       ret_sum += s.ep_ret;
+      if constexpr (TIMEOUT) { if (!r.crashed) record_truncation(A, s, i, k, n_trunc, lane == 0); }
       reset_env<RANDOMIZED>(s, P, env_id);
     }
   }
@@ -422,6 +456,7 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(c
   }
   if (writer) {
     store_state(A.state, i, s);
+    if constexpr (TIMEOUT) close_truncation_slots(A, i, n_trunc);
     if (n_done != 0) {
       atomicAdd(&blk_stats[0], (unsigned long long)n_done);
       atomicAdd(&blk_stats[1], (unsigned long long)n_term);

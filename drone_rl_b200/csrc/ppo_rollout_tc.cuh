@@ -35,7 +35,7 @@ __global__ void __launch_bounds__(tc::kTile) policy_forward_tc_kernel(const floa
   tc::teardown(S);
 }
 
-template <bool RANDOMIZED, bool NORM = false>
+template <bool RANDOMIZED, bool NORM = false, bool TIMEOUT = false>
 __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __grid_constant__ PolicyArgs A) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   tc::Smem& S = tc_smem(smem_raw);
@@ -66,6 +66,7 @@ __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __gr
 
   uint32_t n_done = 0, n_term = 0, len_sum = 0, phase = 0;
   float ret_sum = 0.f;
+  int32_t n_trunc = 0;
   float4* p_act = A.actions + i;
   float* p_logp = A.logp + i;
   float* p_val = A.value + i;
@@ -117,6 +118,7 @@ __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __gr
         n_term += r.crashed ? 1 : 0;
         len_sum += (uint32_t)s.ep_len;
         ret_sum += s.ep_ret;
+        if constexpr (TIMEOUT) { if (!r.crashed) record_truncation(A, s, i, k, n_trunc, true); }
         reset_env<RANDOMIZED>(s, P, env_id);
       }
     }
@@ -136,6 +138,7 @@ __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __gr
                           emit_fast_ok<kObs>(A.last_obs, warp_base, n, valid));
   }
   if (active) store_state(A.state, i, s);
+  if constexpr (TIMEOUT) { if (active) close_truncation_slots(A, i, n_trunc); }
 
   if (__ballot_sync(0xffffffffu, n_done != 0)) {
     n_done = __reduce_add_sync(0xffffffffu, n_done);

@@ -72,11 +72,13 @@ class ObsNormalizer:
     # -- per rollout -----------------------------------------------------------------------------------
     def process_rollout(self, obs_store: torch.Tensor, reward: torch.Tensor, done: torch.Tensor, K: int,
                         allreduce: Optional[Callable[[torch.Tensor], None]] = None, side_env: int = -1,
-                        side_obs: Optional[torch.Tensor] = None) -> int:
+                        side_obs: Optional[torch.Tensor] = None, after_pass: Optional[Callable[[], None]] = None) -> int:
         """After the rollout launch: rewrite the buffer normalised (observations, rewards), then -- when training -- merge
         the rollout's moments into the statistics and derive the next affine record.  ``allreduce`` sums the moment record
-        over the ranks (data parallel).  ``side_obs`` [K,15] receives env ``side_env``'s raw rows.  Returns the number of
-        launches issued."""
+        over the ranks (data parallel).  ``side_obs`` [K,15] receives env ``side_env``'s raw rows.  ``after_pass`` is called
+        between the pass and the merge, while the affine record is still the one the rollout used (the time-limit
+        bootstrap: it adds to the normalised rewards and normalises its rows with that record).  Returns the number of
+        launches issued here."""
         a = _lib.NormPassArgs()
         if self.norm_obs:
             a.d_obs, a.obs_stride, a.d_affine = obs_store.data_ptr(), obs_store.shape[-1], self.affine.data_ptr()
@@ -92,6 +94,8 @@ class ObsNormalizer:
         a.d_partials = self.partials.data_ptr()
         st, dev = _stream_ptr(self.device), self.device.index
         _lib.check(self.lib.dronecu_norm_pass(dev, C.byref(a), st), "dronecu_norm_pass")
+        if after_pass is not None:
+            after_pass()
         if not self.training:
             return 1
         _lib.check(self.lib.dronecu_norm_reduce(dev, _ptr(self.partials), self.n_partials, _ptr(self.moments), st),

@@ -113,6 +113,12 @@ class PPO:
     SB3's does under VecNormalize; episode statistics stay in raw reward.  ``obs_rms`` / ``ret_rms`` / ``training`` /
     ``normalize_obs`` mirror the VecNormalize attributes, and ``predict`` normalises its input with the model's statistics
     (under SB3 the wrapped env does that).
+
+    ``handle_timeout_termination``: a step that ends by the time limit alone (Gymnasium ``truncated``, SB3's
+    ``TimeLimit.truncated``) gets ``reward += gamma * V(terminal observation)``, as SB3's ``collect_rollouts`` does for a
+    Gymnasium env; ``done`` stays set.  Off by default: the reference's legacy-gym env reports the limit as a plain done.
+    The rollout records the truncated steps' pre-reset observations in ``timeout_obs`` / ``timeout_row`` and one launch
+    adds the float32 values afterwards (DESIGN.md section 11).
     """
 
     tc_min_envs = 1024       # rollout_precision "tf32": tensor-core rollout kernel above this many envs per rank
@@ -123,7 +129,8 @@ class PPO:
                  seed: int = 0, device: int = 0, verbose: int = 0, policy_seed: Optional[int] = None,
                  rollout_precision: str = "fp32", update_precision: str = "fp32", cuda_graph: Optional[bool] = None,
                  dp_backend: str = "peer", padded_obs: Optional[bool] = None, norm_obs: bool = False,
-                 norm_reward: bool = False, clip_obs: float = 10.0, clip_reward: float = 10.0, norm_epsilon: float = 1e-8):
+                 norm_reward: bool = False, clip_obs: float = 10.0, clip_reward: float = 10.0, norm_epsilon: float = 1e-8,
+                 handle_timeout_termination: bool = False):
         self.lib = _lib.load()
         self.rank, self.world = 0, 1
         if torch.distributed.is_available() and torch.distributed.is_initialized():
@@ -173,6 +180,15 @@ class PPO:
             from .normalize import ObsNormalizer
             self.normalizer = ObsNormalizer(self.n_envs, self.device, norm_obs, norm_reward, clip_obs, clip_reward, norm_epsilon,
                                             gamma)
+        # time-limit bootstrap side buffers: env i's j-th truncation of a rollout goes to slot [j, i]; ceil(n_steps / max_steps)
+        # slots per env always suffice
+        self.handle_timeout_termination = bool(handle_timeout_termination)
+        self.timeout_obs = self.timeout_row = self._timeout_buf = None
+        if self.handle_timeout_termination:
+            T = -(-n_steps // self.batch.config.max_steps)
+            self.timeout_obs = torch.empty(T, self.n_envs, 16, dtype=torch.float32, device=self.device)
+            self.timeout_row = torch.empty(T, self.n_envs, dtype=torch.int32, device=self.device)
+            self._timeout_buf = _lib.TimeoutBuf(self.timeout_obs.data_ptr(), self.timeout_row.data_ptr(), T)
         self.side_env, self.side_obs = -1, None     # set_raw_obs_tap(): raw rows of one env per rollout
         self.num_timesteps, self.n_updates = 0, 0
         self._perm, self._epochs_done = None, 0
@@ -312,14 +328,26 @@ class PPO:
         # tensor cores pay from ~1k envs (a tile is 128 envs; below that the float32 warp-per-env kernel is both faster and exact)
         use_tc = self.rollout_precision == "tf32" and self.n_envs > self.tc_min_envs
         nz = self.normalizer
-        if nz is None:
+        if self.handle_timeout_termination:
+            _lib.check(self.lib.dronecu_rollout_policy_timeouts(self.batch._h, K, _ptr(self.params), int(deterministic), C.byref(out),
+                                                                None if nz is None else nz.affine_ptr(), int(use_tc),
+                                                                C.byref(self._timeout_buf), st), "dronecu_rollout_policy_timeouts")
+        elif nz is None:
             fn = self.lib.dronecu_rollout_policy_tc if use_tc else self.lib.dronecu_rollout_policy
             _lib.check(fn(self.batch._h, K, _ptr(self.params), int(deterministic), C.byref(out), st), "dronecu_rollout_policy")
         else:
             _lib.check(self.lib.dronecu_rollout_policy_norm(self.batch._h, K, _ptr(self.params), int(deterministic), C.byref(out),
                                                             nz.affine_ptr(), int(use_tc), st), "dronecu_rollout_policy_norm")
-            self.launches += nz.process_rollout(b.obs_store, b.reward, b.done, K, self._allreduce_f64 if self.world > 1 else None,
-                                                self.side_env, self.side_obs)
+        # the bootstrap adds to the reward the buffer finally holds (SB3: to the VecNormalize reward), with the observation
+        # record the rollout used: after the normalisation pass, before the merge replaces the record
+        bootstrap = self._bootstrap_timeouts if self.handle_timeout_termination else None
+        if nz is not None:
+            # not `self.launches += ...`: the bootstrap inside the call counts its own launch
+            issued = nz.process_rollout(b.obs_store, b.reward, b.done, K, self._allreduce_f64 if self.world > 1 else None,
+                                        self.side_env, self.side_obs, after_pass=bootstrap)
+            self.launches += issued
+        elif bootstrap is not None:
+            bootstrap()
         if nz is None and self.side_obs is not None:
             self.side_obs.copy_(b.obs[:, self.side_env])
         _lib.check(self.lib.dronecu_gae(self.device.index, K, n, _ptr(b.reward), _ptr(b.value), _ptr(b.done),
@@ -327,6 +355,14 @@ class PPO:
                    "dronecu_gae")
         self.launches += 2
         self.num_timesteps += K * n * self.world
+
+    def _bootstrap_timeouts(self):
+        """reward += f32(gamma * V(terminal row)) on every truncated step recorded by the rollout (one launch)."""
+        nz = self.normalizer
+        _lib.check(self.lib.dronecu_bootstrap_timeouts(self.device.index, _ptr(self.params), C.byref(self._timeout_buf), self.n_envs,
+                                                       None if nz is None else nz.affine_ptr(), self.gamma, _ptr(self.buf.reward),
+                                                       _stream_ptr(self.device)), "dronecu_bootstrap_timeouts")
+        self.launches += 1
 
     # -- update -------------------------------------------------------------------------------------
     def _minibatch(self, index: Optional[torch.Tensor], first: int, m: int, stats: Optional[torch.Tensor] = None):
@@ -543,6 +579,7 @@ class PPO:
                 "num_timesteps": self.num_timesteps, "n_updates": self.n_updates, "epochs_done": self._epochs_done,
                 "env_state": self.batch.get_state(), "env_global_step": self.batch.global_step,
                 "env_offset": int(self.batch.env_offset), "world": self.world,
+                "handle_timeout_termination": self.handle_timeout_termination,
                 "sb3_policy": {SB3_NAMES[k]: v.clone() for k, v in unpack_params(self.params.cpu()).items()},
                 **({} if self.normalizer is None else {"normalizer": self.normalizer.state_dict(),
                                                        "norm_returns": self.normalizer.returns.cpu().clone()})}
@@ -587,7 +624,8 @@ class PPO:
                  "gae_lambda": self.gae_lambda, "learning_rate": float(self.cfg.learning_rate),
                  "clip_range": float(self.cfg.clip_range), "ent_coef": float(self.cfg.ent_coef),
                  "vf_coef": float(self.cfg.vf_coef), "max_grad_norm": float(self.cfg.max_grad_norm),
-                 "n_envs": self.n_envs, "num_timesteps": self.num_timesteps, "_n_updates": self.n_updates, "seed": self.seed}
+                 "n_envs": self.n_envs, "num_timesteps": self.num_timesteps, "_n_updates": self.n_updates, "seed": self.seed,
+                 "handle_timeout_termination": self.handle_timeout_termination}
         extra = {k: sd[k] for k in ("num_timesteps", "n_updates", "epochs_done", "env_state", "env_global_step", "env_offset", "world",
                                     "normalizer", "norm_returns") if k in sd}
         sb3_zip.export_zip(path if path.endswith(".zip") else path + ".zip", sd["params"], sd["adam"], sd["adam_step"],
@@ -609,13 +647,15 @@ class PPO:
             path = path + ".zip"
         if path.endswith(".pt"):
             sd = torch.load(path, weights_only=False)
+            if "handle_timeout_termination" in sd:
+                kw = {"handle_timeout_termination": bool(sd["handle_timeout_termination"]), **kw}
             model = cls(env, **cls._norm_settings(sd, kw))
             model.load_state_dict(sd)
             return model
         from . import sb3_zip
         z = sb3_zip.import_zip(path)
         for k in ("n_steps", "batch_size", "n_epochs", "gamma", "gae_lambda", "learning_rate", "clip_range", "ent_coef",
-                  "vf_coef", "max_grad_norm"):
+                  "vf_coef", "max_grad_norm", "handle_timeout_termination"):
             if k in z["hyper"] and k not in kw and isinstance(z["hyper"][k], (int, float)):
                 kw[k] = z["hyper"][k]
         model = cls(env, **cls._norm_settings(z["extra"] or {}, kw))

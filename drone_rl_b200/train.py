@@ -166,6 +166,8 @@ def main(argv=None):
     ap.add_argument("--norm-obs", action="store_true", help="normalise observations (SB3 VecNormalize norm_obs) in the rollout")
     ap.add_argument("--norm-reward", action="store_true", help="normalise rewards by the running std of the discounted return")
     ap.add_argument("--clip-obs", type=float, default=10.0, help="clip of the normalised observations")
+    ap.add_argument("--handle-timeout-termination", action="store_true",
+                    help="bootstrap time-limit ends with gamma * V(terminal observation), as SB3 does for Gymnasium time limits")
     ap.add_argument("--eval-freq", type=int, default=0,
                     help="evaluate the policy every this many vec-env steps (SB3 EvalCallback; 0 = no evaluation)")
     ap.add_argument("--n-eval-episodes", type=int, default=5)
@@ -194,6 +196,8 @@ def main(argv=None):
               update_precision=args.update_precision or ("bf16" if args.precision == "tf32" else "fp32"))
     if args.norm_obs or args.norm_reward:       # else: PPO.load takes the archive's own settings
         kw.update(norm_obs=args.norm_obs, norm_reward=args.norm_reward, clip_obs=args.clip_obs)
+    if args.handle_timeout_termination:        # else: PPO.load takes the archive's own setting
+        kw.update(handle_timeout_termination=True)
     if os.path.exists(args.resume):
         model = PPO.load(args.resume, env, **kw)
         if rank == 0:

@@ -265,6 +265,36 @@ int dronecu_gae(int device, int K, int64_t n, const float* d_reward, const float
 int dronecu_rollout_policy_norm(dronecu_env* env, int K, const float* d_params, int deterministic,
                                 const dronecu_policy_out* out, const float* d_norm_affine, int tensor_cores, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Time-limit bootstrap (SB3 handle_timeout_termination: Gymnasium `truncated` / info["TimeLimit.truncated"]; csrc/ppo_timeout.cuh,
+ * DESIGN.md section 11).  A step that ends by the time limit alone (timeout && !crashed) gets
+ *   reward += f32(f32(gamma) * V(terminal observation))
+ * while done stays set (GAE starts a new episode there).  Per rollout, on one stream:
+ *   dronecu_rollout_policy_timeouts   the rollout of dronecu_rollout_policy_norm that also records each truncated step's raw
+ *                                     pre-reset observation and buffer row in a dronecu_timeout_buf
+ *   [dronecu_norm_pass]               rewards normalised first (SB3 adds gamma * V to the VecNormalize reward)
+ *   dronecu_bootstrap_timeouts        the float32 value tower on each recorded row (normalised with the rollout's affine
+ *                                     record), added to its reward in place
+ *   [dronecu_norm_reduce / _combine]  afterwards: the combine overwrites the affine record
+ * ---------------------------------------------------------------------------------------------- */
+typedef struct dronecu_timeout_buf {
+  float* d_obs;          /* [T,n,16] 16-byte aligned: the raw pre-reset observation (info["terminal_observation"]), 16th = 1.0 */
+  int32_t* d_row;        /* [T,n]    its rollout-buffer row k * n + i, -1 in an unused slot; env i's j-th truncation of the
+                            launch goes to slot j * n + i                                                                    */
+  int32_t slots_per_env; /* T >= ceil(K / max_steps): an env truncates at most that often in K steps                        */
+} dronecu_timeout_buf;
+
+/* dronecu_rollout_policy_norm (same kernels' choice and results) that also fills *timeouts; every slot is written (row or -1).
+ * DRONECU_ERR_INVALID when slots_per_env < ceil(K / max_steps), K * n or slots_per_env * n exceed INT32_MAX, a pointer is
+ * NULL or d_obs is misaligned. */
+int dronecu_rollout_policy_timeouts(dronecu_env* env, int K, const float* d_params, int deterministic,
+                                    const dronecu_policy_out* out, const float* d_norm_affine, int tensor_cores,
+                                    const dronecu_timeout_buf* timeouts, void* stream);
+/* d_reward[row] = d_reward[row] + f32(gamma * V(norm(d_obs[slot]))) for every slot with row >= 0 of the n envs, V the float32
+ * value tower of dronecu_policy_forward (bit-identical to it on the same row); d_norm_affine NULL: rows used raw. */
+int dronecu_bootstrap_timeouts(int device, const float* d_params, const dronecu_timeout_buf* timeouts, int64_t n,
+                               const float* d_norm_affine, float gamma, float* d_reward, void* stream);
+
 /* One thread per env walks its K steps of the step-major buffers [K,n,...]. */
 typedef struct dronecu_norm_pass_args {
   float* d_obs;             /* [K,n,obs_stride] raw rows, rewritten normalised; NULL: observations untouched, no obs moments */
