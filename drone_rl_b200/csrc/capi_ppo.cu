@@ -40,6 +40,7 @@ struct dronecu_ppo {
   // data-parallel exchange over peer memory (ppo_dp.cuh)
   DpArgs dp;         // dp.world == 0: not set up
   float* dp_mail;    // this rank's mailbox (cudaMalloc: exportable with cudaIpcGetMemHandle)
+  int dp_alloc_world;  // the world dp_mail was sized for: dronecu_ppo_dp_connect accepts only this one
   bool dp_opened[kDpMaxWorld];   // mail[r] was mapped with cudaIpcOpenMemHandle (to be closed)
 };
 
@@ -616,6 +617,7 @@ extern "C" int dronecu_ppo_dp_alloc(dronecu_ppo* p, int rank, int world, void* i
   CUDA_TRY(cudaMemset(p->dp.status, 0, sizeof(int)));
   CUDA_TRY(cudaDeviceSynchronize());
   p->dp.rank = rank; p->dp.world = 0;          // world is set by dronecu_ppo_dp_connect
+  p->dp_alloc_world = world;
   p->dp.timeout_ns = 30ull * 1000000000ull;
   if (ipc_handle_out) {
     cudaIpcMemHandle_t h;
@@ -624,13 +626,16 @@ extern "C" int dronecu_ppo_dp_alloc(dronecu_ppo* p, int rank, int world, void* i
   }
   if (d_mailbox_out) *d_mailbox_out = p->dp_mail;
   p->dp.mail[rank] = p->dp_mail;
-  (void)world;
   return DRONECU_OK;
 }
 
 extern "C" int dronecu_ppo_dp_connect(dronecu_ppo* p, int world, const void* ipc_handles, void* const* d_mailboxes) {
   if (!p || !p->dp_mail) return fail(DRONECU_ERR_INVALID, "dronecu_ppo_dp_connect: call dronecu_ppo_dp_alloc first");
   if (world < 1 || world > kDpMaxWorld || p->dp.rank >= world) return fail(DRONECU_ERR_INVALID, "dronecu_ppo_dp_connect: bad world");
+  // the slots and flags are indexed with the connected world: a larger one would write past the end of every mailbox
+  if (world != p->dp_alloc_world)
+    return fail(DRONECU_ERR_INVALID, "dronecu_ppo_dp_connect: world differs from the one dronecu_ppo_dp_alloc sized the mailbox for");
+  if (p->dp.world > 0) return fail(DRONECU_ERR_INVALID, "dronecu_ppo_dp_connect: already connected");
   if (!ipc_handles && !d_mailboxes && world > 1) return fail(DRONECU_ERR_INVALID, "dronecu_ppo_dp_connect: no peers given");
   DeviceGuard guard(p->device);
   for (int r = 0; r < world; ++r) {

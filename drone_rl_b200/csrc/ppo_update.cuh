@@ -545,7 +545,11 @@ __device__ __forceinline__ void clip_adam_apply(const AdamArgs& A, const float (
   __syncthreads();
   const float norm = scal[0];
   apply_publish_info(A, stats, scale, norm);
-  const float coef = fminf(A.max_norm / (norm + 1e-6f), 1.0f) * scale;
+  // torch.clamp(clip_coef, max=1.0): a non-finite gradient gives a NaN norm and a NaN coefficient that poisons every
+  // parameter, as in torch (min.NaN; fminf would return 1 and update every finite entry as if nothing happened)
+  float coef = A.max_norm / (norm + 1e-6f);
+  asm("min.NaN.f32 %0, %0, %1;" : "+f"(coef) : "f"(1.0f));
+  coef *= scale;
   const float lr_over_bc1 = scal[1], inv_sqrt_bc2 = scal[2];
   float th[kApplyPer];
 #pragma unroll

@@ -470,7 +470,8 @@ int dronecu_ppo_set_state(dronecu_ppo* ppo, const float* d_moments, int64_t step
 int dronecu_ppo_dp_alloc(dronecu_ppo* ppo, int rank, int world, void* ipc_handle_out /* [64], nullable */,
                          void** d_mailbox_out /* nullable */);
 /* ipc_handles: [world][64] bytes (entry `rank` ignored), or NULL with d_mailboxes[world] = raw device pointers of
- * mailboxes allocated in THIS process (peer access is enabled as needed). */
+ * mailboxes allocated in THIS process (peer access is enabled as needed).  `world` must equal the world passed to
+ * dronecu_ppo_dp_alloc (the mailbox is sized for it), and a handle connects once: DRONECU_ERR_INVALID otherwise. */
 int dronecu_ppo_dp_connect(dronecu_ppo* ppo, int world, const void* ipc_handles, void* const* d_mailboxes);
 /* A rank that waits longer than this for its peers (default 30 s) raises the status flag instead of hanging the GPU. */
 int dronecu_ppo_dp_set_timeout(dronecu_ppo* ppo, double seconds);

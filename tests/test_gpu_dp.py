@@ -1,8 +1,8 @@
 """GPU tests of the data-parallel PPO update over peer memory (csrc/ppo_dp.cuh; north_star configs[4]).
 
-* one GPU: two optimiser handles play two ranks (mailboxes wired with raw pointers, two streams) -- exercises the
-  push / flag / wait / fixed-order sum / clip + Adam kernel, the float64 all-reduce kernel and the time-out path through
-  the C ABI without needing a second device;
+* one GPU: the time-out path and the rejected arguments of the C ABI; ``_handles`` wires optimiser handles of one process
+  as ranks (mailboxes joined with raw pointers).  The exchange kernels at every world size, inside CUDA graphs and under
+  PPO.train() are pinned against float64 in tests/test_gpu_dp_parity.py;
 * two GPUs (skipped on a one-GPU box; run with ``gpurun --gpus 2``): two processes under NCCL-initialised
   torch.distributed run ``PPO.collect_rollouts`` + ``PPO.train`` on their shards.  Asserted: parameters bit-identical
   across the ranks, equal to the "nccl" backend to float rounding, and equal (<= 1e-6) to ONE rank training on the union
@@ -43,64 +43,6 @@ def _handles(lib, n, device=0, timeout=5.0):
         _lib.check(lib.dronecu_ppo_dp_connect(h, n, None, arr))
         _lib.check(lib.dronecu_ppo_dp_set_timeout(h, timeout))
     return hs
-
-
-@pytest.mark.parametrize("world", [2, 3])
-def test_peer_exchange_apply_equals_single_apply_of_the_sum(drl, world):
-    from drone_rl_b200 import _lib
-    from drone_rl_b200.core import _ptr
-    lib, dev = _lib.load(), torch.device("cuda", 0)
-    hs = _handles(lib, world)
-    cfg = _lib.PPOConfig()
-    lib.dronecu_ppo_config_default(C.byref(cfg))
-    href = C.c_void_p()
-    _lib.check(lib.dronecu_ppo_create(C.byref(cfg), 0, C.byref(href)))
-    g = torch.Generator().manual_seed(0)
-    theta0 = (0.1 * torch.randn(_lib.POLICY_PARAMS, generator=g)).to(dev)
-    params = [theta0.clone() for _ in range(world)]
-    pref = theta0.clone()
-    info = [torch.zeros(9, device=dev) for _ in range(world)]
-    iref = torch.zeros(9, device=dev)
-    streams = [torch.cuda.Stream() for _ in range(world)]
-    for step in range(6):
-        scale = 10.0 ** (step % 3 - 1)                  # both sides of the clip threshold
-        grads = []
-        for r in range(world):
-            gr = torch.randn(_lib.GRAD_LEN, generator=g) * scale
-            gr[_lib.POLICY_PARAMS + 4] = 64.0 * (r + 1)  # sample counts differ per rank (power-of-two total below)
-            grads.append(gr.to(dev))
-        if world == 3:
-            grads[2][_lib.POLICY_PARAMS + 4] = 64.0      # 64 + 128 + 64 = 256
-        total = grads[0].clone()
-        for r in range(1, world):
-            total += grads[r]                            # fixed rank order, float32: what the kernel does
-        torch.cuda.synchronize()
-        for r in range(world):
-            with torch.cuda.stream(streams[r]):
-                _lib.check(lib.dronecu_ppo_apply_dp(hs[r], _ptr(params[r]), _ptr(grads[r]), _ptr(info[r]),
-                                                    C.c_void_p(streams[r].cuda_stream)))
-        count = float(total[_lib.POLICY_PARAMS + 4])
-        _lib.check(lib.dronecu_ppo_apply(href, _ptr(pref), _ptr(total), 1.0 / count, _ptr(iref), None))
-        torch.cuda.synchronize()
-        for r in range(world):
-            assert torch.equal(grads[r], total), f"step {step}: rank {r} did not receive the fixed-order sum"
-            assert torch.equal(params[r], pref), f"step {step}: rank {r} parameters differ from apply(sum)"
-            assert torch.equal(info[r], iref)
-    for r, h in enumerate(hs):
-        st, n = C.c_int(), C.c_int64()
-        _lib.check(lib.dronecu_ppo_dp_status(h, C.byref(st), C.byref(n)))
-        assert st.value == 0 and n.value == 6
-    # float64 all-reduce through the same mailboxes (advantage / episode statistics)
-    bufs = [torch.arange(37, dtype=torch.float64, device=dev) * (r + 1) + 0.125 * r for r in range(world)]
-    want = sum(b.clone() for b in bufs)
-    for r in range(world):
-        with torch.cuda.stream(streams[r]):
-            _lib.check(lib.dronecu_ppo_dp_allreduce_f64(hs[r], _ptr(bufs[r]), 37, C.c_void_p(streams[r].cuda_stream)))
-    torch.cuda.synchronize()
-    for r in range(world):
-        assert torch.equal(bufs[r], want)
-    for h in hs + [href]:
-        lib.dronecu_ppo_destroy(h)
 
 
 def test_peer_exchange_times_out_instead_of_hanging(drl):

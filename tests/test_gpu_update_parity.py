@@ -445,10 +445,18 @@ def _adam_state(model):
     return mom, step.value
 
 
-def _spy_train(model, n_train, forced):
+def _spy_train(model, n_train, forced, own_grad=False):
     """Run train() n_train times with cuda_graph=False, recording at every optimiser step the index slice and the statistics
-    row used, and at the steps k with forced(k) the parameters, moments and Adam step before and after and model._grad."""
-    records, orig = [], model._minibatch
+    row used, and at the steps k with forced(k) the parameters, moments and Adam step before and after and model._grad.
+    ``own_grad``: also record model._grad right after the gradient launch, before a data-parallel exchange replaces it by
+    the sum over the ranks.  Every read is ordered on the current stream, so each rank of a one-GPU data-parallel run can
+    call this from its own thread; it ends with a synchronisation of that stream only."""
+    records, orig, orig_grad = [], model._minibatch, model.launch_grad
+    pending = {}
+
+    def spy_grad(index, first, m, stats_ptr, grad, precision=None):
+        orig_grad(index, first, m, stats_ptr, grad, precision)
+        pending["own_grad"] = grad.clone()
 
     def spy(index, first, m, stats=None):
         k = len(records)
@@ -457,6 +465,8 @@ def _spy_train(model, n_train, forced):
             r["theta"] = model.params.clone()
             r["mom"], r["t"] = _adam_state(model)
         orig(index, first, m, stats)
+        r.update(pending)
+        pending.clear()
         if model.normalize_advantage:
             r["stats"] = (model._adv_stats if stats is None else stats).clone()
         else:
@@ -468,12 +478,16 @@ def _spy_train(model, n_train, forced):
             r["mom_after"], r["t_after"] = _adam_state(model)
         records.append(r)
     model._minibatch = spy
+    if own_grad:
+        model.launch_grad = spy_grad
     try:
         for _ in range(n_train):
             model.train()
     finally:
         del model._minibatch
-    torch.cuda.synchronize()
+        if own_grad:
+            del model.launch_grad
+    torch.cuda.current_stream(model.device).synchronize()
     return records
 
 
