@@ -6,6 +6,7 @@
 #include <cstring>
 #include <new>
 #include <string>
+#include <type_traits>
 
 #include "../../include/dronecu.h"
 #include "capi_common.h"
@@ -57,6 +58,20 @@ extern "C" int dronecu_set_rollout_kernel(int mode) {
 
 enum RolloutKernel { kThreadPerEnv, kWarpPerEnv, kTensorCores };
 
+// the kernel flavour of a rollout or an evaluation of env e: tensor cores when asked, else the float32 kernel of
+// dronecu_set_rollout_kernel (small batches: one warp per env, ppo_rollout.cuh)
+static RolloutKernel choose_kernel(const dronecu_env* e, bool tensor_cores) {
+  if (tensor_cores) return kTensorCores;
+  return (g_rollout_kernel_mode == 2 || (g_rollout_kernel_mode == 0 && e->n <= kWarpRolloutMaxEnvs)) ? kWarpPerEnv : kThreadPerEnv;
+}
+
+// f(std::bool_constant<randomized>, std::bool_constant<norm>): the kernels' RANDOMIZED and NORM template flags
+template <class F>
+static int with_flags(bool randomized, bool norm, F&& f) {
+  if (randomized) return norm ? f(std::true_type{}, std::true_type{}) : f(std::true_type{}, std::false_type{});
+  return norm ? f(std::false_type{}, std::true_type{}) : f(std::false_type{}, std::false_type{});
+}
+
 template <bool RANDOMIZED, bool NORM, bool TIMEOUT>
 static int launch_policy_rollout(RolloutKernel which, int64_t n, const PolicyArgs& a, cudaStream_t st) {
   if (which == kTensorCores) {
@@ -71,12 +86,6 @@ static int launch_policy_rollout(RolloutKernel which, int64_t n, const PolicyArg
     policy_rollout_kernel<RANDOMIZED, NORM, TIMEOUT><<<(unsigned)((n + kPolBlock - 1) / kPolBlock), kPolBlock, kPolicySmem, st>>>(a);
   }
   return DRONECU_OK;
-}
-
-template <bool TIMEOUT>
-static int launch_policy_rollout(RolloutKernel which, bool randomized, bool norm, int64_t n, const PolicyArgs& a, cudaStream_t st) {
-  if (norm) return randomized ? launch_policy_rollout<true, true, TIMEOUT>(which, n, a, st) : launch_policy_rollout<false, true, TIMEOUT>(which, n, a, st);
-  return randomized ? launch_policy_rollout<true, false, TIMEOUT>(which, n, a, st) : launch_policy_rollout<false, false, TIMEOUT>(which, n, a, st);
 }
 
 // the side buffer of the time-limit bootstrap: slots_per_env slots per env, 16-byte aligned 64-byte rows
@@ -118,13 +127,11 @@ static int rollout_policy_impl(dronecu_env* e, int K, const float* d_params, int
     a.last_obs = out->d_last_obs;
   }
   if (tb) { a.term_obs = tb->d_obs; a.term_row = tb->d_row; a.term_slots = tb->slots_per_env; }
-  // small batches: one warp per env (ppo_rollout.cuh)
-  const RolloutKernel which = tensor_cores ? kTensorCores
-      : (g_rollout_kernel_mode == 2 || (g_rollout_kernel_mode == 0 && e->n <= kWarpRolloutMaxEnvs)) ? kWarpPerEnv : kThreadPerEnv;
+  const RolloutKernel which = choose_kernel(e, tensor_cores);
   cudaStream_t st = (cudaStream_t)stream;
-  const bool randomized = (e->cfg.flags & DRONECU_RANDOMIZED) != 0;
-  const int rc = tb ? launch_policy_rollout<true>(which, randomized, d_norm_affine != nullptr, e->n, a, st)
-                    : launch_policy_rollout<false>(which, randomized, d_norm_affine != nullptr, e->n, a, st);
+  const int rc = with_flags((e->cfg.flags & DRONECU_RANDOMIZED) != 0, d_norm_affine != nullptr, [&](auto R, auto N) {
+    return tb ? launch_policy_rollout<R, N, true>(which, e->n, a, st) : launch_policy_rollout<R, N, false>(which, e->n, a, st);
+  });
   if (rc != DRONECU_OK) return rc;
   e->launches += 1;
   CUDA_TRY(cudaGetLastError());
@@ -216,14 +223,10 @@ extern "C" int dronecu_evaluate_policy(dronecu_env* e, const float* d_params, co
   a.deterministic = p->deterministic; a.max_eps = p->max_eps; a.env_index0 = p->env_index0; a.n_global = p->n_global;
   a.n_eval_episodes = p->n_eval_episodes; a.theta = d_params; a.norm = d_norm_affine;
   a.steps = p->d_steps; a.count = p->d_count; a.ep_return = p->d_ep_return; a.ep_length = p->d_ep_length; a.pending = p->d_pending;
-  // the kernel choice of rollout_policy_impl
-  const RolloutKernel which = tensor_cores ? kTensorCores
-      : (g_rollout_kernel_mode == 2 || (g_rollout_kernel_mode == 0 && e->n <= kWarpRolloutMaxEnvs)) ? kWarpPerEnv : kThreadPerEnv;
+  const RolloutKernel which = choose_kernel(e, tensor_cores != 0);
   cudaStream_t st = (cudaStream_t)stream;
-  const bool randomized = (e->cfg.flags & DRONECU_RANDOMIZED) != 0;
-  int rc;
-  if (d_norm_affine) rc = randomized ? launch_policy_eval<true, true>(which, e->n, a, st) : launch_policy_eval<false, true>(which, e->n, a, st);
-  else rc = randomized ? launch_policy_eval<true, false>(which, e->n, a, st) : launch_policy_eval<false, false>(which, e->n, a, st);
+  const int rc = with_flags((e->cfg.flags & DRONECU_RANDOMIZED) != 0, d_norm_affine != nullptr,
+                            [&](auto R, auto N) { return launch_policy_eval<R, N>(which, e->n, a, st); });
   if (rc != DRONECU_OK) return rc;
   e->launches += 1;
   CUDA_TRY(cudaGetLastError());

@@ -45,6 +45,13 @@ __device__ __forceinline__ void norm_obs_row(float (&x)[kObs], const volatile fl
   for (int i = 0; i < kObs; ++i) x[i] = norm_obs1(x[i], s[i], s[kObs + i], clip);
 }
 
+// the policy kernels' staging of the record: s = the CTA's __shared__ float[NORM ? kNormAffine : 1]; ordered by the
+// kernel's next CTA barrier
+template <bool NORM>
+__device__ __forceinline__ void load_norm(float* s, const float* affine) {
+  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s[threadIdx.x] = affine[threadIdx.x]; }
+}
+
 struct NormPassArgs {
   float* obs;              // [K,n,stride], rewritten in place (nullptr: observations untouched, no obs moments)
   int32_t stride;          // 15 or 16 (16th value of padded rows left as it is: 1.0)

@@ -9,8 +9,9 @@
 //   probe     each env steps from steps[i] until it reached its target or step `limit`; the envs still below target are
 //             counted into *pending
 //   catch-up  (T known) each env steps from steps[i] to T, recording nothing new
-// Same arithmetic as the rollout kernels on the same operands (tower_forward / tower_forward_warp / tc::tower, step_env,
-// reset_env, norm_obs_row, noise_normals): each evaluation kernel reproduces its rollout counterpart bit for bit.
+// Same functions as the rollout kernels on the same operands (tower_forward / tower_forward_warp / tc::tower, policy_std,
+// policy_action, env_action, step_env, reset_env, norm_obs_row): each evaluation kernel reproduces its rollout counterpart
+// bit for bit.
 #pragma once
 #include "ppo_rollout_tc.cuh"
 
@@ -52,17 +53,9 @@ __device__ __forceinline__ void eval_step(const EvalArgs& A, EnvState& s, const 
                                           uint64_t env_id, int64_t i, int32_t& c, int32_t& count, int32_t target,
                                           bool writer = true) {
   const EnvParams& P = A.P;
-  float4 a;
-  if (A.deterministic) {
-    a = make_float4(mean[0], mean[1], mean[2], mean[3]);
-  } else {
-    const float4 z = noise_normals(P.keys, env_id, A.t0 + (uint64_t)c);
-    a = make_float4(fmaf(std_[0], z.x, mean[0]), fmaf(std_[1], z.y, mean[1]),
-                    fmaf(std_[2], z.z, mean[2]), fmaf(std_[3], z.w, mean[3]));
-  }
-  const float4 f = make_float4(fminf(fmaxf(a.x, 0.f), P.motor_max), fminf(fmaxf(a.y, 0.f), P.motor_max),
-                               fminf(fmaxf(a.z, 0.f), P.motor_max), fminf(fmaxf(a.w, 0.f), P.motor_max));
-  const StepResult r = step_env(s, P, f);
+  float logp;                             // unused: the compiler drops it
+  const float4 a = policy_action(mean, std_, 0.f, P.keys, env_id, A.t0 + (uint64_t)c, A.deterministic, logp);
+  const StepResult r = step_env(s, P, env_action(a, P.motor_max));
   if (r.crashed || r.timeout) {
     if (count < target) {                 // VecMonitor's info["episode"]: float32 return, int length
       if (writer) {
@@ -77,11 +70,6 @@ __device__ __forceinline__ void eval_step(const EvalArgs& A, EnvState& s, const 
   c += 1;
 }
 
-__device__ __forceinline__ void eval_std(const float* log_std, float (&std_)[kAct]) {
-#pragma unroll
-  for (int o = 0; o < kAct; ++o) std_[o] = expf(log_std[o]);
-}
-
 // one env per thread; lanes stop independently (the tower reads shared memory only)
 template <bool RANDOMIZED, bool NORM>
 __global__ void __launch_bounds__(kPolBlock) policy_eval_kernel(const __grid_constant__ EvalArgs A) {
@@ -89,7 +77,7 @@ __global__ void __launch_bounds__(kPolBlock) policy_eval_kernel(const __grid_con
   MlpSmem& S = *reinterpret_cast<MlpSmem*>(smem_raw);
   __shared__ float s_norm[NORM ? kNormAffine : 1];
   load_mlp_smem(S, A.theta);
-  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s_norm[threadIdx.x] = A.norm[threadIdx.x]; }
+  load_norm<NORM>(s_norm, A.norm);
   __syncthreads();
 
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -99,7 +87,7 @@ __global__ void __launch_bounds__(kPolBlock) policy_eval_kernel(const __grid_con
   if (active) {
     EnvState s = load_state(A.state, i);
     float std_[kAct];
-    eval_std(S.log_std, std_);
+    policy_std(S.log_std, std_);
     int32_t c = A.steps[i], count = A.count[i];
     const int32_t target = eval_target(A, i);
     while (eval_live(A, c, count, target)) {
@@ -125,7 +113,7 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_eval_warp_kernel(cons
   MlpSmem& S = *reinterpret_cast<MlpSmem*>(smem_raw);
   __shared__ float s_norm[NORM ? kNormAffine : 1];
   load_mlp_smem(S, A.theta);
-  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s_norm[threadIdx.x] = A.norm[threadIdx.x]; }
+  load_norm<NORM>(s_norm, A.norm);
   __syncthreads();
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -135,7 +123,7 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_eval_warp_kernel(cons
   const uint64_t env_id = A.P.env_offset + (uint64_t)i;
   EnvState s = load_state(A.state, i);
   float std_[kAct];
-  eval_std(S.log_std, std_);
+  policy_std(S.log_std, std_);
   int32_t c = A.steps[i], count = A.count[i];
   const int32_t target = eval_target(A, i);
   while (eval_live(A, c, count, target)) {
@@ -160,7 +148,7 @@ __global__ void __launch_bounds__(tc::kTile) policy_eval_tc_kernel(const __grid_
   extern __shared__ __align__(128) unsigned char smem_raw[];
   tc::Smem& S = tc_smem(smem_raw);
   __shared__ float s_norm[NORM ? kNormAffine : 1];
-  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s_norm[threadIdx.x] = A.norm[threadIdx.x]; }
+  load_norm<NORM>(s_norm, A.norm);
   tc::setup(S, A.theta);
 
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -175,7 +163,7 @@ __global__ void __launch_bounds__(tc::kTile) policy_eval_tc_kernel(const __grid_
     target = eval_target(A, i);
   }
   float std_[kAct];
-  eval_std(S.log_std, std_);
+  policy_std(S.log_std, std_);
   uint32_t phase = 0;
   bool live = active && eval_live(A, c, count, target);
   while (__syncthreads_or(live)) {

@@ -140,6 +140,113 @@ struct PolicyArgs {
   int32_t term_slots;     // T
 };
 
+// ---------------------------------------------------------------------------------------------
+// The policy step, stated once for the three rollout kernels and the three evaluation kernels (ppo_eval.cuh): every kernel
+// computes the std, the action and its log-prob, the env's clipped action and the episode statistics with these functions,
+// so each reproduces the others bit for bit on the same operands.
+// ---------------------------------------------------------------------------------------------
+
+// std = exp(log_std) of SB3's state-independent Gaussian; returns sum(log_std), the log-prob's normaliser
+__device__ __forceinline__ float policy_std(const float* log_std, float (&std_)[kAct]) {
+  float logstd_sum = 0.f;
+#pragma unroll
+  for (int o = 0; o < kAct; ++o) { std_[o] = expf(log_std[o]); logstd_sum += log_std[o]; }
+  return logstd_sum;
+}
+
+// the action of env env_id at step t (Philox noise index) and its log-prob: mean (SB3 deterministic) or mean + std * z,
+// NOT clipped (what SB3 stores in the buffer)
+__device__ __forceinline__ float4 policy_action(const float (&mean)[kAct], const float (&std_)[kAct], float logstd_sum,
+                                                const PhiloxKeys& keys, uint64_t env_id, uint64_t t, bool deterministic,
+                                                float& logp) {
+  float4 a;
+  if (deterministic) {
+    a = make_float4(mean[0], mean[1], mean[2], mean[3]);
+    logp = -logstd_sum - kAct * kHalfLog2Pi;
+  } else {
+    const float4 z = noise_normals(keys, env_id, t);
+    a = make_float4(fmaf(std_[0], z.x, mean[0]), fmaf(std_[1], z.y, mean[1]),
+                    fmaf(std_[2], z.z, mean[2]), fmaf(std_[3], z.w, mean[3]));
+    // Normal(mean, std).log_prob(a) summed over the 4 dims; (a - mean) / std == z up to rounding
+    logp = -0.5f * (z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w) - logstd_sum - kAct * kHalfLog2Pi;
+  }
+  return a;
+}
+
+// np.clip(a, low, high) for the env only (SB3 collect_rollouts); the buffer keeps `a`
+__device__ __forceinline__ float4 env_action(const float4 a, float motor_max) {
+  return make_float4(fminf(fmaxf(a.x, 0.f), motor_max), fminf(fmaxf(a.y, 0.f), motor_max),
+                     fminf(fmaxf(a.z, 0.f), motor_max), fminf(fmaxf(a.w, 0.f), motor_max));
+}
+
+// a 64-byte observation row, the 16th value 1.0 (the bias column of the update kernels' X tile): four 128-bit stores
+// straight from the registers
+__device__ __forceinline__ void store_row16(float* row, const float (&x)[kObs]) {
+  float4* d = reinterpret_cast<float4*>(row);
+  st_quad(d, make_float4(x[0], x[1], x[2], x[3]));
+  st_quad(d + 1, make_float4(x[4], x[5], x[6], x[7]));
+  st_quad(d + 2, make_float4(x[8], x[9], x[10], x[11]));
+  st_quad(d + 3, make_float4(x[12], x[13], x[14], 1.0f));
+}
+
+// The episodes an env (thread per env) or a warp (warp per env) finished in the launch.  At the end each CTA sums its
+// tallies into shared counters, blk[3] (episodes, terminated, length sum) and blk_ret (return sum), zeroed by
+// cta_stats_init; after a CTA barrier, thread 0 adds them to the CTA's StatSlot (cta_stats_commit).
+struct EpisodeTally {
+  // in this order, and declared after the kernels' n_trunc: the rollout kernels keep the register counts (-Xptxas -v)
+  // they had with four local counters
+  float ret_sum = 0.f;
+  uint32_t len_sum = 0, n_term = 0, n_done = 0;
+
+  __device__ __forceinline__ void add(bool crashed, const EnvState& s) {
+    n_done += 1;
+    n_term += crashed ? 1 : 0;
+    len_sum += (uint32_t)s.ep_len;
+    ret_sum += s.ep_ret;
+  }
+  // one env per lane: warp sums, then lane 0's shared atomics (every lane of the warp calls this)
+  __device__ __forceinline__ void flush_warp(unsigned long long (&blk)[3], double& blk_ret, int lane) const {
+    if (__ballot_sync(0xffffffffu, n_done != 0)) {
+      const uint32_t d = __reduce_add_sync(0xffffffffu, n_done);
+      const uint32_t t = __reduce_add_sync(0xffffffffu, n_term);
+      const uint32_t l = __reduce_add_sync(0xffffffffu, len_sum);
+      double rs = (double)ret_sum;
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) rs += __shfl_xor_sync(0xffffffffu, rs, o);
+      if (lane == 0) {
+        atomicAdd(&blk[0], (unsigned long long)d);
+        atomicAdd(&blk[1], (unsigned long long)t);
+        atomicAdd(&blk[2], (unsigned long long)l);
+        atomicAdd(&blk_ret, rs);
+      }
+    }
+  }
+  // the tally is already the warp's (one env per warp): its writer lane adds it as it stands
+  __device__ __forceinline__ void flush_lane(unsigned long long (&blk)[3], double& blk_ret) const {
+    if (n_done != 0) {
+      atomicAdd(&blk[0], (unsigned long long)n_done);
+      atomicAdd(&blk[1], (unsigned long long)n_term);
+      atomicAdd(&blk[2], (unsigned long long)len_sum);
+      atomicAdd(&blk_ret, (double)ret_sum);
+    }
+  }
+};
+
+__device__ __forceinline__ void cta_stats_init(unsigned long long (&blk)[3], double& blk_ret) {
+  if (threadIdx.x < 3) blk[threadIdx.x] = 0;
+  if (threadIdx.x == 3) blk_ret = 0.0;
+}
+
+// thread 0 after the CTA barrier that follows every flush, slot = stats + blockIdx.x % kStatSlots (the CTA's line)
+__device__ __forceinline__ void cta_stats_commit(StatSlot* slot, const unsigned long long (&blk)[3], const double& blk_ret) {
+  if (blk[0] != 0) {
+    atomicAdd(&slot->episodes, blk[0]);
+    atomicAdd(&slot->terminated, blk[1]);
+    atomicAdd(&slot->length_sum, blk[2]);
+    atomicAdd(&slot->return_sum, blk_ret);
+  }
+}
+
 // TIMEOUT: a step that ended by the time limit alone (timeout && !crashed: Gymnasium's truncated), recorded after step_env
 // and before reset_env -- the observation SB3 keeps as info["terminal_observation"].  j counts this env's truncations.
 __device__ __forceinline__ void record_truncation(const PolicyArgs& A, const EnvState& s, const int64_t i, const int k,
@@ -148,11 +255,7 @@ __device__ __forceinline__ void record_truncation(const PolicyArgs& A, const Env
     float x[kObs];
     write_obs<kObs>(x, s);
     const size_t slot = (size_t)j * (size_t)A.n + (size_t)i;
-    float4* d = reinterpret_cast<float4*>(A.term_obs + slot * 16);
-    st_quad(d, make_float4(x[0], x[1], x[2], x[3]));
-    st_quad(d + 1, make_float4(x[4], x[5], x[6], x[7]));
-    st_quad(d + 2, make_float4(x[8], x[9], x[10], x[11]));
-    st_quad(d + 3, make_float4(x[12], x[13], x[14], 1.0f));
+    store_row16(A.term_obs + slot * 16, x);
     A.term_row[slot] = (int32_t)((int64_t)k * A.n + i);
   }
   ++j;
@@ -176,9 +279,8 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
   __shared__ float s_norm[NORM ? kNormAffine : 1];
 
   load_mlp_smem(S, A.theta);
-  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s_norm[threadIdx.x] = A.norm[threadIdx.x]; }
-  if (threadIdx.x < 3) blk_stats[threadIdx.x] = 0;
-  if (threadIdx.x == 3) blk_ret = 0.0;
+  load_norm<NORM>(s_norm, A.norm);
+  cta_stats_init(blk_stats, blk_ret);
   __syncthreads();
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -194,13 +296,11 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
   EnvState s = {};
   if (active) s = load_state(A.state, i);
 
-  float std_[kAct], logstd_sum = 0.f;
-#pragma unroll
-  for (int o = 0; o < kAct; ++o) { std_[o] = expf(S.log_std[o]); logstd_sum += S.log_std[o]; }
+  float std_[kAct];
+  const float logstd_sum = policy_std(S.log_std, std_);
 
-  uint32_t n_done = 0, n_term = 0, len_sum = 0;
-  float ret_sum = 0.f;
   int32_t n_trunc = 0;
+  EpisodeTally tally;
   float4* p_act = A.actions + i;
   float* p_logp = A.logp + i;
   float* p_val = A.value + i;
@@ -213,14 +313,8 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
   for (int k = 0; k < A.K; ++k) {
     float x[kObs];
     write_obs<kObs>(x, s);
-    if (A.obs != nullptr && A.obs_padded) {        // 64-byte rows: four 128-bit stores straight from the registers
-      if (active) {
-        float4* d = reinterpret_cast<float4*>(A.obs + ((size_t)k * (size_t)n + (size_t)i) * 16);
-        st_quad(d, make_float4(x[0], x[1], x[2], x[3]));
-        st_quad(d + 1, make_float4(x[4], x[5], x[6], x[7]));
-        st_quad(d + 2, make_float4(x[8], x[9], x[10], x[11]));
-        st_quad(d + 3, make_float4(x[12], x[13], x[14], 1.0f));
-      }
+    if (A.obs != nullptr && A.obs_padded) {
+      if (active) store_row16(A.obs + ((size_t)k * (size_t)n + (size_t)i) * 16, x);
     } else if (A.obs != nullptr && valid > 0) emit_obs_rows<kObs>(tile, p_obs, s, lane, valid, active, fast_obs);
     if constexpr (NORM) norm_obs_row(x, s_norm);
 
@@ -228,22 +322,9 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
     tower_forward<kAct>(S, 0, x, mean);
     tower_forward<1>(S, 1, x, val);
 
-    float4 a;
     float logp;
-    if (A.deterministic) {
-      a = make_float4(mean[0], mean[1], mean[2], mean[3]);
-      logp = -logstd_sum - kAct * kHalfLog2Pi;
-    } else {
-      const float4 z = noise_normals(P.keys, env_id, A.t0 + (uint64_t)k);
-      a = make_float4(fmaf(std_[0], z.x, mean[0]), fmaf(std_[1], z.y, mean[1]),
-                      fmaf(std_[2], z.z, mean[2]), fmaf(std_[3], z.w, mean[3]));
-      // Normal(mean, std).log_prob(a) summed over the 4 dims; (a - mean) / std == z up to rounding
-      logp = -0.5f * (z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w) - logstd_sum - kAct * kHalfLog2Pi;
-    }
-    // np.clip(a, low, high) for the env only (SB3 collect_rollouts); the buffer keeps `a`
-    const float4 f = make_float4(fminf(fmaxf(a.x, 0.f), P.motor_max), fminf(fmaxf(a.y, 0.f), P.motor_max),
-                                 fminf(fmaxf(a.z, 0.f), P.motor_max), fminf(fmaxf(a.w, 0.f), P.motor_max));
-    const StepResult r = step_env(s, P, f);
+    const float4 a = policy_action(mean, std_, logstd_sum, P.keys, env_id, A.t0 + (uint64_t)k, A.deterministic, logp);
+    const StepResult r = step_env(s, P, env_action(a, P.motor_max));
     const bool done = r.crashed || r.timeout;
     if (active) {
       if (A.actions != nullptr) st_quad(p_act, a);
@@ -252,10 +333,7 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
       if (A.reward != nullptr) *p_rew = r.reward;
       if (A.done != nullptr) *p_done = done ? 1 : 0;
       if (done) {
-        n_done += 1;
-        n_term += r.crashed ? 1 : 0;
-        len_sum += (uint32_t)s.ep_len;
-        ret_sum += s.ep_ret;
+        tally.add(r.crashed, s);
         if constexpr (TIMEOUT) { if (!r.crashed) record_truncation(A, s, i, k, n_trunc, true); }
         reset_env<RANDOMIZED>(s, P, env_id);       // the PPO path always auto-resets (DummyVecEnv)
       }
@@ -279,28 +357,9 @@ __global__ void __launch_bounds__(kPolBlock) policy_rollout_kernel(const __grid_
   if (active) store_state(A.state, i, s);
   if constexpr (TIMEOUT) { if (active) close_truncation_slots(A, i, n_trunc); }
 
-  if (__ballot_sync(0xffffffffu, n_done != 0)) {
-    n_done = __reduce_add_sync(0xffffffffu, n_done);
-    n_term = __reduce_add_sync(0xffffffffu, n_term);
-    len_sum = __reduce_add_sync(0xffffffffu, len_sum);
-    double rs = (double)ret_sum;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) rs += __shfl_xor_sync(0xffffffffu, rs, o);
-    if (lane == 0) {
-      atomicAdd(&blk_stats[0], (unsigned long long)n_done);
-      atomicAdd(&blk_stats[1], (unsigned long long)n_term);
-      atomicAdd(&blk_stats[2], (unsigned long long)len_sum);
-      atomicAdd(&blk_ret, rs);
-    }
-  }
+  tally.flush_warp(blk_stats, blk_ret, lane);
   __syncthreads();
-  if (threadIdx.x == 0 && blk_stats[0] != 0) {
-    StatSlot* slot = A.stats + (blockIdx.x % kStatSlots);
-    atomicAdd(&slot->episodes, blk_stats[0]);
-    atomicAdd(&slot->terminated, blk_stats[1]);
-    atomicAdd(&slot->length_sum, blk_stats[2]);
-    atomicAdd(&slot->return_sum, blk_ret);
-  }
+  if (threadIdx.x == 0) cta_stats_commit(A.stats + (blockIdx.x % kStatSlots), blk_stats, blk_ret);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -361,9 +420,8 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(c
   __shared__ double blk_ret;
   __shared__ float s_norm[NORM ? kNormAffine : 1];
   load_mlp_smem(S, A.theta);
-  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s_norm[threadIdx.x] = A.norm[threadIdx.x]; }
-  if (threadIdx.x < 3) blk_stats[threadIdx.x] = 0;
-  if (threadIdx.x == 3) blk_ret = 0.0;
+  load_norm<NORM>(s_norm, A.norm);
+  cta_stats_init(blk_stats, blk_ret);
   __syncthreads();
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -377,12 +435,10 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(c
 
   EnvState s = {};
   if (active) s = load_state(A.state, i);                                 // every lane holds the whole state
-  float std_[kAct], logstd_sum = 0.f;
-#pragma unroll
-  for (int o = 0; o < kAct; ++o) { std_[o] = expf(S.log_std[o]); logstd_sum += S.log_std[o]; }
-  uint32_t n_done = 0, n_term = 0, len_sum = 0;
-  float ret_sum = 0.f;
+  float std_[kAct];
+  const float logstd_sum = policy_std(S.log_std, std_);
   int32_t n_trunc = 0;
+  EpisodeTally tally;
 
   for (int k = 0; k < A.K; ++k) {
     float x[kObs];
@@ -403,20 +459,9 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(c
     tower_forward_warp<kAct>(S, hbuf, 0, x, mean, lane);
     tower_forward_warp<1>(S, hbuf, 1, x, val, lane);
 
-    float4 a;
     float logp;
-    if (A.deterministic) {
-      a = make_float4(mean[0], mean[1], mean[2], mean[3]);
-      logp = -logstd_sum - kAct * kHalfLog2Pi;
-    } else {
-      const float4 z = noise_normals(P.keys, env_id, A.t0 + (uint64_t)k);
-      a = make_float4(fmaf(std_[0], z.x, mean[0]), fmaf(std_[1], z.y, mean[1]),
-                      fmaf(std_[2], z.z, mean[2]), fmaf(std_[3], z.w, mean[3]));
-      logp = -0.5f * (z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w) - logstd_sum - kAct * kHalfLog2Pi;
-    }
-    const float4 f = make_float4(fminf(fmaxf(a.x, 0.f), P.motor_max), fminf(fmaxf(a.y, 0.f), P.motor_max),
-                                 fminf(fmaxf(a.z, 0.f), P.motor_max), fminf(fmaxf(a.w, 0.f), P.motor_max));
-    const StepResult r = step_env(s, P, f);
+    const float4 a = policy_action(mean, std_, logstd_sum, P.keys, env_id, A.t0 + (uint64_t)k, A.deterministic, logp);
+    const StepResult r = step_env(s, P, env_action(a, P.motor_max));
     const bool done = r.crashed || r.timeout;
     if (writer) {
       if (A.actions != nullptr) A.actions[row] = a;
@@ -426,10 +471,7 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(c
       if (A.done != nullptr) A.done[row] = done ? 1 : 0;
     }
     if (active && done) {                                                 // warp-uniform
-      n_done += 1;
-      n_term += r.crashed ? 1 : 0;
-      len_sum += (uint32_t)s.ep_len;
-      ret_sum += s.ep_ret;
+      tally.add(r.crashed, s);
       if constexpr (TIMEOUT) { if (!r.crashed) record_truncation(A, s, i, k, n_trunc, lane == 0); }
       reset_env<RANDOMIZED>(s, P, env_id);
     }
@@ -457,21 +499,10 @@ __global__ void __launch_bounds__(32 * kSmallWarps) policy_rollout_warp_kernel(c
   if (writer) {
     store_state(A.state, i, s);
     if constexpr (TIMEOUT) close_truncation_slots(A, i, n_trunc);
-    if (n_done != 0) {
-      atomicAdd(&blk_stats[0], (unsigned long long)n_done);
-      atomicAdd(&blk_stats[1], (unsigned long long)n_term);
-      atomicAdd(&blk_stats[2], (unsigned long long)len_sum);
-      atomicAdd(&blk_ret, (double)ret_sum);
-    }
+    tally.flush_lane(blk_stats, blk_ret);
   }
   __syncthreads();
-  if (threadIdx.x == 0 && blk_stats[0] != 0) {
-    StatSlot* slot = A.stats + (blockIdx.x % kStatSlots);
-    atomicAdd(&slot->episodes, blk_stats[0]);
-    atomicAdd(&slot->terminated, blk_stats[1]);
-    atomicAdd(&slot->length_sum, blk_stats[2]);
-    atomicAdd(&slot->return_sum, blk_ret);
-  }
+  if (threadIdx.x == 0) cta_stats_commit(A.stats + (blockIdx.x % kStatSlots), blk_stats, blk_ret);
 }
 
 // policy(obs) for arbitrary observation rows: mean [B,4], value [B]  (PPO.predict / policy.forward)

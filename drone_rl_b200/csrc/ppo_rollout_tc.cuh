@@ -43,9 +43,8 @@ __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __gr
   __shared__ unsigned long long blk_stats[3];
   __shared__ double blk_ret;
   __shared__ float s_norm[NORM ? kNormAffine : 1];
-  if (threadIdx.x < 3) blk_stats[threadIdx.x] = 0;
-  if (threadIdx.x == 3) blk_ret = 0.0;
-  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s_norm[threadIdx.x] = A.norm[threadIdx.x]; }
+  cta_stats_init(blk_stats, blk_ret);
+  load_norm<NORM>(s_norm, A.norm);
   tc::setup(S, A.theta);
 
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -60,13 +59,12 @@ __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __gr
 
   EnvState s = {};
   if (active) s = load_state(A.state, i);
-  float std_[kAct], logstd_sum = 0.f;
-#pragma unroll
-  for (int o = 0; o < kAct; ++o) { std_[o] = expf(S.log_std[o]); logstd_sum += S.log_std[o]; }
+  float std_[kAct];
+  const float logstd_sum = policy_std(S.log_std, std_);
 
-  uint32_t n_done = 0, n_term = 0, len_sum = 0, phase = 0;
-  float ret_sum = 0.f;
   int32_t n_trunc = 0;
+  EpisodeTally tally;
+  uint32_t phase = 0;
   float4* p_act = A.actions + i;
   float* p_logp = A.logp + i;
   float* p_val = A.value + i;
@@ -78,34 +76,17 @@ __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __gr
   for (int k = 0; k < A.K; ++k) {
     float x[kObs];
     write_obs<kObs>(x, s);
-    if (A.obs != nullptr && A.obs_padded) {        // 64-byte rows: four 128-bit stores straight from the registers
-      if (active) {
-        float4* d = reinterpret_cast<float4*>(A.obs + ((size_t)k * (size_t)n + (size_t)i) * 16);
-        st_quad(d, make_float4(x[0], x[1], x[2], x[3]));
-        st_quad(d + 1, make_float4(x[4], x[5], x[6], x[7]));
-        st_quad(d + 2, make_float4(x[8], x[9], x[10], x[11]));
-        st_quad(d + 3, make_float4(x[12], x[13], x[14], 1.0f));
-      }
+    if (A.obs != nullptr && A.obs_padded) {
+      if (active) store_row16(A.obs + ((size_t)k * (size_t)n + (size_t)i) * 16, x);
     } else if (A.obs != nullptr && valid > 0) emit_obs_rows<kObs>(tile, p_obs, s, lane, valid, active, fast_obs);
     if constexpr (NORM) norm_obs_row(x, s_norm);
 
     float mean[kAct], val;
     tc::forward(S, x, phase, mean, val);
 
-    float4 a;
     float logp;
-    if (A.deterministic) {
-      a = make_float4(mean[0], mean[1], mean[2], mean[3]);
-      logp = -logstd_sum - kAct * kHalfLog2Pi;
-    } else {
-      const float4 z = noise_normals(P.keys, env_id, A.t0 + (uint64_t)k);
-      a = make_float4(fmaf(std_[0], z.x, mean[0]), fmaf(std_[1], z.y, mean[1]),
-                      fmaf(std_[2], z.z, mean[2]), fmaf(std_[3], z.w, mean[3]));
-      logp = -0.5f * (z.x * z.x + z.y * z.y + z.z * z.z + z.w * z.w) - logstd_sum - kAct * kHalfLog2Pi;
-    }
-    const float4 f = make_float4(fminf(fmaxf(a.x, 0.f), P.motor_max), fminf(fmaxf(a.y, 0.f), P.motor_max),
-                                 fminf(fmaxf(a.z, 0.f), P.motor_max), fminf(fmaxf(a.w, 0.f), P.motor_max));
-    const StepResult r = step_env(s, P, f);
+    const float4 a = policy_action(mean, std_, logstd_sum, P.keys, env_id, A.t0 + (uint64_t)k, A.deterministic, logp);
+    const StepResult r = step_env(s, P, env_action(a, P.motor_max));
     const bool done = r.crashed || r.timeout;
     if (active) {
       if (A.actions != nullptr) st_quad(p_act, a);
@@ -114,10 +95,7 @@ __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __gr
       if (A.reward != nullptr) *p_rew = r.reward;
       if (A.done != nullptr) *p_done = done ? 1 : 0;
       if (done) {
-        n_done += 1;
-        n_term += r.crashed ? 1 : 0;
-        len_sum += (uint32_t)s.ep_len;
-        ret_sum += s.ep_ret;
+        tally.add(r.crashed, s);
         if constexpr (TIMEOUT) { if (!r.crashed) record_truncation(A, s, i, k, n_trunc, true); }
         reset_env<RANDOMIZED>(s, P, env_id);
       }
@@ -140,28 +118,9 @@ __global__ void __launch_bounds__(tc::kTile) policy_rollout_tc_kernel(const __gr
   if (active) store_state(A.state, i, s);
   if constexpr (TIMEOUT) { if (active) close_truncation_slots(A, i, n_trunc); }
 
-  if (__ballot_sync(0xffffffffu, n_done != 0)) {
-    n_done = __reduce_add_sync(0xffffffffu, n_done);
-    n_term = __reduce_add_sync(0xffffffffu, n_term);
-    len_sum = __reduce_add_sync(0xffffffffu, len_sum);
-    double rs = (double)ret_sum;
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) rs += __shfl_xor_sync(0xffffffffu, rs, o);
-    if (lane == 0) {
-      atomicAdd(&blk_stats[0], (unsigned long long)n_done);
-      atomicAdd(&blk_stats[1], (unsigned long long)n_term);
-      atomicAdd(&blk_stats[2], (unsigned long long)len_sum);
-      atomicAdd(&blk_ret, rs);
-    }
-  }
+  tally.flush_warp(blk_stats, blk_ret, lane);
   tc::teardown(S);        // contains the CTA barrier that orders the atomics above
-  if (threadIdx.x == 0 && blk_stats[0] != 0) {
-    StatSlot* slot = A.stats + (blockIdx.x % kStatSlots);
-    atomicAdd(&slot->episodes, blk_stats[0]);
-    atomicAdd(&slot->terminated, blk_stats[1]);
-    atomicAdd(&slot->length_sum, blk_stats[2]);
-    atomicAdd(&slot->return_sum, blk_ret);
-  }
+  if (threadIdx.x == 0) cta_stats_commit(A.stats + (blockIdx.x % kStatSlots), blk_stats, blk_ret);
 }
 
 }  // namespace dronecu

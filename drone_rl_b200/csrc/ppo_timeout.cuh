@@ -20,7 +20,7 @@ __global__ void __launch_bounds__(kPolBlock) timeout_bootstrap_kernel(const floa
   MlpSmem& S = *reinterpret_cast<MlpSmem*>(smem_raw);
   __shared__ float s_norm[NORM ? kNormAffine : 1];
   load_mlp_smem(S, theta);
-  if constexpr (NORM) { if (threadIdx.x < kNormAffine) s_norm[threadIdx.x] = norm[threadIdx.x]; }
+  load_norm<NORM>(s_norm, norm);
   __syncthreads();
   for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < slots; q += (int64_t)gridDim.x * blockDim.x) {
     const int32_t row = term_row[q];

@@ -296,15 +296,19 @@ __device__ __forceinline__ void tower(Smem& S, const int t, const float (&xv)[16
   // wrote D2 has completed (mbarrier), so no further barrier is needed here.
 }
 
+// this thread's A row of layer 1: the observation rounded to tf32, then the 1.0 of the bias column
+__device__ __forceinline__ void a_row(const float (&x)[kObs], float (&xv)[16]) {
+#pragma unroll
+  for (int i = 0; i < kObs; ++i) xv[i] = to_tf32_fast(x[i]);
+  xv[15] = 1.0f;
+}
+
 // Forward of both towers.  `phase` is the running mbarrier parity (0 before the first call).
 // dbg1 / dbg2 (nullable): this thread's 128 pre-activations (pi 0..63 | vf 64..127) of layer 1 / 2.
 __device__ __forceinline__ void forward(Smem& S, const float (&x)[kObs], uint32_t& phase, float (&mean)[kAct],
                                         float& value, float* dbg1 = nullptr, float* dbg2 = nullptr) {
-  float xv[16];
-#pragma unroll
-  for (int i = 0; i < kObs; ++i) xv[i] = to_tf32_fast(x[i]);
-  xv[15] = 1.0f;
-  float v1[1];
+  float xv[16], v1[1];
+  a_row(x, xv);
   tower<kAct>(S, 0, xv, phase, mean, dbg1, dbg2);
   tower<1>(S, 1, xv, phase, v1, dbg1 ? dbg1 + kHid : nullptr, dbg2 ? dbg2 + kHid : nullptr);
   value = v1[0];
@@ -313,18 +317,14 @@ __device__ __forceinline__ void forward(Smem& S, const float (&x)[kObs], uint32_
 // policy tower only (evaluation: ppo_eval.cuh); the same MMAs on the same operands as the pi tower of forward()
 __device__ __forceinline__ void forward_policy(Smem& S, const float (&x)[kObs], uint32_t& phase, float (&mean)[kAct]) {
   float xv[16];
-#pragma unroll
-  for (int i = 0; i < kObs; ++i) xv[i] = to_tf32_fast(x[i]);
-  xv[15] = 1.0f;
+  a_row(x, xv);
   tower<kAct>(S, 0, xv, phase, mean, nullptr, nullptr);
 }
 
 // value tower only (the GAE bootstrap after the last step)
 __device__ __forceinline__ float forward_value(Smem& S, const float (&x)[kObs], uint32_t& phase) {
   float xv[16], v1[1];
-#pragma unroll
-  for (int i = 0; i < kObs; ++i) xv[i] = to_tf32_fast(x[i]);
-  xv[15] = 1.0f;
+  a_row(x, xv);
   tower<1>(S, 1, xv, phase, v1, nullptr, nullptr);
   return v1[0];
 }

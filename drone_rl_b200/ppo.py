@@ -328,16 +328,14 @@ class PPO:
         # tensor cores pay from ~1k envs (a tile is 128 envs; below that the float32 warp-per-env kernel is both faster and exact)
         use_tc = self.rollout_precision == "tf32" and self.n_envs > self.tc_min_envs
         nz = self.normalizer
+        affine = None if nz is None else nz.affine_ptr()      # NULL: the plain dronecu_rollout_policy[_tc] rollout
         if self.handle_timeout_termination:
             _lib.check(self.lib.dronecu_rollout_policy_timeouts(self.batch._h, K, _ptr(self.params), int(deterministic), C.byref(out),
-                                                                None if nz is None else nz.affine_ptr(), int(use_tc),
-                                                                C.byref(self._timeout_buf), st), "dronecu_rollout_policy_timeouts")
-        elif nz is None:
-            fn = self.lib.dronecu_rollout_policy_tc if use_tc else self.lib.dronecu_rollout_policy
-            _lib.check(fn(self.batch._h, K, _ptr(self.params), int(deterministic), C.byref(out), st), "dronecu_rollout_policy")
+                                                                affine, int(use_tc), C.byref(self._timeout_buf), st),
+                       "dronecu_rollout_policy_timeouts")
         else:
             _lib.check(self.lib.dronecu_rollout_policy_norm(self.batch._h, K, _ptr(self.params), int(deterministic), C.byref(out),
-                                                            nz.affine_ptr(), int(use_tc), st), "dronecu_rollout_policy_norm")
+                                                            affine, int(use_tc), st), "dronecu_rollout_policy_norm")
         # the bootstrap adds to the reward the buffer finally holds (SB3: to the VecNormalize reward), with the observation
         # record the rollout used: after the normalisation pass, before the merge replaces the record
         bootstrap = self._bootstrap_timeouts if self.handle_timeout_termination else None
